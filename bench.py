@@ -17,6 +17,8 @@ torch.distributed.run, one rank per GPU).  Rank 0 prints ONE JSON line.
 * cpu_baseline = oracle/refshape.py (reference-shaped scalar loop) on all host cores, bounded sample.
 * ``--impl reference`` = that same CPU loop as the timed arm (the reference itself cannot run:
   python2 + PyKDL/vfl/arcospyu/yarp are absent; see DESIGN.md).
+* ``--dump-outputs DIR`` = q and qdot after the last timed step, as .npy files (at most 60 MiB: a seeded sample of the
+  instances where the shard is larger); the inputs are seeded, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -51,6 +53,23 @@ WORKLOADS = {
 def algorithmic_bytes(n_joints: int, n_obst: int, elem: int) -> int:
     """Compulsory HBM bytes per instance per launch (SURVEY.md 8d): q in/out 2N, qdot out N, goal 13, obstacles 4M."""
     return elem * (3 * n_joints + 13 + 4 * n_obst)
+
+
+DUMP_BUDGET = 60 << 20      # bytes of array data --dump-outputs writes at most
+
+
+def write_outputs(out_dir: str, arrays: dict, budget: int = DUMP_BUDGET):
+    """Save dense ``[comps, instances]`` arrays as ``out_dir/<name>.npy``.  When they exceed ``budget`` bytes together, the
+    same seeded sample of instances (columns, in order) is taken from every array, so that two runs with the same
+    arguments write the same instances."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = next(iter(arrays.values())).shape[1]
+    per_instance = sum(a.itemsize * a.shape[0] for a in arrays.values())
+    if per_instance * n > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // per_instance, replace=False))
+        arrays = {name: a[:, idx] for name, a in arrays.items()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def kernel_source_stamp() -> str:
@@ -272,7 +291,15 @@ def main():
     ap.add_argument("--cpu-cycles", type=int, default=1000, help="CPU arm: control cycles per core per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the K-fused and FP64 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the joint positions and velocities of the last timed step (rank 0's "
+                         "shard) as DIR/q.npy and DIR/qdot.npy, [joints, instances] in the run's precision, so that two builds "
+                         "can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -370,6 +397,9 @@ def main():
     ms = timed(lambda: step_rotating(args.kcycles), args.steps)
     gpu_launches = eng.launches - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        last = dbs[(rot["i"] - 1) % n_rot]             # the batch the last timed step advanced: q integrated in place, qdot
+        write_outputs(args.dump_outputs, {name: last.download(name) for name in ("q", "qdot")})
     value = world * n_inst * args.kcycles * args.steps / (ms * 1e-3)
     launch_ms = ms / args.steps
     peaks = {}

@@ -1119,3 +1119,35 @@ def test_round2_shapes_stay_inside_their_buffers(lwr, built_lib, monkeypatch, pr
             e.close()
             for key in env:
                 monkeypatch.delenv(key)
+
+
+def test_bench_dump_outputs_are_the_last_timed_launch(lwr, built_lib, tmp_path):
+    """`bench.py --dump-outputs` writes q and qdot of the last timed step.  At 4096 instances the launches rotate over more
+    copies of the seeded batch than warm-up and timed steps together, so the last one advanced its copy once: the dump is
+    one cycle of the engine on that batch, bit for bit."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from vfclik_b200 import workloads
+    from vfclik_b200.engine import DeviceBatch, Engine, Params
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, m = 4096, 32
+    res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1",
+                          "--instances", str(n), "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
+    assert res.returncode == 0, res.stderr[-2000:]
+    line = json.loads(res.stdout.splitlines()[-1])
+    assert line["steps"] == 3 and line["gpu_launches"] == 3
+    chain, cfg = lwr
+    e = Engine(chain, precision=32, params=Params.from_config(cfg))
+    try:
+        w = workloads.random_batch(chain, n, m, seed=1, dtype=np.float32)
+        db = DeviceBatch(e, n, m, outputs=("qdot",))
+        db.upload("q", w["q"]); db.upload("goal", w["goal"]); db.upload("obst", w["obst"])
+        assert db.step(1) == 1
+        for name in ("q", "qdot"):
+            got = np.load(tmp_path / (name + ".npy"))
+            assert got.dtype == np.float32 and np.array_equal(got, db.download(name)), name
+    finally:
+        e.close()

@@ -453,3 +453,25 @@ def test_bench_reference_arm_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] > 0 and "control cycles" in cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_write_outputs_whole_or_seeded_sample(tmp_path):
+    """`bench.py --dump-outputs` writes arrays that fit the budget whole, and larger ones as the same seeded sample of
+    instances (columns) in every array and every run, within the budget."""
+    import bench
+    rng = np.random.default_rng(4)
+    arrays = {"q": rng.normal(size=(7, 5000)).astype(np.float32), "qdot": rng.normal(size=(7, 5000))}
+    bench.write_outputs(str(tmp_path / "whole"), arrays, budget=1 << 20)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "whole" / (name + ".npy"))
+        assert got.dtype == a.dtype and np.array_equal(got, a)
+    budget = 20000
+    for run in ("a", "b"):
+        bench.write_outputs(str(tmp_path / run), arrays, budget=budget)
+    got = {run: {name: np.load(tmp_path / run / (name + ".npy")) for name in arrays} for run in ("a", "b")}
+    assert sum(a.nbytes for a in got["a"].values()) <= budget
+    cols = [int(np.flatnonzero(arrays["q"][0] == x)[0]) for x in got["a"]["q"][0]]
+    assert len(cols) == budget // (7 * 4 + 7 * 8) and cols == sorted(set(cols))
+    for name, a in arrays.items():
+        assert got["a"][name].dtype == a.dtype and np.array_equal(got["a"][name], a[:, cols])
+        assert np.array_equal(got["a"][name], got["b"][name])

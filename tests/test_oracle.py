@@ -280,7 +280,8 @@ def test_ik_mode_kdl_wdls_form(lwr):
     assert not np.allclose(c, b, rtol=1e-3)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(os.environ.get("VFCLIK_REFERENCE", "")),
+                    reason="needs the original vfclik sources: set VFCLIK_REFERENCE to a checkout of them")
 def test_golden_is_reproducible_from_reference(golden):
     """Regenerating from the real reference gives the committed vectors (guards a stale fixture)."""
     from oracle import gen_golden
