@@ -10,12 +10,9 @@ import dataclasses
 import numpy as np
 import pytest
 
-from helpers import oracle_parallel, oracle_params, rel_err, to_oracle
+from helpers import FP32_RTOL, FP64_RTOL, check, oracle_parallel, oracle_params, rel_err, run_gpu, run_oracle, to_oracle
 
 pytestmark = pytest.mark.gpu
-
-FP64_RTOL = 1e-9
-FP32_RTOL = 1e-4
 
 
 @pytest.fixture(scope="module")
@@ -32,43 +29,6 @@ def eng(lwr, built_lib):
     yield get
     for e in engines.values():
         e.close()
-
-
-def run_gpu(engine, w, n_obst, k=1, outputs=("qdot_vf", "qdot_ns", "qdot_jp", "qdot", "cmd", "pose", "flags"),
-            extra=None):
-    from vfclik_b200.engine import DeviceBatch
-    n = w["q"].shape[1]
-    db = DeviceBatch(engine, n, n_obst, obst_ext="obst_ext" in w, outputs=outputs)
-    db.upload("q", w["q"])
-    db.upload("goal", w["goal"])
-    if n_obst:
-        db.upload("obst", w["obst"])
-        if "obst_ext" in w:
-            db.upload("obst_ext", w["obst_ext"])
-    for name, arr in (extra or {}).items():
-        db.upload(name, arr)
-    assert db.step(k) == 1
-    out = {name: db.download(name).T for name in outputs}
-    out["q"] = db.download("q").T
-    if "flags" in out:
-        out["flags"] = out["flags"][:, 0]
-    if "ns_lastvec" in db.t:
-        out["lastvec"] = db.download("ns_lastvec").T
-    return out
-
-
-def run_oracle(chain, params, w, n_obst, k=1, **kw):
-    from oracle import batch
-    q, goal, obst = to_oracle(w, n_obst)
-    return batch.step(chain, oracle_params(params), q, goal, obst, k_cycles=k, **kw)
-
-
-def check(out, ref, rtol, keys=("qdot_vf", "qdot_ns", "qdot_jp", "qdot", "cmd"), pose_atol=None):
-    for k in keys:
-        e = rel_err(out[k].astype(np.float64), ref[k])
-        assert e.max() <= rtol, (k, float(e.max()), int(np.argmax(e)))
-    if pose_atol is not None:
-        assert np.max(np.abs(out["pose"] - ref["pose"])) <= pose_atol
 
 
 @pytest.mark.parametrize("n", [1, 127, 4096])

@@ -450,7 +450,9 @@ __device__ __forceinline__ void attract(const KConst<T>& c, const T (&g)[13], co
     } else {
         angle = T(2) * Prec<T>::atan2_(nrm, qw);
     }
-    const T S1 = Prec<T>::fmin_(T(1), angle * c.rot_slowdown_inv);     // rot_slowdown_inv = +inf when off
+    // rot_slowdown_inv = +inf when off.  The product goes first: at angle = 0 it is 0 * inf = NaN, and fmin_ then selects 1
+    // (FP64's fmin_ is `a < b ? a : b`, which returns its second operand when the first is NaN).
+    const T S1 = Prec<T>::fmin_(angle * c.rot_slowdown_inv, T(1));
     const T sr = c.speed_scale * S1 * c.goal_force * invn;
     w[0] = sr * qx; w[1] = sr * qy; w[2] = sr * qz;
 }
