@@ -9,9 +9,7 @@ from vfclik_b200.engine import DeviceBatch, Engine, Params
 cfg = load_config(config_filename(PACKAGE_CONFIG_DIR + "/lwr/", "lwr", "right"))
 lwr = chain_from_config(cfg)
 
-def run(chain, precision, n, m, k=2, outputs=("qdot",), params=None, extra=None, env=None):
-    for key, val in (env or {}).items():
-        os.environ[key] = val
+def run(chain, precision, n, m, k=2, outputs=("qdot",), params=None, extra=None):
     dt = np.float32 if precision == 32 else np.float64
     e = Engine(chain, precision=precision, params=params or Params())
     w = workloads.random_batch(chain, n, m, seed=5, dtype=dt)
@@ -26,21 +24,16 @@ def run(chain, precision, n, m, k=2, outputs=("qdot",), params=None, extra=None,
     out = db.download("qdot")
     assert np.all(np.isfinite(out))
     e.close()
-    for key in (env or {}):
-        os.environ.pop(key, None)
     return out
 
 full = ("qdot_vf", "qdot_ns", "qdot_jp", "qdot", "cmd", "pose", "twist", "flags")
 for precision in (32, 64):
     run(lwr, precision, 70, 33)                                             # lean, odd obstacle count (padding slot), ragged tile
     run(lwr, precision, 70, 9, outputs=full)                                # general
-    run(workloads.dual_arm_torso_chain(), precision, 100, 20)               # DhPattern lean (slim path, 3 stages)
+    run(workloads.dual_arm_torso_chain(), precision, 100, 20)               # FP32: DhPattern lean (slim path, 3 stages); FP64: lane-split kernel (tensor-map TMA)
     run(workloads.dual_arm_torso_chain(), precision, 40, 20)                # two tiles: two warps of the CTA have no work (they still pass the table barrier)
-    run(workloads.dual_arm_torso_chain(), precision, 100, 20, env={"VFK_SPLIT": "1"})     # lane-split kernel (tensor-map TMA)
-    run(workloads.dual_arm_torso_chain(10), precision, 100, 7, env={"VFK_SPLIT": "1"})
     run(workloads.torso_arm_chain(8), precision, 64, 5, outputs=full)       # padded chain in the 10-joint instantiation
     run(workloads.torso_arm_chain(3), precision, 64, 5, outputs=full)
-run(lwr, 64, 4200, 32, env={"VFK_SPLIT": "1"})                              # FP64 split, 7 joints
 run(workloads.torso_arm_chain(10), 64, 64, 4, outputs=full, params=Params(ns_mode=2, ns_control=(0.3, -0.2, 0.1, 0.2)),
     extra={"ns_lastvec": np.zeros((40, 64))})                               # control nullspace, 4 basis vectors
 run(lwr, 64, 64, 4, outputs=full, params=Params(ns_mode=1, ns_lambda=0.0))  # undamped projector through the Householder basis

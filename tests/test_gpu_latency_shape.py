@@ -351,9 +351,10 @@ def test_field_regimes(lwr_cfg, monkeypatch, precision, shape, rot_slowdown):
     """Goals within 1e-7 m / 1e-7 rad of the tool up to far away, translational slowdowns on and off, obstacles inside and
     outside their safe distance, through every kernel shape: the lean and the general one-thread instantiations, the
     per-obstacle {safe, order} path (FP32: the scalar MUFU repeller), the cooperative shape (FP64, M >= 16) and the lane
-    split (the FP64 17-joint default, FP32 with VFK_SPLIT=1).  Uniform decay orders 2 / 5 / 20 (FP64 multiplication chains),
-    3 (square-and-multiply) and 7.5 (pow), safe distances 0 / 1e-3 / 0.05; rot_slowdown 0.09 (FP32: the small-angle asin
-    series), 0.5 (atan2) and 0 (off)."""
+    split (the FP64 17-joint chain).  "split17" / "split10" are the 17- and 10-joint DH chains in the lean call shape; in
+    FP32 they run the one-thread DhPattern kernel, which took them over when the FP32 split shape was removed.  Uniform
+    decay orders 2 / 5 / 20 (FP64 multiplication chains), 3 (square-and-multiply) and 7.5 (pow), safe distances 0 / 1e-3 /
+    0.05; rot_slowdown 0.09 (FP32: the small-angle asin series), 0.5 (atan2) and 0 (off)."""
     from vfclik_b200 import workloads
     from vfclik_b200.engine import Engine, Params
     chain, cfg = lwr_cfg
@@ -366,10 +367,8 @@ def test_field_regimes(lwr_cfg, monkeypatch, precision, shape, rot_slowdown):
     if shape.startswith("split"):
         chain = workloads.dual_arm_torso_chain(17 if shape == "split17" else 10)
         prm = Params(rot_slowdown=rot_slowdown)
-        monkeypatch.setenv("VFK_SPLIT", "1")
     elif shape != "coop":
         monkeypatch.setenv("VFK_NO_COOP", "1")
-        monkeypatch.setenv("VFK_SPLIT", "0")
     e = Engine(chain, precision=precision, params=prm)
     try:
         for order, safe in ([(20.0, 1e-3)] if shape in ("ext",) else UNIFORM):

@@ -72,11 +72,10 @@ static void build_const(const vfk_ctx& h, KConst<T>& c) {
     const vfk_chain_desc& ch = h.canon;
     const vfk_params& p = h.params;
     const int n = ch.n_joints;
-    using W = typename KConst<T>::W;
-    for (int k = 0; k < 12; ++k) c.base[k] = (W)ch.base[k];
+    for (int k = 0; k < 12; ++k) c.base[k] = ch.base[k];
     bool unit = true, all_xt = true;
     for (int j = 0; j < n; ++j) {
-        for (int k = 0; k < 12; ++k) c.tip[j][k] = (W)ch.tip[j][k];
+        for (int k = 0; k < 12; ++k) c.tip[j][k] = ch.tip[j][k];
         c.q_lo[j] = (T)ch.q_lo[j];
         c.q_hi[j] = (T)ch.q_hi[j];
         const double rng = ch.q_hi[j] - ch.q_lo[j];
@@ -105,8 +104,8 @@ static void build_const(const vfk_ctx& h, KConst<T>& c) {
     c.tool_identity = memcmp(p.tool, ident, sizeof ident) == 0;
     for (int k = 0; k < 12; ++k) c.tool[k] = (T)p.tool[k];
     for (int k = 0; k < 4; ++k) c.ns_control[k] = (T)p.ns_control[k];
-    c.ik_lambda2 = (typename WideNE<T>::type)(p.ik_lambda * p.ik_lambda);
-    c.ns_lambda2 = (typename WideNE<T>::type)(p.ns_lambda * p.ns_lambda);
+    c.ik_lambda2 = (T)(p.ik_lambda * p.ik_lambda);
+    c.ns_lambda2 = (T)(p.ns_lambda * p.ns_lambda);
     c.dt = (T)p.dt;
     c.speed_scale = (T)p.speed_scale;
     c.max_vel = (T)p.max_vel;
@@ -829,15 +828,13 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
     //  the floor set by the two concurrent 29 MB PCIe transfers is 0.62 ms)
     int n_chunks = (int)(s->n / 65536);
     if (n_chunks > 4) n_chunks = 4;
-    if (const char* e = getenv("VFK_SESSION_CHUNKS")) n_chunks = atoi(e);
-    if (n_chunks > kMaxSessionChunks) n_chunks = kMaxSessionChunks;
     if (n_chunks < 1) n_chunks = 1;
     if ((int64_t)n_chunks > s->tiles) n_chunks = (int)s->tiles;
 
     // The pipeline is dozens of API calls; repeated calls with the same buffers replay ONE captured CUDA graph.
     // The first call with a given (buffers, K, parameter generation) runs eagerly (it also warms the launch-plan
     // caches), the second captures, later ones only launch the graph.
-    const bool use_graph = n_chunks > 1 && !getenv("VFK_NO_GRAPH");
+    const bool use_graph = n_chunks > 1;
     auto& key = s->graph_key;
     const bool same = key.src_q == src_q && key.dst_qd == dst_qd && key.dst_qo == dst_qo && key.dst_fl == dst_fl &&
                       key.k == k_cycles && key.hgen == h->generation && key.sgen == s->generation;

@@ -31,54 +31,32 @@
 namespace vfk {
 
 constexpr int kMaxJ = 17;
-#ifndef VFK_BLOCK
-#define VFK_BLOCK 128
-#endif
-constexpr int kBlock = VFK_BLOCK;    // threads per CTA of the cycle kernel (warps are independent workers; 64 measured 0.3 % slower, must divide 128)
+constexpr int kBlock = 128;          // threads per CTA of the cycle kernel (warps are independent workers; 64 measured 0.3 % slower)
 constexpr int kSmallBlock = 128;     // threads per CTA of the small one-element-per-thread kernels
-#ifndef VFK_CHUNK
-#define VFK_CHUNK 8
-#endif
-constexpr int kChunk = VFK_CHUNK;            // obstacles per shared-memory stage (4 measured: FP64 config 2 -13 %, -30 % with 3 CTAs/SM; FP32 headline -14 %)
+constexpr int kChunk = 8;            // obstacles per shared-memory stage (4 measured: FP64 config 2 -13 %, -30 % with 3 CTAs/SM; FP32 headline -14 %)
 constexpr int kMaxStages = 8;
 constexpr int kSmemHeader = 512;     // per-warp mbarriers live in the first 512 bytes of dynamic smem
-// TAB (kernel template parameter): the FP32 mode's wide kinematic chain takes sin / cos from a 128-entry table in shared
+// The FP32 mode's wide kinematic chain takes sin / cos from a 128-entry table in shared
 // memory (sincos_table, vfk_math.cuh: 13 FP64 operations per joint instead of 23, a dependent chain half as long); the
 // table sits between the header and the per-warp regions and is built once per CTA behind the first tile's copies.
 // Measured on B200 (same-box A/Bs, profiles/r02t_sincos_table_ab.txt): 17 joints K = 1 126.7 -> 123.6 us, K = 100 +3.2 %;
 // the headline shape K = 100 +4.7 - 5.3 % (1.34 -> 1.40e10 inst-cycles/s) and 0.983 instead of 0.960 of the HBM roofline
 // over 1000 launches (less FP64 work, later power cap).  Its HBM-bound single-cycle launch lost 3.4 % with the table while
 // every chunk still waited for DRAM (the table's random 16-byte reads are ~10 shared-memory wavefronts each, +45 % on the
-// L1 data pipe that also takes the TMA deliveries); with the L2 prefetch in place it is unchanged, so the host turns the
-// table on for every FP32 instantiation (launch_cycle).  -DVFK_NO_SINCOS_TABLE turns it off everywhere.
-#ifdef VFK_NO_SINCOS_TABLE
-constexpr bool kSinCosTable = false;
-#else
-constexpr bool kSinCosTable = true;
-#endif
+// L1 data pipe that also takes the TMA deliveries); with the L2 prefetch in place it is unchanged.  So every FP32 kernel
+// has the table, and K fused cycles stay bit-identical to K single-cycle launches.  The FP64 chain (every cooperative
+// kernel included) evaluates sincos_wide instead.
 template <typename T>
-constexpr bool kCanTab = kSinCosTable && sizeof(T) == 4 && sizeof(typename WideOf<T>::type) == 8;
-template <typename T, bool TAB>
-constexpr uint32_t kTabBytes = (TAB && kCanTab<T>) ? kSinCosTabEntries * 16 : 0;
-// FP32 decay order 20 (the reference's typical value, old/README.old:75) by five multiplications instead of MUFU lg2 / ex2:
-// two more instructions per obstacle but two fewer on the quarter-rate XU pipe, which also carries rsqrt and the
-// FP64 <-> FP32 conversions.  Measured on B200 (1 M instances): 109.1 us vs 110.3 us per launch at K = 1, -0.6 % at
-// K = 100; also the more accurate of the two.  -DVFK_NO_F32_POWCHAIN restores the MUFU form.
-#ifdef VFK_NO_F32_POWCHAIN
-constexpr bool kF32PowChain = false;
-#else
-constexpr bool kF32PowChain = true;
-#endif
+constexpr uint32_t kTabBytes = sizeof(T) == 4 ? kSinCosTabEntries * 16 : 0;
 
 // Kernel-side constants in the kernel's arithmetic type.  Joints are canonicalised on
 // the host (vfk_api.cu: canonicalise_chain) so that every joint acts about / along its
 // local Z axis: RotX/RotY/TransX/TransY are conjugated into the neighbouring tips.
 template <typename T>
 struct KConst {
-    using W = typename WideOf<T>::type;
     SinCosTab sincos;          // reduction constants and polynomial coefficients of sincos_wide
-    W base[12];
-    W tip[kMaxJ][12];
+    double base[12];           // the kinematic chain is carried in double in both modes (vfk_math.cuh)
+    double tip[kMaxJ][12];
     T q_lo[kMaxJ], q_hi[kMaxJ];
     T ns_q0_scale[kMaxJ];      // -k / (hi - lo)^2
     T ns_mid[kMaxJ];
@@ -88,7 +66,7 @@ struct KConst {
     T mixer_w[6];
     T tool[12];
     T ns_control[4];
-    typename WideNE<T>::type ik_lambda2, ns_lambda2;
+    T ik_lambda2, ns_lambda2;
     T dt, speed_scale, max_vel, jp_kp, jp_delta;
     T ns_gain, ns_lookahead, rot_slowdown_inv, goal_force, obst_force, obst_safe_inv, obst_order;
     int32_t prismatic_mask;    // bit j set: joint j is TransZ, else RotZ
@@ -198,18 +176,16 @@ struct DhPattern {
 };
 
 // ------------------------------------------------------------------------------ FK + J
-// T_{j+1} = T_j * RotZ(q_j) * tip_j, carried in the wide type W (double in both modes: an FP32 chain leaves ~1e-7 m in the
+// T_{j+1} = T_j * RotZ(q_j) * tip_j, carried in double in both modes (an FP32 chain leaves ~1e-7 m in the
 // tool position, which the order-20 repeller decay turns into 1e-4 relative field errors near obstacles).  Records the
 // joint axis z_j = R_j[:,2] and origin p_j before each joint, then forms J = [z x (p_e - p_j); z] (revolute) or [z; 0]
-// in T.  Outputs: R, and the tool-less flange position as hi + lo parts in T (lo = 0 when T is already wide).
-template <typename T, int N, class PAT, bool TAB = false>
-__device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N], typename WideOf<T>::type (&R)[9],
-                                            typename WideOf<T>::type (&p)[3], T (&Jl)[N][3], T (&Ja)[N][3], int nc,
-                                            [[maybe_unused]] const double2* sctab) {
-    using W = typename WideOf<T>::type;
+// in T.  Outputs: R, and the tool-less flange position as hi + lo parts in T (lo = 0 when T is double).
+template <typename T, int N, class PAT>
+__device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N], double (&R)[9], double (&p)[3], T (&Jl)[N][3],
+                                            T (&Ja)[N][3], int nc, [[maybe_unused]] const double2* sctab) {
     if constexpr (PAT::base_identity) {
 #pragma unroll
-        for (int k = 0; k < 9; ++k) R[k] = (k % 4 == 0) ? W(1) : W(0);
+        for (int k = 0; k < 9; ++k) R[k] = (k % 4 == 0) ? 1.0 : 0.0;
     } else {
 #pragma unroll
         for (int k = 0; k < 9; ++k) R[k] = c.base[k];
@@ -225,24 +201,21 @@ __device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N],
         }
         Ja[j][0] = (T)R[2]; Ja[j][1] = (T)R[5]; Ja[j][2] = (T)R[8];
         Jl[j][0] = (T)p[0]; Jl[j][1] = (T)p[1]; Jl[j][2] = (T)p[2];      // holds p_j until p_e is known
-        const W qj = (W)q[j];
+        const double qj = (double)q[j];
         if (PAT::generic && (c.prismatic_mask & (1 << j))) {
             p[0] = fma(R[2], qj, p[0]); p[1] = fma(R[5], qj, p[1]); p[2] = fma(R[8], qj, p[2]);
         } else {
-            W s, co;
-            // FP32 mode's wide chain: the quarter-angle form (no quadrant logic, ~10 instructions fewer per joint; measured on B200
-            // against sincos_wide<5>: K = 1 headline 109.5 vs 109.9 us, K = 100 +3.2 %, 17 joints +2.6 % / +3.3 %)
-            if constexpr (kTabBytes<T, TAB> != 0) sincos_table(c.sincos, sctab, qj, &s, &co);
-            else if constexpr (sizeof(T) == 4 && sizeof(W) == 8) sincos_quarter<5>(c.sincos, qj, &s, &co);
-            else sincos_wide<(sizeof(T) == sizeof(W)) ? 7 : 5>(c.sincos, qj, &s, &co);
+            double s, co;
+            if constexpr (kTabBytes<T> != 0) sincos_table(c.sincos, sctab, qj, &s, &co);
+            else sincos_wide(c.sincos, qj, &s, &co);
 #pragma unroll
             for (int r = 0; r < 3; ++r) {
-                const W a = R[3 * r + 0], b = R[3 * r + 1];
+                const double a = R[3 * r + 0], b = R[3 * r + 1];
                 R[3 * r + 0] = fma(co, a, s * b);
                 R[3 * r + 1] = fma(co, b, -s * a);
             }
         }
-        const W* tp = c.tip[j];
+        const double* tp = c.tip[j];
         static_for<0, 3>([&](auto kc) {
             constexpr int k = decltype(kc)::value;
             if constexpr (PAT::pnz(j, k)) {
@@ -251,26 +224,26 @@ __device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N],
             }
         });
         if constexpr (PAT::dh) {
-            const W ca = tp[4], sa = tp[7];
+            const double ca = tp[4], sa = tp[7];
 #pragma unroll
             for (int r = 0; r < 3; ++r) {
-                const W a = R[3 * r + 1], b = R[3 * r + 2];
+                const double a = R[3 * r + 1], b = R[3 * r + 2];
                 R[3 * r + 1] = fma(ca, a, sa * b);
                 R[3 * r + 2] = fma(ca, b, -sa * a);
             }
             return;
         }
-        W Rn[9];
+        double Rn[9];
         if constexpr (PAT::generic) {
             // warp-uniform choice on the robot's constants: identity tip (nothing), X-twist tip (12 ops), general (27)
             if (c.tipident_mask & (1 << j)) {
 #pragma unroll
                 for (int k = 0; k < 9; ++k) Rn[k] = R[k];
             } else if (c.xtwist_mask & (1 << j)) {
-                const W ca = tp[4], sa = tp[7];
+                const double ca = tp[4], sa = tp[7];
 #pragma unroll
                 for (int r = 0; r < 3; ++r) {
-                    const W a = R[3 * r + 1], b = R[3 * r + 2];
+                    const double a = R[3 * r + 1], b = R[3 * r + 2];
                     Rn[3 * r + 0] = R[3 * r + 0];
                     Rn[3 * r + 1] = fma(ca, a, sa * b);
                     Rn[3 * r + 2] = fma(ca, b, -sa * a);
@@ -294,7 +267,7 @@ __device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N],
         for (int k = 0; k < 9; ++k) R[k] = Rn[k];
     });
     const T pe[3] = {(T)p[0], (T)p[1], (T)p[2]};
-    const T pel[3] = {(T)(p[0] - (W)pe[0]), (T)(p[1] - (W)pe[1]), (T)(p[2] - (W)pe[2])};
+    const T pel[3] = {(T)(p[0] - (double)pe[0]), (T)(p[1] - (double)pe[1]), (T)(p[2] - (double)pe[2])};
     static_for<0, N>([&](auto jc) {
         constexpr int j = decltype(jc)::value;
         if (PAT::generic && (c.prismatic_mask & (1 << j))) {
@@ -310,7 +283,7 @@ __device__ __forceinline__ void fk_jacobian(const KConst<T>& c, const T (&q)[N],
 }
 
 // Tool position as a sum of two T values (hi + lo): differences against it are accurate to an ulp of the difference
-// even though T alone cannot represent the position to better than 6e-8 m.  lo is identically zero when T is wide.
+// even though T alone cannot represent the position to better than 6e-8 m.  lo is identically zero when T is double.
 template <typename T>
 struct Pos {
     T hi[3], lo[3];
@@ -321,7 +294,7 @@ struct Pos {
     }
     // x - position_k
     __device__ __forceinline__ T from(T x, int k) const {
-        if constexpr (sizeof(T) == sizeof(typename WideOf<T>::type)) return x - hi[k];
+        if constexpr (sizeof(T) == 8) return x - hi[k];
         else return (x - hi[k]) - lo[k];
     }
 };
@@ -579,7 +552,7 @@ __device__ __forceinline__ void issue_qg(const KArgs<T>& a, int64_t tile, int bu
 // small batches -- a warp takes 4 instances of a tile, the 8 lanes of a group split each chunk of 8 obstacles between
 // them and combine their partial repulsor sums with __shfl_xor_sync; the rest of the cycle is computed redundantly by
 // the group and lane 0 of the group stores.  A tile is then spread over 8 warps instead of one.
-template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool TAB = false>
+template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1>
 __global__ void __launch_bounds__(kBlock, MINB)
 vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a) {
     using WS = WarpStage<T, N, EXT>;
@@ -589,7 +562,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     // the bulk copies then live in uniform registers, and the copies issue without an elect-one loop around them
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem) + warp * WS::kBars;
-    unsigned char* region = smem + kSmemHeader + kTabBytes<T, TAB> + (size_t)warp * WS::warp_bytes(a.n_stages);
+    unsigned char* region = smem + kSmemHeader + kTabBytes<T> + (size_t)warp * WS::warp_bytes(a.n_stages);
     [[maybe_unused]] const double2* sctab = reinterpret_cast<const double2*>(smem + kSmemHeader);
     const uint32_t bars_a = smem_u32(bars), region_a = smem_u32(region);       // shared-window addresses, once per warp
     static_assert(G == 1 || G == kChunk, "a cooperative group takes one obstacle of a chunk per lane");
@@ -598,7 +571,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     const int64_t n_units = n_tiles * kSub;
     const int64_t stride = (int64_t)gridDim.x * (kBlock / 32);
     int64_t unit = (int64_t)blockIdx.x * (kBlock / 32) + warp;
-    if constexpr (kTabBytes<T, TAB> == 0) {
+    if constexpr (kTabBytes<T> == 0) {
         if (unit >= n_units) return;
     }
     const int ol = lane & (G - 1);                              // obstacle lane within the group
@@ -622,7 +595,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     __syncwarp();
     int64_t p_unit = unit;
     int p_u = 0, p_chunk = 0;
-    if (kTabBytes<T, TAB> == 0 || unit < n_units) {
+    if (kTabBytes<T> == 0 || unit < n_units) {
         issue_qg<T, N, EXT>(a, unit / kSub, 0, region_a, bars_a, lane, nc);
         for (int u = 0; u < S; ++u) {
             issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, u, region_a, bars_a, lane);
@@ -630,7 +603,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             if (++p_u == U) { p_u = 0; p_unit += stride; }
         }
     }
-    if constexpr (kTabBytes<T, TAB> != 0) {
+    if constexpr (kTabBytes<T> != 0) {
         // the sin / cos table is built behind the first tile's copies; the only CTA-wide barrier, passed once by every warp
         // (those without work included) before any can leave
         sincos_table_fill(c.sincos, reinterpret_cast<double2*>(smem + kSmemHeader), (int)threadIdx.x, kBlock);
@@ -657,14 +630,12 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         // tile's kinematic chain (~1.5 us) a third of what it gains here.  Blocks over 32 KB (M = 256) are left to the ring,
         // which is at the copy peak there; a launch of fewer than four tiles per warp is dominated by its start, where every
         // warp's demand copies are queued at once, and skips the prefetch on its first tile (FP64 config 2: -3 % otherwise).
-#ifndef VFK_NO_PREFETCH
         if constexpr (G == 1) {
             const int first = S * kChunk;
             const uint32_t bytes = a.n_obst_p > first ? (uint32_t)(a.n_obst_p - first) * 32u * (uint32_t)sizeof(Vec4<T>) : 0u;
             if (!resident && bytes != 0 && bytes <= 32768u && (it > 0 || n_units >= 4 * stride) && lane == 0)
                 bulk_prefetch_l2(a.obst + (tile * a.n_obst_p + first) * 32, bytes);
         }
-#endif
         mbar_wait_a(bars_a + 8u * (uint32_t)(kMaxStages + (it & 1)), (uint32_t)(it >> 1) & 1u);
         const T* qg = reinterpret_cast<const T*>(region + (size_t)a.n_stages * WS::kStage + (size_t)(it & 1) * WS::kQg) + slot;
 
@@ -686,13 +657,12 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         int flags = 0;
 
         // 1. FK, Jacobian, tool frame
-        using W = typename WideOf<T>::type;
         T Jl[N][3], Ja[N][3];
         T Rt[9], dp[3];
         Pos<T> pt;
         {
-            W Rw[9], pw[3];
-            fk_jacobian<T, N, PAT, TAB>(c, q, Rw, pw, Jl, Ja, nc, sctab);
+            double Rw[9], pw[3];
+            fk_jacobian<T, N, PAT>(c, q, Rw, pw, Jl, Ja, nc, sctab);
             if (LEAN || c.tool_identity) {
 #pragma unroll
                 for (int k = 0; k < 9; ++k) Rt[k] = (T)Rw[k];
@@ -700,15 +670,15 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
 #pragma unroll
                 for (int k = 0; k < 3; ++k) dp[k] = T(0);
             } else {
-                W ptw[3];
+                double ptw[3];
 #pragma unroll
                 for (int r = 0; r < 3; ++r) {
-                    const W off = fma(Rw[3 * r + 0], (W)c.tool[9], fma(Rw[3 * r + 1], (W)c.tool[10], Rw[3 * r + 2] * (W)c.tool[11]));
+                    const double off = fma(Rw[3 * r + 0], (double)c.tool[9], fma(Rw[3 * r + 1], (double)c.tool[10], Rw[3 * r + 2] * (double)c.tool[11]));
                     ptw[r] = pw[r] + off;
                     dp[r] = (T)(-off);
 #pragma unroll
                     for (int cc = 0; cc < 3; ++cc)
-                        Rt[3 * r + cc] = (T)fma(Rw[3 * r + 0], (W)c.tool[cc], fma(Rw[3 * r + 1], (W)c.tool[3 + cc], Rw[3 * r + 2] * (W)c.tool[6 + cc]));
+                        Rt[3 * r + cc] = (T)fma(Rw[3 * r + 0], (double)c.tool[cc], fma(Rw[3 * r + 1], (double)c.tool[3 + cc], Rw[3 * r + 2] * (double)c.tool[6 + cc]));
                 }
                 pt.set(ptw);
             }
@@ -753,7 +723,11 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                             for (int p = 0; p < kChunk / 2; ++p)
                                 repel2<decltype(order_c)::value>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
                         };
-                        if (kF32PowChain && c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
+                        // decay order 20 (the reference's typical value, old/README.old:75) by five multiplications instead of
+                        // MUFU lg2 / ex2: two more instructions per obstacle but two fewer on the quarter-rate XU pipe, which also
+                        // carries rsqrt and the FP64 <-> FP32 conversions.  Measured on B200 (1 M instances): 109.1 us vs 110.3 us
+                        // per launch at K = 1, -0.6 % at K = 100; also the more accurate of the two.
+                        if (c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
                         else full_chunk(std::integral_constant<int, 0>{});
                     } else {
                         for (int p = 0; p < (a.n_rem + 1) >> 1; ++p)
@@ -810,9 +784,8 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         }
 
         // 5. weighted damped least squares: qdot = Wj Jw^T (Jw Jw^T + l^2 I)^-1 Wt t.  The normal matrix, its Cholesky
-        // factor and the triangular solves are carried in W: formed in FP32, A's rounding error (~1e-6 absolute) is 1e-4
-        // of lambda^2 = 0.01 and lands directly in the joints' weakest direction.  J itself stays in T.
-        using WN = typename WideNE<T>::type;
+        // factor and the triangular solves are carried in T (FP32 here costs a smaller error tail than an FP32 chain:
+        // vfk_math.cuh, the working types' table).
         const bool unitw = LEAN || c.unit_weights;
         const bool ns_on = LEAN || c.ns_mode != 0;
         const bool ns_proj = LEAN || c.ns_mode == 1;
@@ -828,44 +801,44 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                 for (int j = 0; j < N; ++j) x[j] = c.ns_q0_scale[j] * (q[j] - c.ns_mid[j]);
             }
         }
-        WN A[21], invd[6], Jx[6];
+        T A[21], invd[6], Jx[6];
 #pragma unroll
         for (int r = 0; r < 6; ++r) {
-            Jx[r] = WN(0);
+            Jx[r] = T(0);
 #pragma unroll
-            for (int s = 0; s <= r; ++s) A[tri(r, s)] = (r == s) ? c.ik_lambda2 : WN(0);
+            for (int s = 0; s <= r; ++s) A[tri(r, s)] = (r == s) ? c.ik_lambda2 : T(0);
         }
         static_for<0, N>([&](auto jc) {
             constexpr int j = decltype(jc)::value;
-            WN col[6] = {(WN)Jl[j][0], (WN)Jl[j][1], (WN)Jl[j][2], (WN)Ja[j][0], (WN)Ja[j][1], (WN)Ja[j][2]};
+            T col[6] = {Jl[j][0], Jl[j][1], Jl[j][2], Ja[j][0], Ja[j][1], Ja[j][2]};
             // (the short-chain lean tail wants the projector's right-hand side negated: -J x, see dot6x2 there)
-            if (ns_proj && share) axpy6(Jx, col, kSlim ? (WN)x_slim(j) : ((LEAN && !kSlim) ? -(WN)x[j] : (WN)x[j]));
+            if (ns_proj && share) axpy6(Jx, col, kSlim ? x_slim(j) : ((LEAN && !kSlim) ? -x[j] : x[j]));
             if (!unitw) {
 #pragma unroll
-                for (int r = 0; r < 6; ++r) col[r] *= (WN)c.w_task[r] * (WN)c.w_joint[j];
+                for (int r = 0; r < 6; ++r) col[r] *= c.w_task[r] * c.w_joint[j];
             }
             syr6(A, col);
         });
         // FP64 accepts ik_lambda = 0 (the reference's undamped pinv): at a singular posture a pivot of J J^T is zero or, by
         // rounding, negative.  Flooring it relative to the trace keeps the factor finite (the step is then clamped like any
         // other); FP32 requires lambda > 0, whose pivots are >= lambda^2.
-        [[maybe_unused]] WN pivot_floor = WN(0);
-        if constexpr (sizeof(WN) == 8)
-            pivot_floor = WN(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + WN(1e-300);
-        chol6<WN>(A, invd, pivot_floor);
+        [[maybe_unused]] T pivot_floor = T(0);
+        if constexpr (sizeof(T) == 8)
+            pivot_floor = T(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + T(1e-300);
+        chol6<T>(A, invd, pivot_floor);
         T mix[N];
         [[maybe_unused]] T qd_vf[N], qd_ns[N], qd_jp[N];
         bool nan = false;
         if constexpr (kSlim) {
             T yv[6], yn[6];
             {
-                WN y[6];
+                T y[6];
 #pragma unroll
-                for (int r = 0; r < 6; ++r) y[r] = (WN)tw[r];
-                chol6_fwd<WN>(A, invd, y);                 // (chol6_solve2's register pairs cost ~150 moves at this register count)
-                chol6_bwd<WN>(A, invd, y);
-                chol6_fwd<WN>(A, invd, Jx);
-                chol6_bwd<WN>(A, invd, Jx);
+                for (int r = 0; r < 6; ++r) y[r] = tw[r];
+                chol6_fwd<T>(A, invd, y);                 // (chol6_solve2's register pairs cost ~150 moves at this register count)
+                chol6_bwd<T>(A, invd, y);
+                chol6_fwd<T>(A, invd, Jx);
+                chol6_bwd<T>(A, invd, Jx);
 #pragma unroll
                 for (int r = 0; r < 6; ++r) { yv[r] = (T)y[r]; yn[r] = (T)Jx[r]; }
             }
@@ -889,9 +862,9 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             // more output never changes a bit of qdot; measured: FP64 config 2 21.2 against 21.8 us per launch, FP32 unchanged.
             T yv[6], yn[6];
             {
-                WN y[6];
+                T y[6];
 #pragma unroll
-                for (int r = 0; r < 6; ++r) y[r] = (WN)tw[r];
+                for (int r = 0; r < 6; ++r) y[r] = tw[r];
                 chol6_solve2(A, invd, y, Jx);
 #pragma unroll
                 for (int r = 0; r < 6; ++r) { yv[r] = (T)y[r]; yn[r] = (T)Jx[r]; }        // Jx holds -(J x) here
@@ -911,14 +884,14 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             for (int j = 0; j < N; ++j) mix[j] = fma(raw[j] * gain, c.mixer_w[1], mix[j] * c.mixer_w[0]);
         } else {
             {
-                WN y[6];
+                T y[6];
     #pragma unroll
-                for (int r = 0; r < 6; ++r) y[r] = unitw ? (WN)tw[r] : (WN)tw[r] * (WN)c.w_task[r];
-                chol6_fwd<WN>(A, invd, y);
-                chol6_bwd<WN>(A, invd, y);
+                for (int r = 0; r < 6; ++r) y[r] = unitw ? tw[r] : tw[r] * c.w_task[r];
+                chol6_fwd<T>(A, invd, y);
+                chol6_bwd<T>(A, invd, y);
                 T yt[6];
     #pragma unroll
-                for (int r = 0; r < 6; ++r) yt[r] = unitw ? (T)y[r] : (T)(y[r] * (WN)c.w_task[r]);
+                for (int r = 0; r < 6; ++r) yt[r] = unitw ? (T)y[r] : (T)(y[r] * c.w_task[r]);
     #pragma unroll
                 for (int j = 0; j < N; ++j) {
                     const T cj[6] = {Jl[j][0], Jl[j][1], Jl[j][2], Ja[j][0], Ja[j][1], Ja[j][2]};
@@ -954,22 +927,22 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     if (!share) {                               // own damping or weighted IK: factor J J^T + ns_lambda^2 I
     #pragma unroll
                         for (int r = 0; r < 6; ++r) {
-                            Jx[r] = WN(0);
+                            Jx[r] = T(0);
     #pragma unroll
-                            for (int s = 0; s <= r; ++s) A[tri(r, s)] = (r == s) ? c.ns_lambda2 : WN(0);
+                            for (int s = 0; s <= r; ++s) A[tri(r, s)] = (r == s) ? c.ns_lambda2 : T(0);
                         }
                         static_for<0, N>([&](auto jc) {
                             constexpr int j = decltype(jc)::value;
-                            const WN col[6] = {(WN)Jl[j][0], (WN)Jl[j][1], (WN)Jl[j][2], (WN)Ja[j][0], (WN)Ja[j][1], (WN)Ja[j][2]};
-                            axpy6(Jx, col, (WN)x[j]);
+                            const T col[6] = {Jl[j][0], Jl[j][1], Jl[j][2], Ja[j][0], Ja[j][1], Ja[j][2]};
+                            axpy6(Jx, col, x[j]);
                             syr6(A, col);
                         });
-                        if constexpr (sizeof(WN) == 8)
-                            pivot_floor = WN(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + WN(1e-300);
-                        chol6<WN>(A, invd, pivot_floor);
+                        if constexpr (sizeof(T) == 8)
+                            pivot_floor = T(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + T(1e-300);
+                        chol6<T>(A, invd, pivot_floor);
                     }
-                    chol6_fwd<WN>(A, invd, Jx);
-                    chol6_bwd<WN>(A, invd, Jx);
+                    chol6_fwd<T>(A, invd, Jx);
+                    chol6_bwd<T>(A, invd, Jx);
                     T yt[6];
     #pragma unroll
                     for (int r = 0; r < 6; ++r) yt[r] = (T)Jx[r];

@@ -13,27 +13,18 @@ using namespace vfk;
 // obstacles x 32 instances) and two q/goal buffers.  Two stages measured best on B200 for both K = 1
 // (106 us vs 110 us with three at the headline shape) and K = 100 (streaming the ring from L2 every cycle at
 // full occupancy beats keeping four chunks resident at 2 CTAs/SM): gpurun_out t03, DESIGN.md section 4.1.
-template <typename T, int N, bool EXT, bool TAB>
-static void plan_stages(int n_obst, int k_cycles, int* n_chunks, int* n_stages, size_t* smem_bytes) {
+template <typename T, int N, bool EXT>
+static void plan_stages(int n_obst, int* n_chunks, int* n_stages, size_t* smem_bytes) {
     using WS = WarpStage<T, N, EXT>;
-    (void)k_cycles;
     *n_chunks = (n_obst + kChunk - 1) / kChunk;
     // long FP32 chains run 2 CTAs per SM on registers, so a third stage is free: config 5 0.684 -> 0.708 of the HBM roofline
     // (4: 0.697; 6 and 8 cost a resident CTA: 0.44); everywhere else a third stage costs occupancy (config 4: 1.009 -> 0.988)
     int stages = (sizeof(T) == 4 && N >= 10) ? 3 : 2;
-    if (const char* e = getenv("VFK_STAGES")) {
-        const int v = atoi(e);
-        if (v >= 1 && v <= kMaxStages) stages = v;
-    }
     if (*n_chunks > 0 && *n_chunks < stages) stages = *n_chunks;
     if (*n_chunks == 0) stages = 0;
     *n_stages = stages;
-    *smem_bytes = kSmemHeader + kTabBytes<T, TAB> + (size_t)(kBlock / 32) * WS::warp_bytes(stages);
+    *smem_bytes = kSmemHeader + kTabBytes<T> + (size_t)(kBlock / 32) * WS::warp_bytes(stages);
 }
-
-// Lanes per instance of the split shape for (precision, joints, pattern); 0 = the one-thread-per-instance kernel only.
-template <typename T, int N, class PAT>
-constexpr int kSplitLanes = (N >= 10 || (sizeof(T) == 8 && N == 7)) ? 2 : 0;
 
 // Launch plan of one kernel instantiation: resident CTAs per SM for a given dynamic shared-memory size, per device.  One
 // instance per instantiation (function-local static at the call site); a handful of (device, smem) entries behind a mutex, so
@@ -64,7 +55,7 @@ static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
     return c.tool_identity && c.unit_weights && c.share_factor && c.ik_mode == 0 && c.ns_mode == VFK_NS_PROJECTOR && !c.need_jp && !b->ns_in &&
            !c.shoulder_clamp &&
            !b->jp_ref && !b->jp_lo && !b->q_cmded && !b->ext_cmd[0] && !b->ext_cmd[1] && !b->ext_cmd[2] && !b->qdot_vf && !b->qdot_ns &&
-           !b->qdot_jp && !b->cmd && !b->pose && !b->twist && !b->flags && !(b->aux && b->n_aux > 0) && b->qdot && !getenv("VFK_NO_LEAN");
+           !b->qdot_jp && !b->cmd && !b->pose && !b->twist && !b->flags && !(b->aux && b->n_aux > 0) && b->qdot;
 }
 
 // HIOCC: the single-cycle lean FP32 launch asks for one more resident CTA per SM (4 x 128 threads at 128 registers, no
@@ -104,42 +95,12 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     a.n_obst_p = (n_obst + 1) & ~1;
     a.k_cycles = k_cycles;
     size_t smem = 0;
-    // sin / cos of the FP32 mode's wide chain from the shared-memory table (vfk_kernels.cuh: TAB) in EVERY instantiation of the
-    // throughput shape, so that K fused cycles stay bit-identical to K single-cycle launches.  Before the L2 prefetch of the
-    // obstacle block the HBM-bound single-cycle lean launch of the short chains lost 3.4 % with the table; with the prefetch
-    // it is unchanged (104.9 vs 104.7 us) and the K-fused launch gains 4.7 % (profiles/r02t_sincos_table_ab.txt).
-    // -DVFK_TAB_MIN_JOINTS=10 restricts the table to the long chains again.
-#ifndef VFK_TAB_MIN_JOINTS
-#define VFK_TAB_MIN_JOINTS 1
-#endif
-    constexpr bool TAB = kCanTab<T> && N >= VFK_TAB_MIN_JOINTS && G == 1;
-    plan_stages<T, N, EXT, TAB>(n_obst, k_cycles, &a.n_chunks, &a.n_stages, &smem);
+    plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
     a.n_full = n_obst / kChunk;
     a.n_rem = n_obst % kChunk;
-#ifndef VFK_MINB_F32
-#define VFK_MINB_F32 3
-#endif
-#ifndef VFK_MINB_LEAN
-#define VFK_MINB_LEAN 3
-#endif
-#ifndef VFK_MINB_F64
-#define VFK_MINB_F64 2
-#endif
-#ifndef VFK_MINB_LEAN_K1
-#define VFK_MINB_LEAN_K1 4
-#endif
-#ifndef VFK_MINB_LEAN_BIG
-#define VFK_MINB_LEAN_BIG 2
-#endif
-    constexpr int MINB0 = (HIOCC ? VFK_MINB_LEAN_K1
-                                 : ((sizeof(T) == 4) ? (N <= 10 ? (LEAN ? VFK_MINB_LEAN : VFK_MINB_F32) : (LEAN ? VFK_MINB_LEAN_BIG : 2))
-                                                     : (N <= 7 ? VFK_MINB_F64 : 1))) * (128 / kBlock);
-#ifdef VFK_MINB_LEAN_BIG_ABS          // experiment: resident CTAs of kBlock threads for the long-chain lean FP32 kernel, as given
-    constexpr int MINB = (sizeof(T) == 4 && N > 10 && LEAN) ? VFK_MINB_LEAN_BIG_ABS : MINB0;
-#else
-    constexpr int MINB = MINB0;
-#endif
-    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, TAB>;
+    // resident CTAs per SM that the register allocation aims for
+    constexpr int MINB = HIOCC ? 4 : (sizeof(T) == 4 ? (N <= 10 ? 3 : 2) : (N <= 7 ? 2 : 1));
+    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G>;
     // per (instantiation, device, smem size): opt in to > 48 KB of dynamic shared memory and ask the occupancy once
     static PlanCache plans;
     int per_sm = 0;
@@ -187,25 +148,25 @@ static int encode_map3(vfk_ctx* h, CUtensorMap* m, const void* base, uint64_t in
     return VFK_OK;
 }
 
+// The lane-split shape is instantiated for the FP64 17-joint kernel only: there the one-thread-per-instance kernel cannot
+// hold its Jacobian (102 doubles for 17 joints) and runs 1 CTA per SM with 568 B of spills, while two lanes per instance fit
+// 255 registers without spills at 2 CTAs per SM: 173 us against 217 us per launch (256 k x 17 joints x 64 obstacles, 0.60
+// against 0.48 of the HBM roofline).  Everywhere else it measured slower and was removed (FP32 config 5: 184 vs 154 us;
+// 10 joints: 98 vs 70 us in FP64, 95 vs 70 us in FP32; FP64 config 2: 29.6 vs 23.4 us; DESIGN.md section 4.2), and so were
+// four lanes per instance (231 us on the FP64 17-joint shape: every lane repeats the attractor, the Cholesky and the solves).
+template <typename T, int N>
+constexpr bool kSplit = sizeof(T) == 8 && N == 17;
+
 // May this call run in the lane-split shape?  Lean call on blocked device buffers, DH-form chain of exactly the instantiated
-// length.  Default: ON for the FP64 17-joint instantiation -- there the one-thread-per-instance kernel cannot hold its
-// Jacobian (102 doubles for 17 joints) and runs 1 CTA per SM with 568 B of spills, while two lanes per instance fit 255
-// registers without spills at 2 CTAs per SM: 173 us against 217 us per launch (256 k x 17 joints x 64 obstacles, 0.60 against
-// 0.48 of the HBM roofline).  OFF elsewhere, where it measured slower (FP32 config 5: 184 vs 154 us; 10 joints: 98 vs 70 us in
-// FP64, 95 vs 70 us in FP32; FP64 config 2: 29.6 vs
-// 23.4 us; DESIGN.md section 4.2).  Four lanes per instance (the kernel is written for L = 2 and 4) measured 231 us on the
-// FP64 17-joint shape: every lane repeats the attractor, the Cholesky and the solves.  VFK_SPLIT=1 / 0 forces the shape on
-// (where instantiated) / off.
+// length.  VFK_NO_SPLIT=1 runs the one-thread-per-instance kernel instead (the reference the tests compare against).
 template <typename T>
 static bool split_ok(vfk_ctx* h, int n_kernel, const KConst<T>& c, const vfk_buffers* b, const vfk_io* io) {
-    const char* e = getenv("VFK_SPLIT");
-    const bool on = e ? atoi(e) != 0 : (sizeof(T) == 8 && n_kernel == 17);
-    return on && h->dh_chain && h->chain.n_joints == n_kernel && is_lean<T>(c, b) && !(io && (io->q_src || io->qdot));
+    return !getenv("VFK_NO_SPLIT") && h->dh_chain && h->chain.n_joints == n_kernel && is_lean<T>(c, b) && !(io && (io->q_src || io->qdot));
 }
 
-template <typename T, int N, int L>
+template <typename T, int N>
 static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st) {
-    using SH = SplitShape<T, N, L>;
+    using SH = SplitShape<T, N>;
     KArgs<T> a;
     memset(&a, 0, sizeof a);
     a.q = static_cast<T*>(b->q);
@@ -218,14 +179,8 @@ static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     a.n_chunks = (n_obst + kChunk - 1) / kChunk;
     a.n_full = n_obst / kChunk;
     a.n_rem = n_obst % kChunk;
-    int stages = 2;
-    if (const char* e = getenv("VFK_STAGES")) {
-        const int v = atoi(e);
-        if (v >= 1 && v <= kMaxStages) stages = v;
-    }
-    if (a.n_chunks < stages) stages = a.n_chunks;
-    a.n_stages = stages;
-    const size_t smem = kSmemHeader + SH::kTab + (size_t)(kBlock / 32) * SH::warp_bytes(stages);
+    a.n_stages = a.n_chunks < 2 ? a.n_chunks : 2;
+    const size_t smem = kSmemHeader + SH::kTab + (size_t)(kBlock / 32) * SH::warp_bytes(a.n_stages);
     const uint64_t tiles = (uint64_t)((n + 31) / 32);
     SplitMaps maps;
     memset(&maps, 0, sizeof maps);
@@ -237,19 +192,12 @@ static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
         if ((rc = encode_map3<T>(h, &maps.obst, b->obst, 32 * 16 / sizeof(T), rows, tiles, SH::kRowBytes / sizeof(T), SH::kRowsPerChunk)) != VFK_OK)
             return rc;
     }
-#ifndef VFK_MINB_SPLIT_F32
-#define VFK_MINB_SPLIT_F32 4
-#endif
-#ifndef VFK_MINB_SPLIT_F64
-#define VFK_MINB_SPLIT_F64 2          // 255 registers: no spills for 17 joints (3 CTAs / 168 registers spill and measured equal to the solo kernel)
-#endif
-    constexpr int MINB = (sizeof(T) == 4 ? VFK_MINB_SPLIT_F32 : VFK_MINB_SPLIT_F64) * (128 / kBlock);
-    auto kern = vfk_split_kernel<T, N, L, MINB>;
+    auto kern = vfk_split_kernel<T, N>;
     static PlanCache plans;
     int per_sm = 0;
     VFK_CUDA(h, plans.get(kern, h->device, smem, &per_sm));
     if (per_sm < 1) return fail(h, VFK_ERR_CUDA, "split kernel does not fit an SM with %zu bytes of shared memory", smem);
-    const int64_t units = (n + 31) / 32 * L;
+    const int64_t units = (n + 31) / 32 * SH::L;
     const int64_t want = (units + kBlock / 32 - 1) / (kBlock / 32);
     const int64_t cap = (int64_t)h->sm_count * per_sm;
     const unsigned grid = (unsigned)(want < cap ? want : cap);
@@ -272,9 +220,9 @@ static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, i
                              : launch_cycle<T, N, PAT, false, false, kChunk>(h, c, b, n, n_obst, k_cycles, st, io);
     }
     if (ext) return launch_cycle<T, N, PAT, true, false>(h, c, b, n, n_obst, k_cycles, st, io);
-    // Two lanes per instance (vfk_split.cuh): default for the FP64 17-joint kernel, opt-in elsewhere.
-    if constexpr (kSplitLanes<T, N, PAT> > 0) {
-        if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N, kSplitLanes<T, N, PAT>>(h, c, b, n, n_obst, k_cycles, st);
+    // Two lanes per instance (vfk_split.cuh) for the FP64 17-joint kernel.
+    if constexpr (kSplit<T, N>) {
+        if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N>(h, c, b, n, n_obst, k_cycles, st);
     }
     if (is_lean<T>(c, b) && h->chain.n_joints == N) {
         if constexpr (sizeof(T) == 4 && N <= 7) {

@@ -2,20 +2,23 @@
 //
 // The one-thread-per-instance kernel (vfk_kernels.cuh) keeps the whole 6 x N Jacobian of its instance in registers.  For a
 // 17-joint chain that is 102 registers before anything else (248 in all: 2 CTAs per SM, 8 warps, latency-bound at 0.58 of
-// the HBM roofline), and in FP64 even 7 joints cost 234.  Here the JOINTS of an instance are split over L = 2 (or 4) lanes:
+// the HBM roofline), and in FP64 even 7 joints cost 234.  Here the JOINTS of an instance are split over L = 2 lanes:
 //
 //   * lane h of an instance owns joints [h * NL, (h + 1) * NL), NL = ceil(N / L): their angles, their Jacobian columns,
 //     their share of J J^T, J x and J^T y, their limits, their outputs -- a warp takes 32 / L instances of a tile;
-//   * forward kinematics runs as L partial chains in parallel, each from the identity (lane 0: from the base frame); the
-//     partial frames are combined by a shuffle scan (frame product is associative), which hands every lane the frame its
-//     partial chain starts from and all lanes the flange frame; joint axes and origins are then moved to the base frame;
+//   * forward kinematics runs as L partial chains in parallel, each from the identity (lane 0: from the base frame); one
+//     shuffle exchange of the partial frames hands lane 1 the frame its partial chain starts from and both lanes the
+//     flange frame; joint axes and origins are then moved to the base frame;
 //   * the 21 + 6 partial sums of J J^T and J x are added across the L lanes by xor-shuffles; the 6 x 6 Cholesky and the
 //     triangular solves are repeated by every lane (same instructions whether one lane or 32 execute them);
 //   * the obstacle pairs of a chunk are dealt round-robin to the L lanes and the three partial repulsor sums shuffled
 //     together (north_star's "reduced with warp shuffles"); the all-or-nothing limit check and the leading-joint clamp
 //     combine their per-lane verdicts the same way.
 //
-// Staging: a warp needs the rows of HALF (a quarter) of a tile -- 32 / L lanes of every 32-lane row.  Those are strided
+// The shape runs the FP64 17-joint chain only (vfk_launch.cuh: split_ok): every other chain and the FP32 mode measured
+// slower here than in the one-thread-per-instance kernel, and four lanes per instance slower than two (DESIGN.md 4.2).
+//
+// Staging: a warp needs the rows of HALF a tile -- 32 / L lanes of every 32-lane row.  Those are strided
 // pieces, so the 1-D bulk copies of the full-tile kernel would become one copy per row; instead the arrays are described to
 // the TMA unit as 3-D tensors [tile][row][lane] (cuTensorMapEncodeTiled on the host, one descriptor per array per launch)
 // and ONE cp.async.bulk.tensor (SASS UTMALDG) per stage gathers the box {32 / L lanes, rows of the chunk, 1 tile} into a
@@ -37,19 +40,21 @@ struct alignas(64) SplitMaps {
 };
 
 constexpr int kSplitTabJoints = kMaxJ + 3;       // L * NL can exceed N by up to L - 1 padding joints
+constexpr int kSplitLanes = 2;                   // L: lanes per instance
 
 // Per-joint constants of a DH chain: tip = {cos alpha, sin alpha, tx, ty, tz} (RotX(alpha) and the translation), limits and
 // the limit-avoidance gradient's scale / centre.  Padding joints (index >= N): identity tip, zeros.
 template <typename T>
 struct SplitTab {
-    typename WideOf<T>::type tip[kSplitTabJoints][6];
+    T tip[kSplitTabJoints][6];
     T lim[kSplitTabJoints][4];                   // q_lo, q_hi, ns_scale, ns_mid
 };
 
 __host__ __device__ constexpr uint32_t round128(uint32_t x) { return (x + 127u) & ~127u; }
 
-template <typename T, int N, int L>
+template <typename T, int N>
 struct SplitShape {
+    static constexpr int L = kSplitLanes;
     static constexpr int NL = (N + L - 1) / L;                                  // joints per lane
     static constexpr int SUB = 32 / L;                                          // instances per warp
     static constexpr uint32_t kRowBytes = SUB * 16;                             // one obstacle plane row of the warp's instances
@@ -72,8 +77,8 @@ __device__ __forceinline__ void tma_box3(void* dst_smem, const CUtensorMap* map,
         : "memory");
 }
 
-template <typename W>
-__device__ __forceinline__ void frame_mul(const W (&Ra)[9], const W (&pa)[3], const W (&Rb)[9], const W (&pb)[3], W (&R)[9], W (&p)[3]) {
+template <typename T>
+__device__ __forceinline__ void frame_mul(const T (&Ra)[9], const T (&pa)[3], const T (&Rb)[9], const T (&pb)[3], T (&R)[9], T (&p)[3]) {
 #pragma unroll
     for (int r = 0; r < 3; ++r) {
 #pragma unroll
@@ -83,13 +88,13 @@ __device__ __forceinline__ void frame_mul(const W (&Ra)[9], const W (&pa)[3], co
     }
 }
 
-template <typename T, int N, int L, int MINB>
-__global__ void __launch_bounds__(kBlock, MINB)
+// 2 resident CTAs per SM: 255 registers, no spills for 17 joints (3 CTAs / 168 registers spill and measured equal to the solo kernel)
+template <typename T, int N>
+__global__ void __launch_bounds__(kBlock, 2)
 vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a, const __grid_constant__ SplitMaps maps) {
-    using SH = SplitShape<T, N, L>;
-    using W = typename WideOf<T>::type;
-    using WN = typename WideNE<T>::type;
-    constexpr int NL = SH::NL, SUB = SH::SUB;
+    static_assert(sizeof(T) == 8, "the lane-split shape is FP64 only");
+    using SH = SplitShape<T, N>;
+    constexpr int L = SH::L, NL = SH::NL, SUB = SH::SUB;
     extern __shared__ __align__(128) unsigned char smem[];
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);     // tells the compiler it is warp-uniform: no divergence guards around the shuffles
@@ -104,19 +109,19 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     // per-joint robot constants -> shared memory
     for (int j = threadIdx.x; j < L * NL; j += kBlock) {
         const bool real = j < N;
-        tab->tip[j][0] = real ? c.tip[j][4] : W(1);
-        tab->tip[j][1] = real ? c.tip[j][7] : W(0);
-        tab->tip[j][2] = real ? c.tip[j][9] : W(0);
-        tab->tip[j][3] = real ? c.tip[j][10] : W(0);
-        tab->tip[j][4] = real ? c.tip[j][11] : W(0);
-        tab->tip[j][5] = W(0);
+        tab->tip[j][0] = real ? c.tip[j][4] : T(1);
+        tab->tip[j][1] = real ? c.tip[j][7] : T(0);
+        tab->tip[j][2] = real ? c.tip[j][9] : T(0);
+        tab->tip[j][3] = real ? c.tip[j][10] : T(0);
+        tab->tip[j][4] = real ? c.tip[j][11] : T(0);
+        tab->tip[j][5] = T(0);
         tab->lim[j][0] = real ? c.q_lo[j] : T(0);
         tab->lim[j][1] = real ? c.q_hi[j] : T(0);
         tab->lim[j][2] = real ? c.ns_q0_scale[j] : T(0);
         tab->lim[j][3] = real ? c.ns_mid[j] : T(0);
     }
     __syncthreads();
-    const typename WideOf<T>::type (*tipb)[6] = tab->tip + j0;   // this lane's joints: compile-time offsets from here on
+    const T (*tipb)[6] = tab->tip + j0;   // this lane's joints: compile-time offsets from here on
     const T (*limb)[4] = tab->lim + j0;
     // joint k of this lane exists unless it is one of the last lane's padding slots (N is not a multiple of L)
     auto real_joint = [&](int k) { return k < N - (L - 1) * NL || h != L - 1; };
@@ -192,24 +197,23 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             T Rt[9];
             Pos<T> pt;
             {
-                W R[9], p[3];
+                T R[9], p[3];
 #pragma unroll
-                for (int k = 0; k < 9; ++k) R[k] = (h == 0) ? c.base[k] : ((k % 4 == 0) ? W(1) : W(0));
+                for (int k = 0; k < 9; ++k) R[k] = (h == 0) ? c.base[k] : ((k % 4 == 0) ? T(1) : T(0));
 #pragma unroll
-                for (int k = 0; k < 3; ++k) p[k] = (h == 0) ? c.base[9 + k] : W(0);
+                for (int k = 0; k < 3; ++k) p[k] = (h == 0) ? c.base[9 + k] : T(0);
                 static_for<0, NL>([&](auto kc) {
                     constexpr int k = decltype(kc)::value;
                     Ja[k][0] = (T)R[2]; Ja[k][1] = (T)R[5]; Ja[k][2] = (T)R[8];
                     Jl[k][0] = (T)p[0]; Jl[k][1] = (T)p[1]; Jl[k][2] = (T)p[2];
-                    const W* tp = tipb[k];
-                    W s, co;
-                    if constexpr (sizeof(T) == 4 && sizeof(W) == 8) sincos_quarter<5>(c.sincos, (W)q[k], &s, &co);
-                    else sincos_wide<(sizeof(T) == sizeof(W)) ? 7 : 5>(c.sincos, (W)q[k], &s, &co);
-                    const W ca = tp[0], sa = tp[1], t0 = tp[2], t1 = tp[3], t2 = tp[4];
+                    const T* tp = tipb[k];
+                    T s, co;
+                    sincos_wide(c.sincos, q[k], &s, &co);
+                    const T ca = tp[0], sa = tp[1], t0 = tp[2], t1 = tp[3], t2 = tp[4];
 #pragma unroll
                     for (int r = 0; r < 3; ++r) {
-                        const W x0 = R[3 * r + 0], y0 = R[3 * r + 1], z0 = R[3 * r + 2];
-                        const W x = fma(co, x0, s * y0), y = fma(co, y0, -s * x0);            // RotZ(q)
+                        const T x0 = R[3 * r + 0], y0 = R[3 * r + 1], z0 = R[3 * r + 2];
+                        const T x = fma(co, x0, s * y0), y = fma(co, y0, -s * x0);            // RotZ(q)
                         p[r] = fma(x, t0, fma(y, t1, fma(z0, t2, p[r])));                     // tip translation
                         R[3 * r + 0] = x;
                         R[3 * r + 1] = fma(ca, y, sa * z0);                                   // tip rotation RotX(alpha)
@@ -217,58 +221,25 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     }
                 });
 
-                // Combine the partial frames.  Every lane needs the frame its part starts from (lane 0: none -- it began at the
-                // base) and all need the flange frame.
-                T Rs[9], ps[3];
-                W pe[3];
-                if constexpr (L == 2) {
-                    // one exchange: lane 0 holds X0 and receives X1, lane 1 the other way round; flange = X0 X1 on both
-                    W Ry[9], py[3];
+                // Combine the partial frames.  Lane 1 needs the frame its part starts from (lane 0 began at the base) and both
+                // need the flange frame.  One exchange: lane 0 holds X0 and receives X1, lane 1 the other way round; flange = X0 X1.
+                T Rs[9], ps[3], pe[3];
+                {
+                    T Ry[9], py[3];
 #pragma unroll
                     for (int k = 0; k < 9; ++k) Ry[k] = __shfl_xor_sync(0xffffffffu, R[k], SUB);
 #pragma unroll
                     for (int k = 0; k < 3; ++k) py[k] = __shfl_xor_sync(0xffffffffu, p[k], SUB);
-                    W Ra[9], pa[3], Rb[9], pb[3], Re[9];
+                    T Ra[9], pa[3], Rb[9], pb[3], Re[9];
 #pragma unroll
                     for (int k = 0; k < 9; ++k) { Ra[k] = h ? Ry[k] : R[k]; Rb[k] = h ? R[k] : Ry[k]; }
 #pragma unroll
                     for (int k = 0; k < 3; ++k) { pa[k] = h ? py[k] : p[k]; pb[k] = h ? p[k] : py[k]; }
-                    frame_mul<W>(Ra, pa, Rb, pb, Re, pe);
+                    frame_mul<T>(Ra, pa, Rb, pb, Re, pe);
 #pragma unroll
-                    for (int k = 0; k < 9; ++k) { Rt[k] = (T)Re[k]; Rs[k] = h ? (T)Ry[k] : ((k % 4 == 0) ? T(1) : T(0)); }
+                    for (int k = 0; k < 9; ++k) { Rt[k] = Re[k]; Rs[k] = h ? Ry[k] : ((k % 4 == 0) ? T(1) : T(0)); }
 #pragma unroll
-                    for (int k = 0; k < 3; ++k) ps[k] = h ? (T)py[k] : T(0);
-                } else {
-                    // inclusive scan P_h = X_0 ... X_h, then the exclusive prefix one lane up and the total from the last lane
-                    W Rx[9], px[3];
-#pragma unroll
-                    for (int d = 1; d < L; d <<= 1) {
-                        W Ry[9], py[3];
-#pragma unroll
-                        for (int k = 0; k < 9; ++k) Ry[k] = __shfl_up_sync(0xffffffffu, R[k], d * SUB);
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) py[k] = __shfl_up_sync(0xffffffffu, p[k], d * SUB);
-                        frame_mul<W>(Ry, py, R, p, Rx, px);
-                        const bool take = h >= d;
-#pragma unroll
-                        for (int k = 0; k < 9; ++k) R[k] = take ? Rx[k] : R[k];
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) p[k] = take ? px[k] : p[k];
-                    }
-#pragma unroll
-                    for (int k = 0; k < 9; ++k) {
-                        const W v = __shfl_up_sync(0xffffffffu, R[k], SUB);
-                        Rs[k] = (h == 0) ? ((k % 4 == 0) ? T(1) : T(0)) : (T)v;
-                    }
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        const W v = __shfl_up_sync(0xffffffffu, p[k], SUB);
-                        ps[k] = (h == 0) ? T(0) : (T)v;
-                    }
-#pragma unroll
-                    for (int k = 0; k < 9; ++k) Rt[k] = (T)__shfl_sync(0xffffffffu, R[k], (L - 1) * SUB + sl);
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) pe[k] = __shfl_sync(0xffffffffu, p[k], (L - 1) * SUB + sl);
+                    for (int k = 0; k < 3; ++k) ps[k] = h ? py[k] : T(0);
                 }
                 pt.set(pe);
                 // joint axes and origins to the base frame, then the Jacobian columns [z x (p_e - p_j); z]
@@ -297,57 +268,34 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             {
                 T V[3], S0, w[3], acc[3] = {T(0), T(0), T(0)};
                 attract<T>(c, g, Rt, pt, V, S0, w);
-                [[maybe_unused]] NegPos2 np2;
-                [[maybe_unused]] float2 acc2[3] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
-                if constexpr (sizeof(T) == 4) np2.set(pt);
                 for (int ch = 0; ch < a.n_chunks; ++ch) {
                     const int stage = resident ? ch : c_stage;
                     mbar_wait(&bars[stage], resident ? (uint32_t)(it & 1) : c_phase);
                     const unsigned char* sb = region + (size_t)stage * SH::kStage;
                     const int n_here = ch < a.n_full ? kChunk : a.n_rem;
                     const int n_pairs = (n_here + 1) >> 1;
-                    if constexpr (sizeof(T) == 4) {
-                        // stage = [pair][plane][SUB lanes] of float4; the pairs of the chunk are dealt round-robin to the lanes
-                        const float4* pl = reinterpret_cast<const float4*>(sb) + sl;
-                        auto deal = [&](auto order_c, auto full_c) {
+                    // stage = [pair][4 planes][SUB lanes] of double2 {slot 0, slot 1}
+                    const double2* pl = reinterpret_cast<const double2*>(sb) + sl;
+                    auto deal = [&](auto order_c) {
+                        constexpr int ORD = decltype(order_c)::value;
+                        const bool full = ch < a.n_full;
 #pragma unroll
-                            for (int i = 0; i < (kChunk / 2 + L - 1) / L; ++i) {
-                                const int pr = i * L + h;
-                                if (decltype(full_c)::value || pr < n_pairs)
-                                    repel2<decltype(order_c)::value>(pl[(2 * pr) * SUB], pl[(2 * pr + 1) * SUB], c.obst_safe_inv, c.obst_order, np2, acc2);
+                        for (int i = 0; i < (kChunk / 2 + L - 1) / L; ++i) {
+                            const int pr = i * L + h;
+                            if (full || pr < n_pairs) {
+                                const double2 X = pl[(4 * pr) * SUB], Y = pl[(4 * pr + 1) * SUB], Z = pl[(4 * pr + 2) * SUB], Rr = pl[(4 * pr + 3) * SUB];
+                                Vec4<T> o0, o1;
+                                o0.x = X.x; o0.y = Y.x; o0.z = Z.x; o0.w = Rr.x;
+                                o1.x = X.y; o1.y = Y.y; o1.z = Z.y; o1.w = Rr.y;
+                                repel<T, ORD>(o0, c.obst_safe_inv, c.obst_order, pt, acc);
+                                repel<T, ORD>(o1, c.obst_safe_inv, c.obst_order, pt, acc);       // zero radius in a padding slot: adds 0
                             }
-                        };
-                        static_assert((kChunk / 2) % L == 0, "a full chunk deals the same number of pairs to every lane");
-                        if (ch < a.n_full) {
-                            if (kF32PowChain && c.order_int == 20) deal(std::integral_constant<int, 20>{}, std::true_type{});
-                            else deal(std::integral_constant<int, 0>{}, std::true_type{});
-                        } else {
-                            deal(std::integral_constant<int, 0>{}, std::false_type{});
                         }
-                    } else {
-                        // stage = [pair][4 planes][SUB lanes] of double2 {slot 0, slot 1}
-                        const double2* pl = reinterpret_cast<const double2*>(sb) + sl;
-                        auto deal = [&](auto order_c) {
-                            constexpr int ORD = decltype(order_c)::value;
-                            const bool full = ch < a.n_full;
-#pragma unroll
-                            for (int i = 0; i < (kChunk / 2 + L - 1) / L; ++i) {
-                                const int pr = i * L + h;
-                                if (full || pr < n_pairs) {
-                                    const double2 X = pl[(4 * pr) * SUB], Y = pl[(4 * pr + 1) * SUB], Z = pl[(4 * pr + 2) * SUB], Rr = pl[(4 * pr + 3) * SUB];
-                                    Vec4<T> o0, o1;
-                                    o0.x = X.x; o0.y = Y.x; o0.z = Z.x; o0.w = Rr.x;
-                                    o1.x = X.y; o1.y = Y.y; o1.z = Z.y; o1.w = Rr.y;
-                                    repel<T, ORD>(o0, c.obst_safe_inv, c.obst_order, pt, acc);
-                                    repel<T, ORD>(o1, c.obst_safe_inv, c.obst_order, pt, acc);       // zero radius in a padding slot: adds 0
-                                }
-                            }
-                        };
-                        if (c.order_int == 20) deal(std::integral_constant<int, 20>{});
-                        else if (c.order_int == 5) deal(std::integral_constant<int, 5>{});
-                        else if (c.order_int == 2) deal(std::integral_constant<int, 2>{});
-                        else deal(std::integral_constant<int, 0>{});
-                    }
+                    };
+                    if (c.order_int == 20) deal(std::integral_constant<int, 20>{});
+                    else if (c.order_int == 5) deal(std::integral_constant<int, 5>{});
+                    else if (c.order_int == 2) deal(std::integral_constant<int, 2>{});
+                    else deal(std::integral_constant<int, 0>{});
                     if (!resident || last) {
                         __syncwarp();
                         if (p_unit < n_units) issue_obst(p_unit, p_chunk, stage);
@@ -355,10 +303,6 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                         if (++p_u == U) { p_u = 0; p_unit += stride; }
                     }
                     if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
-                }
-                if constexpr (sizeof(T) == 4) {
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) acc[k] = acc2[k].x + acc2[k].y;
                 }
 #pragma unroll
                 for (int off = SUB; off < 32; off <<= 1) {
@@ -375,17 +319,17 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             T x[NL];
 #pragma unroll
             for (int k = 0; k < NL; ++k) x[k] = limb[k][2] * (q[k] - limb[k][3]);
-            WN A[21], invd[6], Jx[6];
+            T A[21], invd[6], Jx[6];
 #pragma unroll
             for (int r = 0; r < 6; ++r) {
-                Jx[r] = WN(0);
+                Jx[r] = T(0);
 #pragma unroll
-                for (int s = 0; s <= r; ++s) A[tri(r, s)] = WN(0);
+                for (int s = 0; s <= r; ++s) A[tri(r, s)] = T(0);
             }
             static_for<0, NL>([&](auto kc) {
                 constexpr int k = decltype(kc)::value;
-                const WN col[6] = {(WN)Jl[k][0], (WN)Jl[k][1], (WN)Jl[k][2], (WN)Ja[k][0], (WN)Ja[k][1], (WN)Ja[k][2]};
-                axpy6(Jx, col, (WN)x[k]);
+                const T col[6] = {Jl[k][0], Jl[k][1], Jl[k][2], Ja[k][0], Ja[k][1], Ja[k][2]};
+                axpy6(Jx, col, x[k]);
                 syr6(A, col);
             });
 #pragma unroll
@@ -397,21 +341,20 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             }
 #pragma unroll
             for (int r = 0; r < 6; ++r) A[tri(r, r)] += c.ik_lambda2;
-            [[maybe_unused]] WN pivot_floor = WN(0);                  // see vfk_cycle_kernel: FP64 accepts ik_lambda = 0
-            if constexpr (sizeof(WN) == 8)
-                pivot_floor = WN(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + WN(1e-300);
-            chol6<WN>(A, invd, pivot_floor);
+            // see vfk_cycle_kernel: FP64 accepts ik_lambda = 0
+            const T pivot_floor = T(1e-28) * (A[tri(0, 0)] + A[tri(1, 1)] + A[tri(2, 2)] + A[tri(3, 3)] + A[tri(4, 4)] + A[tri(5, 5)]) + T(1e-300);
+            chol6<T>(A, invd, pivot_floor);
             T yv[6], yn[6];
             {
-                WN y[6];
+                T y[6];
 #pragma unroll
-                for (int r = 0; r < 6; ++r) y[r] = (WN)tw[r];
-                chol6_fwd<WN>(A, invd, y);
-                chol6_bwd<WN>(A, invd, y);
-                chol6_fwd<WN>(A, invd, Jx);
-                chol6_bwd<WN>(A, invd, Jx);
+                for (int r = 0; r < 6; ++r) y[r] = tw[r];
+                chol6_fwd<T>(A, invd, y);
+                chol6_bwd<T>(A, invd, y);
+                chol6_fwd<T>(A, invd, Jx);
+                chol6_bwd<T>(A, invd, Jx);
 #pragma unroll
-                for (int r = 0; r < 6; ++r) { yv[r] = (T)y[r]; yn[r] = (T)Jx[r]; }
+                for (int r = 0; r < 6; ++r) { yv[r] = y[r]; yn[r] = Jx[r]; }
             }
 
             // 6. nullspace projector on the limit-avoidance gradient, all-or-nothing lookahead check over ALL joints; 8-9. mixer, clamp
@@ -443,7 +386,7 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             for (int off = SUB; off < 32; off <<= 1) lead = Prec<T>::fmax_(lead, __shfl_xor_sync(0xffffffffu, lead, off));
             T ratio = T(1);
             if (lead > c.max_vel) ratio = Prec<T>::div(c.max_vel, lead);
-            if constexpr (sizeof(T) == 8) {                          // never integrate a non-finite step
+            {                                                        // never integrate a non-finite step
                 T z = T(0);
 #pragma unroll
                 for (int k = 0; k < NL; ++k) z = fma(mix[k], T(0), z);
