@@ -117,9 +117,10 @@ typedef struct vfk_chain_desc {
 /* Per-robot constants (uniform over the batch; kept in constant memory). */
 typedef struct vfk_params {
     double ik_lambda;            /* damping of J^T (J J^T + lambda^2 I)^-1           (getIKV, scripts/vf:461) */
-    double ns_lambda;            /* damping of the projector's pseudo-inverse (VFK_NS_PROJECTOR); 0 = the reference's pinv
-                                    (scripts/nullspace:78), computed through a Householder basis of null(J) (error cond(J)*eps,
-                                    valid in both precisions).  FP32 mode needs ik_lambda > 0: the undamped normal equations
+    double ns_lambda;            /* damping of the projector's pseudo-inverse (VFK_NS_PROJECTOR); 0 = the reference's
+                                    I - pinv(J) J (scripts/nullspace:78), computed through a one-sided Jacobi SVD of J with
+                                    pinv's cutoff, so it projects onto all of null(J) where J loses rank (error cond(J)*eps;
+                                    FP32 cuts singular values below 1e-6 sigma_max, see vfk_nullspace.cuh).  FP32 mode needs ik_lambda > 0: the undamped normal equations
                                     of the velocity IK lose their pivots to FP32 rounding near singular postures */
     double dt;                   /* config.rate (scripts/bridge:91) */
     double speed_scale;          /* speedScale (scripts/vf:137,197-207) */

@@ -248,3 +248,55 @@ def near_obstacles(chain, n, n_obst, seed, dtype=np.float64, obst_ext=True, safe
     if obst_ext:
         w["obst_ext"] = ext.astype(dtype)
     return w, dict(slot=slot, d=dist)
+
+
+# ---------------------------------------------------------------------------------------------- batches near singular postures
+SINGULAR_LEVELS = (0.0, 1e-12, 1e-9, 1e-6, 1e-3, 1e-1)
+
+
+def singular_values(chain, q):
+    """Singular values [I, 6] (descending) of the oracle's Jacobian at q [N, I] (dense GPU layout), in FP64."""
+    from oracle import batch
+    J = batch.fk_jac(chain, np.asarray(q, dtype=np.float64).T)[2]
+    return np.linalg.svd(J, compute_uv=False)
+
+
+def near_singular(chain, n, n_obst, seed, dtype=np.float64, kind="home", levels=SINGULAR_LEVELS, **kw):
+    """``workloads.random_batch`` with every posture moved next to a kinematic singularity, where J loses rank.
+
+    Base postures: ``home`` is q = 0, rank-deficient on every chain of the suite (LWR: rank 3; torso_arm_chain: 4;
+    dual_arm_torso_chain: 5, generic form 4); ``elbow`` (the 7-joint LWR) keeps random_batch's q with the elbow straight,
+    q[3] = 0 (rank 5).  The base posture is asserted singular through the oracle's Jacobian: sigma_min / sigma_max < 1e-15.
+    Each instance then moves by one of ``levels`` (delta, each drawn about equally often): ``home`` along a random unit
+    direction of joint space, ``elbow`` by q[3] = +-delta only.  q is rounded to ``dtype`` (delta = 0 stays exactly singular
+    in FP32 too) and stays inside the chain's limits.  Returns (w, meta): meta = dict(delta [I], sigma [I, 6] and cond [I]
+    = sigma_max / sigma_min, both of the oracle's Jacobian at q as rounded)."""
+    from vfclik_b200 import workloads
+    w = workloads.random_batch(chain, n, n_obst, seed, dtype=dtype, **kw)
+    rng = np.random.default_rng(seed + 15485863)
+    N = w["q"].shape[0]
+    if kind == "home":
+        base = np.zeros((N, n))
+    elif kind == "elbow":
+        assert N == 7, "the elbow singularity is the 7-joint LWR's"
+        base = w["q"].astype(np.float64).copy()
+        base[3] = 0.0
+    else:
+        raise ValueError(kind)
+    s0 = singular_values(chain, base)
+    assert np.all(s0[:, -1] <= 1e-15 * s0[:, 0]), "base posture is not singular"
+    lv = np.asarray(levels, dtype=np.float64)
+    delta = lv[np.concatenate([rng.permutation(len(lv)) for _ in range(-(-n // len(lv)))])[:n]]
+    if kind == "home":
+        u = rng.normal(size=(N, n))
+        step = u / np.linalg.norm(u, axis=0, keepdims=True)
+    else:
+        step = np.zeros((N, n))
+        step[3] = rng.choice((-1.0, 1.0), size=n)
+    q = (base + delta[None, :] * step).astype(dtype)
+    assert np.all(q >= chain.q_lo[:, None]) and np.all(q <= chain.q_hi[:, None])
+    w["q"] = q
+    sigma = singular_values(chain, q)
+    with np.errstate(divide="ignore"):
+        cond = sigma[:, 0] / sigma[:, -1]
+    return w, dict(delta=delta, sigma=sigma, cond=cond)

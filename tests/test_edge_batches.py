@@ -1,11 +1,11 @@
-"""The batch constructors of tests/helpers.py that put goals and obstacles next to the tool (CPU only): through the oracle's
-FK the requested distances and angles come out as asked, every combination is drawn, and FP32 batches stay clear of the
-repeller-weight saturation."""
+"""The batch constructors of tests/helpers.py that put goals and obstacles next to the tool, and postures next to kinematic
+singularities (CPU only): through the oracle's FK the requested distances and angles come out as asked, every combination
+is drawn, FP32 batches stay clear of the repeller-weight saturation, and singular postures have the chain's known rank."""
 import numpy as np
 import pytest
 
 import helpers
-from helpers import near_goal, near_obstacles, tool_frame
+from helpers import near_goal, near_obstacles, near_singular, tool_frame
 
 
 def _chains(lwr):
@@ -72,3 +72,53 @@ def test_near_obstacles_fp32_weights_stay_below_saturation(lwr, ext, safe, order
         assert np.all(wgt <= 1.5 * helpers.FP32_WEIGHT_LIMIT)
         if ext:
             assert np.any(wgt > 1e10)                              # still steep: the bound lowers orders only where needed
+
+
+def _singular_cases():
+    return [("lwr", "home"), ("lwr", "elbow"), ("tool10", "home"), ("dh17", "home"), ("generic17", "home")]
+
+
+@pytest.mark.parametrize("which,kind", _singular_cases())
+@pytest.mark.parametrize("dtype", [np.float64, np.float32])
+def test_near_singular_levels_rank_and_limits(lwr, which, kind, dtype):
+    """near_singular: every level is drawn; at delta = 0 the oracle's Jacobian has the chain's known rank (numpy's pinv cutoff,
+    1e-15 sigma_max); sigma_min / sigma_max grows linearly with delta (all these singularities are first order: within a
+    factor of the median over the batch at every level); q stays inside the limits and in the requested dtype; elbow moves
+    q[3] only."""
+    from vfclik_b200 import workloads
+    chain = {"lwr": lambda: lwr[0], "tool10": lambda: workloads.torso_arm_chain(10),
+             "dh17": lambda: workloads.dual_arm_torso_chain(17),
+             "generic17": lambda: workloads.dual_arm_torso_chain(17, dh=False)}[which]()
+    rank0 = {("lwr", "home"): 3, ("lwr", "elbow"): 5, ("tool10", "home"): 4, ("dh17", "home"): 5, ("generic17", "home"): 4}
+    n = 1200
+    w, meta = near_singular(chain, n, 4, seed=8, dtype=dtype, kind=kind)
+    q = w["q"]
+    assert q.dtype == dtype and q.shape == (len(chain.q_lo), n)
+    assert np.all(q >= chain.q_lo[:, None]) and np.all(q <= chain.q_hi[:, None])
+    assert set(meta["delta"]) == set(helpers.SINGULAR_LEVELS)
+    counts = np.array([np.count_nonzero(meta["delta"] == d) for d in helpers.SINGULAR_LEVELS])
+    assert counts.max() - counts.min() <= 1
+    sigma = meta["sigma"]
+    assert np.array_equal(sigma, helpers.singular_values(chain, q))
+    rel = sigma / sigma[:, :1]
+    at0 = meta["delta"] == 0
+    assert np.all(np.count_nonzero(rel[at0] > 1e-15, axis=1) == rank0[(which, kind)])
+    assert np.all(np.isinf(meta["cond"][at0]) | (meta["cond"][at0] > 1e15))
+    if kind == "home":
+        assert np.all(q[:, at0] == 0)
+    else:
+        ref = workloads.random_batch(chain, n, 4, seed=8, dtype=dtype)["q"]
+        assert np.all(q[3, at0] == 0)
+        assert np.array_equal(np.delete(q, 3, axis=0), np.delete(ref, 3, axis=0))
+        assert np.array_equal(np.abs(q[3]).astype(np.float64), meta["delta"].astype(dtype).astype(np.float64))
+    # first order: sigma_min / sigma_max / delta stays within a factor of its median, at every level from 1e-12 to 1e-1
+    smin = rel[:, -1]
+    med = {}
+    for d in helpers.SINGULAR_LEVELS[1:]:
+        at = meta["delta"] == d
+        med[d] = np.median(smin[at] / d)
+        assert np.all(smin[at] > 0)
+        assert np.quantile(smin[at] / d, 0.05) > med[d] / 100
+        assert np.all(smin[at] / d < 30 * med[d])
+    ratios = np.array(list(med.values()))
+    assert ratios.max() / ratios.min() < 10

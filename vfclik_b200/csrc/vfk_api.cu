@@ -126,8 +126,9 @@ static void build_const(const vfk_ctx& h, KConst<T>& c) {
     c.shoulder_neg = (T)p.shoulder_vel[1];
     c.integrate = p.integrate ? 1 : 0;
     c.unit_weights = unit ? 1 : 0;
-    // the reference's nullspace (control interface) and the undamped projector go through the Householder basis of
-    // null(J) (vfk_nullspace.cuh): no normal equations, so no cond(J)^2 and no pivot to lose at ns_lambda = 0
+    // the reference's nullspace (control interface: Householder basis of null(J)) and the undamped projector (one-sided
+    // Jacobi SVD of J, rank-revealing) skip the normal equations (vfk_nullspace.cuh): no cond(J)^2, no pivot to lose at
+    // ns_lambda = 0
     c.ns_qr = (p.ns_mode == VFK_NS_CONTROL || (p.ns_mode == VFK_NS_PROJECTOR && p.ns_lambda == 0.0)) ? 1 : 0;
     c.share_factor = (unit && p.ns_lambda == p.ik_lambda && !c.ns_qr) ? 1 : 0;
     c.ik_mode = p.ik_mode;

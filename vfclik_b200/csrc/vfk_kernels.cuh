@@ -952,26 +952,32 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                         raw[j] = dot6(cj, yt, x[j], true);
                     }
                 } else {
-                    // the reference's own form (scripts/nullspace:75-117): orthonormal basis u_i of null(J) -- Householder QR of
-                    // J^T, error cond(J) * eps, no damping (vfk_nullspace.cuh) -- then either the projector
-                    // (I - pinv(J) J) x = sum_i u_i (u_i . x), or the control interface sum_{i < min(4, k)} control_i u_i with
-                    // every u_i's sign kept continuous against the previous cycle's vector (ns_lastvec, [min(4, k)][N]).
+                    // the reference's own forms (scripts/nullspace:75-117), undamped (vfk_nullspace.cuh): the projector
+                    // (I - pinv(J) J) x through a one-sided Jacobi SVD of J, rank-revealing with pinv's cutoff; or the control
+                    // interface sum_{i < min(4, k)} control_i u_i over an orthonormal basis u_i of null(J) from a Householder
+                    // QR of J^T, every u_i's sign kept continuous against the previous cycle's vector (ns_lastvec, [min(4, k)][N]).
     #pragma unroll
                     for (int j = 0; j < N; ++j) raw[j] = T(0);
                     if constexpr (!LEAN && ns_null_vectors(N) > 0) {
-                        double At[N * 6], tau[6], wv[N];
-    #pragma unroll
-                        for (int j = 0; j < N; ++j)
-    #pragma unroll
-                            for (int r = 0; r < 6; ++r) At[j * 6 + r] = (double)(r < 3 ? Jl[j][r] : Ja[j][r - 3]);
-                        ns_qr_factor(At, nc, tau);
                         if (ns_proj) {
+                            double g[6 * N], wv[N];
     #pragma unroll
-                            for (int j = 0; j < N; ++j) wv[j] = (double)x[j];
-                            ns_qr_project(At, tau, nc, wv);
+                            for (int j = 0; j < N; ++j) {
+                                wv[j] = (double)x[j];
+    #pragma unroll
+                                for (int r = 0; r < 6; ++r)
+                                    if (j < nc) g[r * nc + j] = (double)(r < 3 ? Jl[j][r] : Ja[j][r - 3]);
+                            }
+                            ns_svd_project(g, nc, sizeof(T) == 8 ? kNsCutF64 : kNsCutF32, wv);
     #pragma unroll
                             for (int j = 0; j < N; ++j) raw[j] = j < nc ? (T)wv[j] : T(0);
                         } else {
+                            double At[N * 6], tau[6], wv[N];
+    #pragma unroll
+                            for (int j = 0; j < N; ++j)
+    #pragma unroll
+                                for (int r = 0; r < 6; ++r) At[j * 6 + r] = (double)(r < 3 ? Jl[j][r] : Ja[j][r - 3]);
+                            ns_qr_factor(At, nc, tau);
                             const int kk = ns_ctrl_vectors(nc);                      // rows of ns_lastvec
                             double rawd[N];
     #pragma unroll

@@ -1,5 +1,5 @@
-// vfk_nullspace.cuh -- rare-path dense linear algebra: orthonormal basis of null(J) for the reference's nullspace interface
-// (Householder QR), and the truncated velocity IK (one-sided Jacobi SVD) at the end of the file.
+// vfk_nullspace.cuh -- rare-path dense linear algebra: orthonormal basis of null(J) for the reference's nullspace control
+// interface (Householder QR), and a one-sided Jacobi SVD shared by the undamped projector and the truncated velocity IK.
 //
 // scripts/nullspace:75-107 builds B = I - pinv(J) J (LAPACK SVD) and takes the left singular vectors of B^T whose
 // singular value is >= 1e-8: an orthonormal basis of null(J), k = N - rank(J) vectors.  Forming B through the normal
@@ -8,11 +8,15 @@
 // i.e. they span null(J) (exactly N - 6 of them when J has full row rank; at a rank-deficient posture they are still
 // null vectors, the reference would find one more).  The reflectors follow LAPACK's dgeqr2 / dlarfg convention
 // (beta = -sign(alpha) |x|, v_0 = 1, H = I - tau v v^T), so numpy.linalg.qr(J.T, mode="complete") gives the same
-// vectors up to rounding -- that is what oracle/batch.py:ns_basis pins this against.  The projector needs no basis at
-// all: (I - pinv(J) J) x = Q diag(0, .., 0, 1, .., 1) Q^T x.
+// vectors up to rounding -- that is what oracle/batch.py:ns_basis pins this against.
 //
-// Rare path (control mode / undamped projector), any N <= 17: rolled loops over thread-local arrays, compiled once per
-// translation unit and called -- it costs the throughput instantiations neither registers nor instruction-cache lines.
+// The projector (I - pinv(J) J) x does not use that basis: Q diag(0, .., 0, 1, .., 1) Q^T x projects onto N - 6
+// dimensions, and at a posture where J loses rank (rank r < 6) null(J) has N - r.  It goes through the singular values
+// instead (ns_svd_project): rank-revealing, with the cutoff of numpy's pinv that the reference calls.
+//
+// Rare path (control mode / undamped projector / truncated IK), any N <= 17: rolled loops over thread-local arrays,
+// compiled once per translation unit and called -- it costs the throughput instantiations neither registers nor
+// instruction-cache lines.
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -60,20 +64,11 @@ static __device__ __noinline__ void ns_qr_column(const double* a, const double* 
     for (int j = 5; j >= 0; --j) ns_reflect(a, tau[j], j, n, w);
 }
 
-// w <- (I - pinv(J) J) w = Q diag(0 x 6, 1 ...) Q^T w: the orthogonal projector onto null(J), without forming a basis.
-static __device__ __noinline__ void ns_qr_project(const double* a, const double* tau, int n, double* w) {
-    for (int j = 0; j < 6; ++j) ns_reflect(a, tau[j], j, n, w);          // Q^T w = H_5 ( ... (H_0 w))
-    for (int r = 0; r < 6 && r < n; ++r) w[r] = 0.0;
-    for (int j = 5; j >= 0; --j) ns_reflect(a, tau[j], j, n, w);
-}
-
-// ---- truncated weighted least squares (VFK_IK_TRUNCATED), same rare-path style.
-// g: Jw = Wt J Wj, 6 x n row-major (g[r * n + j]); y: Wt t (6).  One-sided Jacobi (Hestenes): plane rotations of row pairs
-// until the rows are mutually orthogonal -- G' = U^T Jw = Sigma V^T, the same rotations applied to y give U^T y -- which
-// resolves every singular value to relative accuracy (no squaring of the condition number).  Then
-//   qd = V diag(f(sigma)) U^T y = sum_i row_i * c_i * (U^T y)_i,  c_i = 1 / sigma_i^2 (sigma_i >= eps), 1 / (sigma_i^2 + lambda^2) below.
-// qd: n values (before the joint weights).  Restated by oracle/batch.py:ikv_dls (ik_mode 1) through numpy's SVD.
-static __device__ __noinline__ void ik_truncated(double* g, int n, double* y, double lambda2, double eps, double* qd) {
+// ---- one-sided Jacobi SVD (Hestenes), same rare-path style.
+// g: 6 x n row-major (g[r * n + j]).  Plane rotations of row pairs until the rows are mutually orthogonal: on return
+// g = U^T G = Sigma V^T, row i being sigma_i v_i^T, which resolves every singular value to relative accuracy (no squaring
+// of the condition number).  y (6 values, or null) receives the same rotations: U^T y.
+static __device__ __noinline__ void jacobi_rows(double* g, int n, double* y) {
     for (int sweep = 0; sweep < 30; ++sweep) {
         double off = 0.0;
         for (int p = 0; p < 5; ++p)
@@ -95,12 +90,51 @@ static __device__ __noinline__ void ik_truncated(double* g, int n, double* y, do
                     g[p * n + j] = cs * u - sn * v;
                     g[q * n + j] = sn * u + cs * v;
                 }
-                const double u = y[p], v = y[q];
-                y[p] = cs * u - sn * v;
-                y[q] = sn * u + cs * v;
+                if (y) {
+                    const double u = y[p], v = y[q];
+                    y[p] = cs * u - sn * v;
+                    y[q] = sn * u + cs * v;
+                }
             }
         if (off < 1e-15) break;
     }
+}
+
+// Relative cutoff of the undamped projector: singular values sigma_i <= cut * sigma_max count as zero.  FP64: 1e-15, the
+// default of numpy.linalg.pinv and so the reference's own rule (scripts/nullspace:78).  FP32: the Jacobian is rounded to
+// float (6e-8 relative) before this FP64 factorisation, which lifts an exactly zero singular value to ~1e-9 .. 1e-8 of
+// sigma_max; with 1e-15 those would count as rank and turn the projector O(1) wrong.  Any cutoff in 1e-7 .. 1e-5 cuts
+// them: at exactly singular LWR postures the projector of the rounded Jacobian then matches the FP64 one to 2e-7.  Near
+// a singularity (cond(J) ~ 1e6) the FP32 projector is O(1) off either way (DESIGN.md section 2).
+constexpr double kNsCutF64 = 1e-15, kNsCutF32 = 1e-6;
+
+// w <- (I - pinv(J) J) w, g = J (6 x n row-major, destroyed): after jacobi_rows row i of g is sigma_i v_i^T, so
+// pinv(J) J = sum over sigma_i > cut * sigma_max of v_i v_i^T, and w loses its component g_i (g_i . w) / |g_i|^2 along
+// each kept row.  Rank-revealing: at rank r < 6 the result lies in the whole (N - r)-dimensional null(J).
+static __device__ __noinline__ void ns_svd_project(double* g, int n, double cut, double* w) {
+    jacobi_rows(g, n, nullptr);
+    double s2[6], smax2 = 0.0;
+    for (int r = 0; r < 6; ++r) {
+        s2[r] = 0.0;
+        for (int j = 0; j < n; ++j) s2[r] = fma(g[r * n + j], g[r * n + j], s2[r]);
+        smax2 = fmax(smax2, s2[r]);
+    }
+    const double cut2 = cut * cut * smax2;
+    for (int r = 0; r < 6; ++r) {
+        if (!(s2[r] > cut2)) continue;
+        double d = 0.0;
+        for (int j = 0; j < n; ++j) d = fma(g[r * n + j], w[j], d);
+        d /= s2[r];
+        for (int j = 0; j < n; ++j) w[j] = fma(-d, g[r * n + j], w[j]);
+    }
+}
+
+// ---- truncated weighted least squares (VFK_IK_TRUNCATED).
+// g: Jw = Wt J Wj, 6 x n row-major (g[r * n + j]); y: Wt t (6).  jacobi_rows gives G' = U^T Jw = Sigma V^T and U^T y, so
+//   qd = V diag(f(sigma)) U^T y = sum_i row_i * c_i * (U^T y)_i,  c_i = 1 / sigma_i^2 (sigma_i >= eps), 1 / (sigma_i^2 + lambda^2) below.
+// qd: n values (before the joint weights).  Restated by oracle/batch.py:ikv_dls (ik_mode 1) through numpy's SVD.
+static __device__ __noinline__ void ik_truncated(double* g, int n, double* y, double lambda2, double eps, double* qd) {
+    jacobi_rows(g, n, y);
     for (int j = 0; j < n; ++j) qd[j] = 0.0;
     const double eps2 = eps * eps;
     for (int r = 0; r < 6; ++r) {
