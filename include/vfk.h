@@ -215,6 +215,25 @@ const char* vfk_last_error(vfk_handle h);   /* h may be NULL: last error of vfk_
 int  vfk_step(vfk_handle h, const vfk_buffers* bufs, int64_t n_instances, int n_obstacles,
               int k_cycles, void* stream);
 
+/* Run each instance's control loop until its tool reaches the goal: the batched HandleArm.gotoFrame / gotThere
+ * (src/handlers.py:346-387), which poll the distance monitor until the tool is within goal_precision.  Inputs and
+ * parameters as for vfk_step (params.integrate must be 1).  q_c = q after c cycles; the rule at q_c is
+ *     |p_goal - p_tool| < tol_trans (metres)  and  angle(R_goal R_tool^T) < tol_rot (radians, [0, pi])
+ * for the tool frame (params.tool), strict as in the reference; tol_rot >= pi drops the orientation condition, and a
+ * tolerance of 0 can never be met.  Per instance:
+ *     cycles_out [1] (int32, blocked)  the smallest c in 0..max_cycles with the rule at q_c, or -1 if there is none;
+ *     q (in/out)                       q_c for that c (the instance stops there: no further integration), else q_max_cycles;
+ *     dist_out [2] (blocked, or NULL)  {|p_goal - p_tool|, angle} at the returned q;
+ *     jp_ref (with jp_lo / jp_hi) and ns_lastvec hold the state of the instance's last cycle, as after vfk_step.
+ * The returned q is bit-identical to vfk_step with k_cycles = cycles_out (or max_cycles) on the same batch.  A warp
+ * whose 32 instances have all stopped takes its next tile, so converged work costs nothing.  The per-cycle outputs of
+ * vfk_buffers (qdot_vf, qdot_ns, qdot_jp, qdot, cmd, pose, twist, flags) must be NULL: they have no single meaning in
+ * a batch whose instances stop at different cycles.  In precision 32 the tool frame is rounded to float (6e-8), so
+ * tolerances below about 1e-6 m / 1e-6 rad may never be met.  No allocation, no synchronisation; returns the number
+ * of kernels launched or a negative vfk_status. */
+int  vfk_solve(vfk_handle h, const vfk_buffers* bufs, int64_t n_instances, int n_obstacles, int max_cycles,
+               double tol_trans, double tol_rot, int32_t* cycles_out, void* dist_out, void* stream);
+
 /* Field visualisation query (scripts/vf:469-503): twist the composed field commands at
  * arbitrary tool poses pose_in [12]; twist_out [6] (blocked layout).  Same goal/obst layout. */
 int  vfk_field_eval(vfk_handle h, const void* pose_in, const void* goal, const void* obst,
@@ -274,6 +293,11 @@ int  vfk_session_set_jp_limits(vfk_session s, const void* lo_host,          /* [
 int  vfk_session_set_ns_input(vfk_session s, const void* ns_host);          /* [N|4][n] or NULL */
 int  vfk_session_cycle(vfk_session s, const void* q_in_host, int k_cycles,
                        void* qdot_out_host, void* q_out_host, int32_t* flags_out_host);
+/* vfk_solve on the session's resident scene and state: q from the host (if q_in != NULL, through vfk_session_set_q),
+ * the stop rule as in vfk_solve, then q_out [N][n], cycles_out [n] (int32) and dist_out [2][n] back to the host (each
+ * may be NULL); synchronises. */
+int  vfk_session_solve(vfk_session s, const void* q_in_host, int max_cycles, double tol_trans, double tol_rot,
+                       void* q_out_host, int32_t* cycles_out_host, void* dist_out_host);
 /* Optional per-controller outputs the kernel writes each cycle ("qdot_vf","qdot_ns","qdot_jp","cmd","pose","twist");
  * all off by default so the resident path only moves q in and qdot out. */
 int  vfk_session_enable(vfk_session s, const char* what, int on);

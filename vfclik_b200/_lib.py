@@ -34,9 +34,9 @@ LIB_PATH = os.environ.get("VFK_LIB") or os.path.join(os.path.dirname(os.path.abs
 EXPORTS = [
     "vfk_version", "vfk_default_params", "vfk_create", "vfk_set_params", "vfk_get_params", "vfk_chain_pattern",
     "vfk_destroy",
-    "vfk_last_error", "vfk_step", "vfk_field_eval", "vfk_mix", "vfk_set_vel", "vfk_monitor", "vfk_pack", "vfk_unpack", "vfk_session_create", "vfk_session_set_goal",
+    "vfk_last_error", "vfk_step", "vfk_solve", "vfk_field_eval", "vfk_mix", "vfk_set_vel", "vfk_monitor", "vfk_pack", "vfk_unpack", "vfk_session_create", "vfk_session_set_goal",
     "vfk_session_set_obstacles", "vfk_session_set_aux", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_jp_limits", "vfk_session_set_ns_input",
-    "vfk_session_cycle", "vfk_session_enable", "vfk_session_read", "vfk_session_buffers", "vfk_session_destroy",
+    "vfk_session_cycle", "vfk_session_solve", "vfk_session_enable", "vfk_session_read", "vfk_session_buffers", "vfk_session_destroy",
 ]
 
 
@@ -116,6 +116,7 @@ def load():
     lib.vfk_last_error.argtypes = [vp]
     lib.vfk_last_error.restype = C.c_char_p
     lib.vfk_step.argtypes = [vp, C.POINTER(BuffersC), i64, i32, i32, vp]
+    lib.vfk_solve.argtypes = [vp, C.POINTER(BuffersC), i64, i32, i32, C.c_double, C.c_double, vp, vp, vp]
     lib.vfk_field_eval.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, i64, i32, vp]
     lib.vfk_mix.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_double), i32, i32, vp, vp, i64, vp]
     lib.vfk_set_vel.argtypes = [vp, vp, vp, vp, C.c_double, i32, vp, vp, i32, i64, vp]
@@ -129,6 +130,7 @@ def load():
     lib.vfk_session_set_jp_limits.argtypes = [vp, vp, vp]
     lib.vfk_session_set_aux.argtypes = [vp, vp, i32]
     lib.vfk_session_cycle.argtypes = [vp, vp, i32, vp, vp, vp]
+    lib.vfk_session_solve.argtypes = [vp, vp, i32, C.c_double, C.c_double, vp, vp, vp]
     lib.vfk_session_read.argtypes = [vp, C.c_char_p, vp]
     lib.vfk_session_enable.argtypes = [vp, C.c_char_p, i32]
     lib.vfk_session_buffers.argtypes = [vp, C.POINTER(BuffersC)]

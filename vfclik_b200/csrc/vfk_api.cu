@@ -267,8 +267,8 @@ static int check_layout(vfk_ctx* h, const void* ptr, const char* name, bool requ
     return VFK_OK;
 }
 
-static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream, const vfk_io* io) {
-    if (!h || !b) return fail(h, VFK_ERR_INVALID, "vfk_step: null argument");
+// The argument checks vfk_step and vfk_solve share.
+static int check_step(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles) {
     if (n < 0) return fail(h, VFK_ERR_INVALID, "n_instances must be >= 0 (got %lld)", (long long)n);
     if (n_obst < 0) return fail(h, VFK_ERR_INVALID, "n_obstacles must be >= 0");
     if (k_cycles < 1) return fail(h, VFK_ERR_INVALID, "k_cycles must be >= 1");
@@ -286,6 +286,13 @@ static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, in
     for (int e = 0; e < 3; ++e)
         if ((rc = check_layout(h, b->ext_cmd[e], "ext_cmd", false))) return rc;
     if ((b->jp_lo == nullptr) != (b->jp_hi == nullptr)) return fail(h, VFK_ERR_INVALID, "jp_lo and jp_hi go together");
+    return VFK_OK;
+}
+
+static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream, const vfk_io* io) {
+    if (!h || !b) return fail(h, VFK_ERR_INVALID, "vfk_step: null argument");
+    int rc = check_step(h, b, n, n_obst, k_cycles);
+    if (rc) return rc;
     if (n == 0) return 0;
     VFK_CUDA(h, cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -297,6 +304,33 @@ static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, in
 
 extern "C" int vfk_step(vfk_handle h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream) {
     return step_impl(h, b, n, n_obst, k_cycles, stream, nullptr);
+}
+
+// -------------------------------------------------------------------------------- public: solve
+extern "C" int vfk_solve(vfk_handle h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, double tol_trans,
+                         double tol_rot, int32_t* cycles_out, void* dist_out, void* stream) {
+    if (!h || !b) return fail(h, VFK_ERR_INVALID, "vfk_solve: null argument");
+    if (!h->params.integrate) return fail(h, VFK_ERR_INVALID, "vfk_solve needs params.integrate = 1: without the plant q never moves");
+    if (max_cycles < 1) return fail(h, VFK_ERR_INVALID, "max_cycles must be >= 1");
+    if (!(tol_trans >= 0) || !(tol_rot >= 0))
+        return fail(h, VFK_ERR_INVALID, "tolerances must be >= 0 and not NaN (got tol_trans = %g, tol_rot = %g)", tol_trans, tol_rot);
+    if (!cycles_out) return fail(h, VFK_ERR_INVALID, "vfk_solve: cycles_out is required");
+    const struct { const void* p; const char* name; } per_cycle[] = {
+        {b->qdot_vf, "qdot_vf"}, {b->qdot_ns, "qdot_ns"}, {b->qdot_jp, "qdot_jp"}, {b->qdot, "qdot"},
+        {b->cmd, "cmd"}, {b->pose, "pose"}, {b->twist, "twist"}, {b->flags, "flags"}};
+    for (const auto& o : per_cycle)
+        if (o.p) return fail(h, VFK_ERR_INVALID, "vfk_solve: output %s must be NULL (a per-cycle output has no single meaning when instances stop at different cycles)", o.name);
+    int rc = check_step(h, b, n, n_obst, max_cycles);
+    if (rc || (rc = check_layout(h, cycles_out, "cycles_out", true)) || (rc = check_layout(h, dist_out, "dist_out", false))) return rc;
+    if (n == 0) return 0;
+    VFK_CUDA(h, cudaSetDevice(h->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    vfk_solve_io sv;
+    sv.tol_trans = tol_trans;
+    sv.tol_rot = tol_rot;
+    sv.cycles = cycles_out;
+    sv.dist = dist_out;
+    return h->precision == 32 ? vfk_solve_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_f64(h, b, n, n_obst, max_cycles, st, &sv);
 }
 
 extern "C" int vfk_field_eval(vfk_handle h, const void* pose_in, const void* goal, const void* obst, const void* obst_ext,
@@ -466,6 +500,7 @@ struct vfk_session_s {
     bool have_jp_ref, have_ns_in, have_jp_lim;
     bool en_vf, en_ns, en_jp, en_cmd, en_pose, en_twist;   // optional per-controller outputs (off by default)
     void *d_jp_ref, *d_ns_in, *d_jp_lo, *d_jp_hi;
+    void *d_cycles, *d_dist;         // vfk_session_solve's results: cycles [1] int32, dist [2]
     char* aux_dev;                   // auxiliary field records (blocked + dense staging), grown on demand
     char* pin;                       // pinned host staging: q in (N rows), qdot / q out (2N rows), flags
     size_t pin_bytes;
@@ -503,9 +538,10 @@ extern "C" int vfk_session_create(vfk_handle h, int64_t n, int n_obst, int with_
     const int N = s->N;
     const size_t row = align_up((size_t)s->tiles * 32 * s->es, 128);     // one component over all tiles
     const size_t obst_rows = (size_t)((n_obst + 1) & ~1) * 4 + (size_t)n_obst * (s->has_ext ? 2 : 0);
-    // blocked: q N, goal 13, obst, jp_ref N, ns_in N, lastvec N, qdot_vf N, qdot_ns N, qdot_jp N, qdot N, cmd N, pose 12, twist 6, flags 1
+    // blocked: q N, goal 13, obst, jp_ref N, ns_in N, lastvec N, qdot_vf N, qdot_ns N, qdot_jp N, qdot N, cmd N, pose 12, twist 6, flags 1,
+    // solve cycles 1 + dist 2
     const int lv_rows = (ns_ctrl_vectors(N) > 0 ? ns_ctrl_vectors(N) : 1) * N;   // sign-continuity state: [min(4, N - 6)][N]
-    const size_t rows = (size_t)N * 10 + lv_rows + 13 + obst_rows + 12 + 6 + 1;
+    const size_t rows = (size_t)N * 10 + lv_rows + 13 + obst_rows + 12 + 6 + 1 + 3;
     const size_t stage_in_rows = obst_rows > (size_t)(N > 13 ? N : 13) ? obst_rows : (size_t)(N > 13 ? N : 13);
     const size_t first_out = (size_t)(lv_rows > 12 ? lv_rows : 12);
     const size_t stage_out_rows = first_out + (size_t)N;                          // qdot (or a read()) + q_out
@@ -532,6 +568,8 @@ extern "C" int vfk_session_create(vfk_handle h, int64_t n, int n_obst, int with_
     s->b.pose = take(12);
     s->b.twist = take(6);
     s->b.flags = (int32_t*)take(1);
+    s->d_cycles = take(1);
+    s->d_dist = take(2);
     s->stage_in = take(stage_in_rows);
     s->stage_out = take(stage_out_rows);
     s->have_jp_ref = s->have_ns_in = s->have_jp_lim = false;
@@ -881,6 +919,39 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
     if (qdot_out && !d_qd) memcpy(qdot_out, pin_qd, blk);
     if (q_out && !d_qo) memcpy(q_out, pin_qo, blk);
     if (flags_out && !d_fl) memcpy(flags_out, pin_fl, (size_t)s->n * 4);
+    return launches;
+}
+
+extern "C" int vfk_session_solve(vfk_session s, const void* q_in, int max_cycles, double tol_trans, double tol_rot, void* q_out,
+                                 int32_t* cycles_out, void* dist_out) {
+    if (!s) return fail(nullptr, VFK_ERR_INVALID, "vfk_session_solve: null session");
+    vfk_ctx* h = s->h;
+    int rc;
+    if (q_in && (rc = vfk_session_set_q(s, q_in)) != VFK_OK) return rc;
+    vfk_buffers b;
+    if ((rc = vfk_session_buffers(s, &b)) != VFK_OK) return rc;
+    b.qdot_vf = b.qdot_ns = b.qdot_jp = b.qdot = b.cmd = b.pose = b.twist = nullptr;
+    b.flags = nullptr;
+    if ((rc = vfk_solve(h, &b, s->n, s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
+                        s->stream)) < 0)
+        return rc;
+    int launches = rc;
+    char* stage = (char*)s->stage_out;                          // dense q [N][n], then dist [2][n]
+    const size_t blk = (size_t)s->N * (size_t)s->n * s->es;
+    if (q_out) {
+        if ((rc = pack_dispatch(h, stage, b.q, s->N, 1, s->n, true, s->stream)) < 0) return rc;
+        launches += rc;
+        VFK_CUDA(h, cudaMemcpyAsync(q_out, stage, blk, cudaMemcpyDeviceToHost, s->stream));
+    }
+    if (dist_out) {
+        if ((rc = pack_dispatch(h, stage + blk, s->d_dist, 2, 1, s->n, true, s->stream)) < 0) return rc;
+        launches += rc;
+        VFK_CUDA(h, cudaMemcpyAsync(dist_out, stage + blk, 2 * (size_t)s->n * s->es, cudaMemcpyDeviceToHost, s->stream));
+    }
+    if (cycles_out)         // one component: blocked == dense
+        VFK_CUDA(h, cudaMemcpyAsync(cycles_out, s->d_cycles, (size_t)s->n * 4, cudaMemcpyDeviceToHost, s->stream));
+    VFK_CUDA(h, cudaStreamSynchronize(s->stream));
+    s->launches = launches;
     return launches;
 }
 

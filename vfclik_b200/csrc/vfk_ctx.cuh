@@ -18,6 +18,13 @@ struct vfk_io {
     int64_t qdot_ld = 0;
 };
 
+// Stop rule and result buffers of vfk_solve, handed to the SOLVE instantiations of the cycle kernel.
+struct vfk_solve_io {
+    double tol_trans, tol_rot;  // metres, radians (>= pi: orientation not checked)
+    int32_t* cycles;            // [1] blocked
+    void* dist;                 // [2] blocked, or null
+};
+
 struct vfk_ctx {
     vfk_chain_desc chain;       // as given
     vfk_chain_desc canon;       // every joint about / along Z
@@ -60,3 +67,6 @@ int vfk_launch_f32_small(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst
 int vfk_launch_f32_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);   // N = 10, 17
 int vfk_launch_f64_small(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
 int vfk_launch_f64_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
+// The vfk_solve variants, one translation unit per precision.
+int vfk_solve_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+int vfk_solve_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);

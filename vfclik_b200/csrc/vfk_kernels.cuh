@@ -27,6 +27,7 @@
 #include "vfk_math.cuh"
 #include "vfk_tma.cuh"
 #include "vfk_nullspace.cuh"
+#include "vfk_ring.cuh"
 
 namespace vfk {
 
@@ -128,6 +129,11 @@ struct KArgs {
     int32_t k_cycles;
     int32_t n_aux;
     int32_t n_comp;            // joint components per instance in memory (<= N: generic chains of fewer joints run padded, see nc below)
+    // vfk_solve (SOLVE kernels only): the stop rule's thresholds and the per-instance results
+    T tol_d2;                  // tol_trans^2
+    T tol_q2;                  // sin^2(tol_rot / 2) against |xyz|^2 of the error quaternion; +inf when tol_rot >= pi
+    int32_t* cycles;           // [1] first cycle c whose q_c met the rule, or -1
+    T* dist;                   // [2] {|p_goal - p_tool|, rotation angle} at the returned q, or null
 };
 
 // ------------------------------------------------------------------------------ chain patterns
@@ -390,11 +396,18 @@ __device__ __forceinline__ void repel2(const float4& A, const float4& B, float s
     acc[0] = __ffma2_rn(wgt, dx, acc[0]); acc[1] = __ffma2_rn(wgt, dy, acc[1]); acc[2] = __ffma2_rn(wgt, dz, acc[2]);
 }
 
+// What the attractor knows about the distance to the goal: d2 = |p_goal - p_tool|^2 (+ the tiny bias), dist = its root,
+// and the error rotation R_g Rt^T as the quaternion's w and |xyz|^2 = sin^2(angle / 2).
+template <typename T>
+struct GoalErr {
+    T d2, dist, n2, qw;
+};
+
 // Goal attractor (vfl type 1) at tool frame (Rt, pt): unit direction to the goal, unit rotation
 // axis of R_g Rt^T scaled by the rotational slowdown, and the translational slowdown scalar.
 template <typename T>
 __device__ __forceinline__ void attract(const KConst<T>& c, const T (&g)[13], const T (&Rt)[9], const Pos<T>& pt,
-                                        T (&V)[3], T& S0, T (&w)[3]) {
+                                        T (&V)[3], T& S0, T (&w)[3], GoalErr<T>& ge) {
     const T ex = pt.from(g[9], 0), ey = pt.from(g[10], 1), ez = pt.from(g[11], 2);
     const T d2 = fma(ex, ex, fma(ey, ey, fma(ez, ez, Prec<T>::tiny())));
     const T invd = Prec<T>::rsqrt_pos(d2);
@@ -428,6 +441,14 @@ __device__ __forceinline__ void attract(const KConst<T>& c, const T (&g)[13], co
     const T S1 = Prec<T>::fmin_(angle * c.rot_slowdown_inv, T(1));
     const T sr = c.speed_scale * S1 * c.goal_force * invn;
     w[0] = sr * qx; w[1] = sr * qy; w[2] = sr * qz;
+    ge.d2 = d2; ge.dist = dist; ge.n2 = n2; ge.qw = qw;
+}
+
+template <typename T>
+__device__ __forceinline__ void attract(const KConst<T>& c, const T (&g)[13], const T (&Rt)[9], const Pos<T>& pt,
+                                        T (&V)[3], T& S0, T (&w)[3]) {
+    GoalErr<T> ge;
+    attract<T>(c, g, Rt, pt, V, S0, w, ge);
 }
 
 // Auxiliary fields (SURVEY.md section 8 row f2): records of VFK_AUX_COMPS = 12 scalars {type, force, p0..p9} in slots of a
@@ -552,7 +573,14 @@ __device__ __forceinline__ void issue_qg(const KArgs<T>& a, int64_t tile, int bu
 // small batches -- a warp takes 4 instances of a tile, the 8 lanes of a group split each chunk of 8 obstacles between
 // them and combine their partial repulsor sums with __shfl_xor_sync; the rest of the cycle is computed redundantly by
 // the group and lane 0 of the group stores.  A tile is then spread over 8 warps instead of one.
-template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1>
+// SOLVE = vfk_solve: every cycle first checks the stop rule on the q it starts from (|p_goal - p_tool|^2 < tol_d2 and
+// |xyz|^2 of the error quaternion < tol_q2, both by-products of the attractor), and one more cycle index, k_cycles, only
+// evaluates FK and the rule.  An instance that meets it is done: it stores its cycle index and distance, never integrates
+// again and keeps taking part in everything warp-collective.  Padding lanes start done; in the cooperative shape the
+// group follows its lane 0.  Once every lane of the unit is done the warp retires the unit's part of the obstacle ring
+// (ring_leave, vfk_ring.cuh) and moves on to its next unit.  The per-cycle outputs (qdot, flags, pose, ...) do not exist
+// in this mode; the state a cycle carries (q, jp_ref, ns_lastvec) freezes with the instance.
+template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool SOLVE = false>
 __global__ void __launch_bounds__(kBlock, MINB)
 vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a) {
     using WS = WarpStage<T, N, EXT>;
@@ -583,7 +611,9 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     // resident: S = n_chunks, every chunk is loaded once per tile and reused by all K cycles (U = n_chunks);
     // streaming: S < n_chunks, chunks are re-requested every cycle (U = K * n_chunks).
     // The producer cursor (p_*) is always exactly S uses ahead of the consumer, so a refill targets the slot
-    // the consumer has just finished with.  Everything advances by increments (no integer division).
+    // the consumer has just finished with.  Everything advances by increments (no integer division).  The advance below is
+    // what ring_produced / ring_consumed (vfk_ring.cuh) restate for the host; it stays written out here because routing it
+    // through them changes the register allocation of every instantiation.
     const bool resident = a.n_chunks <= a.n_stages;
     const int S = resident ? a.n_chunks : a.n_stages;
     const int U = resident ? a.n_chunks : a.n_chunks * a.k_cycles;
@@ -652,7 +682,8 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         for (int k = 0; k < 13; ++k) g[k] = qg[(N + k) * 32];
     }
 
-    for (int cyc = 0; cyc < a.k_cycles; ++cyc) {
+    bool done = SOLVE && !((tile << 5) + slot < a.n);           // SOLVE: this lane's instance has stopped (padding: from the start)
+    for (int cyc = 0; cyc < a.k_cycles + (SOLVE ? 1 : 0); ++cyc) {
         const bool last = (cyc == a.k_cycles - 1);
         int flags = 0;
 
@@ -692,7 +723,38 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
 #pragma unroll
                 for (int k = 0; k < 13; ++k) g[k] = qg[(N + k) * 32];
             }
-            attract<T>(c, g, Rt, pt, V, S0, w);
+            GoalErr<T> ge;
+            attract<T>(c, g, Rt, pt, V, S0, w, ge);
+            if constexpr (SOLVE) {
+                bool hit = ge.d2 < a.tol_d2 && ge.n2 < a.tol_q2;
+                if constexpr (G > 1) hit = __shfl_sync(0xffffffffu, hit, lane & ~(G - 1));     // the group cannot split
+                if (!done && (hit || cyc == a.k_cycles)) {
+                    done = true;
+                    if (active) {
+                        a.cycles[(tile << 5) + slot] = hit ? cyc : -1;
+                        if (a.dist) {
+                            a.dist[tile * (2 * 32) + slot] = ge.dist;
+                            a.dist[tile * (2 * 32) + 32 + slot] = T(2) * Prec<T>::atan2_(Prec<T>::sqrt_(ge.n2), Prec<T>::fabs_(ge.qw));
+                        }
+                    }
+                }
+                if (__all_sync(0xffffffffu, done)) {
+                    // the whole unit has stopped: wait what the ring still has in flight for it, refill those slots with the
+                    // next unit's chunks, and move on.  A resident ring requests the next unit's chunks in the last cycle,
+                    // so a cycle that leaves early does that instead.
+                    const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
+                                              : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
+                    for (int i = 0; i < left; ++i) {
+                        const int stage = resident ? i : c_stage;
+                        mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
+                        __syncwarp();
+                        if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
+                        ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
+                        if (!resident) ring_consumed(c_stage, c_phase, S);
+                    }
+                    break;
+                }
+            }
             [[maybe_unused]] NegPos2 np2;                               // FP32 packed repulsor: duplicated tool position, paired sums
             [[maybe_unused]] float2 acc2[3] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) np2.set(pt);
@@ -991,7 +1053,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                                 for (int j = 0; j < N; ++j) if (j < nc) dotl = fma(wv[j], (double)lv[j * 32], dotl);
                                 const double sgn = dotl < 0.0 ? -1.0 : 1.0;      // |s u - last| > |s u + last|  <=>  s u . last < 0
                                 const double ci = a.ns_in ? (double)__ldg(a.ns_in + tile * (4 * 32) + i * 32 + slot) : (double)c.ns_control[i];
-                                if (active) {
+                                if (active && !(SOLVE && done)) {
     #pragma unroll
                                     for (int j = 0; j < N; ++j) if (j < nc) lv[j * 32] = (T)(sgn * wv[j]);
                                 }
@@ -1027,7 +1089,8 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     const T lo = (a.jp_lo && j < nc) ? __ldg(a.jp_lo + tN + j * 32) : c.q_lo[j];
                     const T hi = (a.jp_lo && j < nc) ? __ldg(a.jp_hi + tN + j * 32) : c.q_hi[j];
                     ref = ref < lo ? lo : (ref > hi ? hi : ref);
-                    if (a.jp_lo && a.jp_ref && last && active && j < nc) a.jp_ref[tN + j * 32] = ref;      // the clamp persists
+                    // the clamp persists (SOLVE: stored by every cycle the instance runs; it is the same value each time)
+                    if (a.jp_lo && a.jp_ref && (SOLVE ? !done : last) && active && j < nc) a.jp_ref[tN + j * 32] = ref;
                     const T err = ref - q[j];
                     qd_jp[j] = err * c.jp_kp;
                     all_reached = all_reached && (err < c.jp_delta);
@@ -1084,7 +1147,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             ratio *= r2;
         }
 
-        if (last && active) {
+        if (!SOLVE && last && active) {
             if (!LEAN && a.qdot_vf) {
 #pragma unroll
                 for (int j = 0; j < N; ++j) if (j < nc) a.qdot_vf[tN + j * 32] = qd_vf[j];
@@ -1125,7 +1188,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             if (!LEAN && a.flags) a.flags[(tile << 5) + slot] = flags;
         }
         // 10. plant
-        if (c.integrate) {
+        if (c.integrate && !(SOLVE && done)) {
 #pragma unroll
             for (int j = 0; j < N; ++j) q[j] = fma(c.dt, mix[j] * ratio, q[j]);
         }

@@ -1,5 +1,6 @@
 // vfk_launch.cuh -- launch plan and feature dispatch of the fused cycle kernel (included by vfk_cycle_*.cu).
 #pragma once
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
@@ -49,21 +50,27 @@ struct PlanCache {
 
 constexpr int64_t kCoopMaxInstances = 4096;      // <= 128 tiles: 1024 cooperative warps instead of 128 solo ones
 
-// The LEAN kernel's preconditions (see vfk_kernels.cuh).
+// The LEAN kernel's preconditions (see vfk_kernels.cuh): on the constants and inputs (all a solve has to meet, since it
+// has no per-cycle outputs), and for a step also on the outputs.
 template <typename T>
-static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
+static bool lean_inputs(const KConst<T>& c, const vfk_buffers* b) {
     return c.tool_identity && c.unit_weights && c.share_factor && c.ik_mode == 0 && c.ns_mode == VFK_NS_PROJECTOR && !c.need_jp && !b->ns_in &&
            !c.shoulder_clamp &&
-           !b->jp_ref && !b->jp_lo && !b->q_cmded && !b->ext_cmd[0] && !b->ext_cmd[1] && !b->ext_cmd[2] && !b->qdot_vf && !b->qdot_ns &&
-           !b->qdot_jp && !b->cmd && !b->pose && !b->twist && !b->flags && !(b->aux && b->n_aux > 0) && b->qdot;
+           !b->jp_ref && !b->jp_lo && !b->q_cmded && !b->ext_cmd[0] && !b->ext_cmd[1] && !b->ext_cmd[2] && !(b->aux && b->n_aux > 0);
+}
+
+template <typename T>
+static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
+    return lean_inputs<T>(c, b) && !b->qdot_vf && !b->qdot_ns && !b->qdot_jp && !b->cmd && !b->pose && !b->twist && !b->flags && b->qdot;
 }
 
 // HIOCC: the single-cycle lean FP32 launch asks for one more resident CTA per SM (4 x 128 threads at 128 registers, no
 // spills).  Measured on B200, 1 M instances: 109.5 us vs 111.2 us per launch at K = 1 (more warps hide more HBM latency),
 // but 1.6 % slower at K = 100, where the kernel is issue-bound and the tighter register budget costs instructions.
-template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false>
+// SOLVE: the vfk_solve variant (vfk_kernels.cuh), with its stop rule and result buffers in `sv`.
+template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false, bool SOLVE = false>
 static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io) {
+                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     KArgs<T> a;
     memset(&a, 0, sizeof a);
     a.q = static_cast<T*>(b->q);
@@ -94,13 +101,22 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     a.n_obst = n_obst;
     a.n_obst_p = (n_obst + 1) & ~1;
     a.k_cycles = k_cycles;
+    if constexpr (SOLVE) {
+        // thresholds in T: |dp|^2 against tol_trans^2, and |xyz|^2 = sin^2(angle / 2) of the error quaternion against
+        // sin^2(tol_rot / 2) -- exact and monotone on [0, pi], no transcendental in the kernel
+        a.tol_d2 = (T)(sv->tol_trans * sv->tol_trans);
+        const double sh = std::sin(0.5 * sv->tol_rot);
+        a.tol_q2 = sv->tol_rot >= 3.14159265358979323846 ? (T)INFINITY : (T)(sh * sh);
+        a.cycles = sv->cycles;
+        a.dist = static_cast<T*>(sv->dist);
+    }
     size_t smem = 0;
     plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
     a.n_full = n_obst / kChunk;
     a.n_rem = n_obst % kChunk;
     // resident CTAs per SM that the register allocation aims for
     constexpr int MINB = HIOCC ? 4 : (sizeof(T) == 4 ? (N <= 10 ? 3 : 2) : (N <= 7 ? 2 : 1));
-    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G>;
+    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, SOLVE>;
     // per (instantiation, device, smem size): opt in to > 48 KB of dynamic shared memory and ask the occupancy once
     static PlanCache plans;
     int per_sm = 0;
@@ -206,9 +222,11 @@ static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     return 1;
 }
 
-template <typename T, int N, class PAT>
+// SOLVE: the same choice of shape for vfk_solve, except that the lane-split shape has no solve variant (those calls run
+// the one-thread-per-instance kernel) and the lean kernel's output conditions do not apply.
+template <typename T, int N, class PAT, bool SOLVE = false>
 static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                         cudaStream_t st, const vfk_io* io) {
+                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     const bool ext = b->obst_ext && n_obst > 0;
     // Small FP64 batches cannot fill the GPU with one thread per instance: switch to the cooperative latency shape.
     // Measured (scripts/latency.py, one robot, 1000 fused cycles): FP64 M = 32: 6.4 vs 7.1 us per cycle, M = 256: 23.6 vs
@@ -216,32 +234,32 @@ static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, i
     // so it is neither selected nor instantiated there.
     if constexpr (sizeof(T) == 8) {
         const bool coop = n <= kCoopMaxInstances && n_obst >= 2 * kChunk && !getenv("VFK_NO_COOP");
-        if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk>(h, c, b, n, n_obst, k_cycles, st, io)
-                             : launch_cycle<T, N, PAT, false, false, kChunk>(h, c, b, n, n_obst, k_cycles, st, io);
+        if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv)
+                             : launch_cycle<T, N, PAT, false, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    if (ext) return launch_cycle<T, N, PAT, true, false>(h, c, b, n, n_obst, k_cycles, st, io);
+    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     // Two lanes per instance (vfk_split.cuh) for the FP64 17-joint kernel.
-    if constexpr (kSplit<T, N>) {
+    if constexpr (kSplit<T, N> && !SOLVE) {
         if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N>(h, c, b, n, n_obst, k_cycles, st);
     }
-    if (is_lean<T>(c, b) && h->chain.n_joints == N) {
-        if constexpr (sizeof(T) == 4 && N <= 7) {
+    if ((SOLVE ? lean_inputs<T>(c, b) : is_lean<T>(c, b)) && h->chain.n_joints == N) {
+        if constexpr (sizeof(T) == 4 && N <= 7 && !SOLVE) {
             if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true>(h, c, b, n, n_obst, k_cycles, st, io);
         }
-        return launch_cycle<T, N, PAT, false, true>(h, c, b, n, n_obst, k_cycles, st, io);
+        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    return launch_cycle<T, N, PAT, false, false>(h, c, b, n, n_obst, k_cycles, st, io);
+    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
 }
 
-template <typename T, int N>
+template <typename T, int N, bool SOLVE = false>
 static int dispatch_ext(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io) {
+                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     if constexpr (N == 7) {
-        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern>(h, c, b, n, n_obst, k_cycles, st, io);
+        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
     if constexpr (N >= 10) {
-        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern>(h, c, b, n, n_obst, k_cycles, st, io);
+        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    return dispatch_feat<T, N, GenericPattern>(h, c, b, n, n_obst, k_cycles, st, io);
+    return dispatch_feat<T, N, GenericPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
 }
 

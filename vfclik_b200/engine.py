@@ -118,6 +118,7 @@ def round_up(n: int, m: int = 32) -> int:
 
 _BUF_FIELDS = ("q", "goal", "obst", "obst_ext", "aux", "jp_ref", "jp_lo", "jp_hi", "ns_in", "ns_lastvec", "q_cmded", "qdot_vf", "qdot_ns", "qdot_jp",
                "qdot", "cmd", "pose", "twist", "flags")
+_PER_CYCLE = ("qdot_vf", "qdot_ns", "qdot_jp", "qdot", "cmd", "pose", "twist", "flags")     # outputs vfk_solve does not take
 
 
 def _dev_ptr(x) -> Optional[int]:
@@ -206,6 +207,26 @@ class Engine:
         b.n_aux = 0 if aux is None else int(aux.shape[1]) // 12
         rc = self._check(self._lib.vfk_step(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(k_cycles),
                                             self._stream(stream)))
+        self.launches += rc
+        return rc
+
+    def solve(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, max_cycles: int, tol_trans: float,
+              tol_rot: float, cycles_out, dist_out=None, stream: Optional[int] = None, ext_cmd=(None, None, None)) -> int:
+        """Run each instance's control loop until its tool frame is within ``tol_trans`` metres and ``tol_rot`` radians of
+        its goal (strict), for at most ``max_cycles`` cycles (``vfk_solve``, include/vfk.h): the batched
+        ``HandleArm.gotoFrame``.  ``cycles_out`` [1] int32 gets the cycle at which each instance stopped (-1: never),
+        ``dist_out`` [2] the distance and angle to the goal at the returned q; q is updated in place.  ``bufs`` may hold
+        no per-cycle output.  Returns the number of kernels launched."""
+        b = BuffersC()
+        for f in _BUF_FIELDS:
+            setattr(b, f, _dev_ptr(bufs.get(f)))
+        for e in range(3):
+            b.ext_cmd[e] = _dev_ptr(ext_cmd[e])
+        aux = bufs.get("aux")
+        b.n_aux = 0 if aux is None else int(aux.shape[1]) // 12
+        rc = self._check(self._lib.vfk_solve(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(max_cycles),
+                                             float(tol_trans), float(tol_rot), _dev_ptr(cycles_out), _dev_ptr(dist_out),
+                                             self._stream(stream)))
         self.launches += rc
         return rc
 
@@ -384,6 +405,30 @@ class Session:
         self.e.launches += rc
         return rc
 
+    def solve(self, q_in=None, max_cycles: int = 1000, tol_trans: float = 1e-3, tol_rot: float = 1e-2, q_out=None,
+              cycles_out=None, dist_out=None) -> int:
+        """``vfk_session_solve``: q from the host (if given), then every instance runs until its tool reaches the goal
+        (see ``Engine.solve``).  Outputs are filled in place: q ``[N, n]`` and dist ``[2, n]`` of the engine dtype, cycles
+        int32 ``[n]``."""
+        N = self.e.n_joints
+
+        def out_ptr(a, shape, dt):
+            if a is None:
+                return None
+            if a.dtype != dt or a.shape != shape or not a.flags.c_contiguous:
+                raise ValueError("output array must be contiguous %s %r" % (dt, shape))
+            return _lib.np_ptr(a)
+
+        qp = None
+        if q_in is not None:
+            q_in = self._arr(q_in, N)
+            qp = _lib.np_ptr(q_in)
+        rc = self.e._check(self.e._lib.vfk_session_solve(
+            self._s, qp, int(max_cycles), float(tol_trans), float(tol_rot), out_ptr(q_out, (N, self.n), self.e.np_dtype),
+            out_ptr(cycles_out, (self.n,), np.int32), out_ptr(dist_out, (2, self.n), self.e.np_dtype)))
+        self.e.launches += rc
+        return rc
+
     def enable(self, *what: str, on: bool = True):
         """Ask the kernel to also write per-controller outputs ("qdot_vf", "qdot_ns", "qdot_jp", "cmd", "pose")."""
         for w in what:
@@ -405,7 +450,7 @@ class DeviceBatch:
     library's pack kernel; ``download`` converts back.  ``bufs`` is what ``Engine.step`` takes.
     """
 
-    _ROWS = {"goal": 13, "pose": 12, "flags": 1, "twist": 6, "track": 8, "dist": 2, "mon_f": 32}
+    _ROWS = {"goal": 13, "pose": 12, "flags": 1, "twist": 6, "track": 8, "dist": 2, "mon_f": 32, "solve_dist": 2}
 
     def __init__(self, engine: Engine, n_instances: int, n_obstacles: int, obst_ext: bool = False,
                  outputs=("qdot",), inputs=()):
@@ -432,8 +477,8 @@ class DeviceBatch:
         if name in self.t:
             return self.t[name]
         import torch
-        if name in ("flags", "mon_i", "tracking_state"):
-            self.t[name] = self.e.alloc({"flags": 1, "mon_i": 6, "tracking_state": 2}[name], self.n, dtype=torch.int32)
+        if name in ("flags", "mon_i", "tracking_state", "cycles"):
+            self.t[name] = self.e.alloc({"flags": 1, "mon_i": 6, "tracking_state": 2, "cycles": 1}[name], self.n, dtype=torch.int32)
         elif name in ("obst", "obst_ext"):
             raise KeyError("%s was not allocated (n_obstacles = 0 or obst_ext=False)" % name)
         else:
@@ -516,3 +561,13 @@ class DeviceBatch:
 
     def step(self, k_cycles: int = 1, stream=None) -> int:
         return self.e.step(self.bufs, self.n, self.m, k_cycles, stream=stream, ext_cmd=tuple(self.ext_cmd))
+
+    def solve(self, max_cycles: int, tol_trans: float, tol_rot: float, stream=None):
+        """``Engine.solve`` on this batch: q moves in place (``download("q")``); returns ``(cycles [n] int32, dist [2, n])``.
+        The batch's per-cycle outputs (qdot, flags, ...) are left out of the call and keep their contents."""
+        self._ensure("cycles")
+        self._ensure("solve_dist")                                   # metres, radians (the monitor's "dist" is in degrees)
+        bufs = {k: v for k, v in self.bufs.items() if k not in _PER_CYCLE}
+        self.e.solve(bufs, self.n, self.m, max_cycles, tol_trans, tol_rot, self.t["cycles"], self.t["solve_dist"], stream=stream,
+                     ext_cmd=tuple(self.ext_cmd))
+        return self.download("cycles")[0], self.download("solve_dist")
