@@ -60,6 +60,7 @@ extern "C" {
 #define VFK_GOAL_COMPS 13        /* R_goal row-major (9), p_goal (3), slowdown distance (1) */
 #define VFK_POSE_COMPS 12        /* R row-major (9), p (3) */
 #define VFK_AUX_COMPS 12         /* auxiliary field record: type, force, 10 parameters */
+#define VFK_MAX_SHARED_OBSTACLES 1024  /* largest shared obstacle list (vfk_buffers.obst_shared = 1) */
 
 typedef enum vfk_status {
     VFK_OK = 0,
@@ -184,7 +185,14 @@ typedef struct vfk_buffers {
     void*       twist;           /* out [6]  commanded tool twist velPos, velRot (/vectorField/vector_out, scripts/vf:346-347) */
     int32_t*    flags;           /* out [1]  VFK_FLAG_*                                            */
     int32_t     n_aux;           /* slots in aux (0..64)                                           */
-    int32_t     reserved;
+    int32_t     obst_shared;     /* 0: obst / obst_ext are per instance (layout above).  1: one scene for the whole batch:
+                                    obst is dense [M][4] {x, y, z, radius} and obst_ext (or NULL) dense [M][2] {safe, order},
+                                    in the handle's precision, 128-byte aligned, M <= VFK_MAX_SHARED_OBSTACLES (larger M:
+                                    VFK_ERR_UNSUPPORTED).  Each CTA reads the list into shared memory once per launch, so
+                                    an instance costs no obstacle traffic at all; the field is bit-identical to the
+                                    per-instance path given the same list replicated to every instance.  aux stays per
+                                    instance.  This field was once reserved: C callers must zero it (ctypes structures
+                                    start zeroed).  A library that has it exports vfk_session_set_shared_obstacles. */
     const void* jp_lo;           /* [N]  per-instance joint limits the joint controller clamps its reference into --      */
     const void* jp_hi;           /* [N]  config.updateJntLimits(q) (scripts/joint_p_controller:79-89; posture-dependent on the
                                     iCub) evaluated by the caller per instance -- or NULL (both) -> the chain's static limits */
@@ -285,6 +293,12 @@ int  vfk_session_create(vfk_handle h, int64_t n_instances, int n_obstacles, int 
 int  vfk_session_set_goal(vfk_session s, const void* goal_host);            /* [13][n] */
 int  vfk_session_set_obstacles(vfk_session s, const void* obst_host,         /* [M][n][4] */
                                const void* obst_ext_host);                  /* [M][n][2] or NULL */
+/* One scene for every instance (vfk_buffers.obst_shared): copies obst_host [M][4] and obst_ext_host [M][2] (or NULL ->
+ * params.obst_safe / obst_order) to a device buffer the session owns, M in 0..VFK_MAX_SHARED_OBSTACLES.  From then on
+ * vfk_session_cycle, vfk_session_solve and vfk_session_buffers use it, until vfk_session_set_obstacles is called on a
+ * session created with n_obstacles > 0 (on one created with 0 that call stays a no-op).  A session created with
+ * n_obstacles = 0 allocates no per-instance scene. */
+int  vfk_session_set_shared_obstacles(vfk_session s, const void* obst_host, const void* obst_ext_host, int n_obstacles);
 int  vfk_session_set_aux(vfk_session s, const void* aux_host, int n_aux);   /* [n_aux * 12][n] records, or NULL / 0 to clear */
 int  vfk_session_set_q(vfk_session s, const void* q_host);                  /* [N][n] */
 int  vfk_session_set_jp_ref(vfk_session s, const void* ref_host);           /* [N][n] or NULL -> params.jp_ref */

@@ -17,6 +17,7 @@ VFK_GOAL_COMPS = 13
 VFK_POSE_COMPS = 12
 VFK_AUX_COMPS = 12
 VFK_TILE = 32
+VFK_MAX_SHARED_OBSTACLES = 1024     # largest shared obstacle list (BuffersC.obst_shared = 1)
 
 VFK_OK = 0
 VFK_ERR_INVALID = -1
@@ -35,7 +36,7 @@ EXPORTS = [
     "vfk_version", "vfk_default_params", "vfk_create", "vfk_set_params", "vfk_get_params", "vfk_chain_pattern",
     "vfk_destroy",
     "vfk_last_error", "vfk_step", "vfk_solve", "vfk_field_eval", "vfk_mix", "vfk_set_vel", "vfk_monitor", "vfk_pack", "vfk_unpack", "vfk_session_create", "vfk_session_set_goal",
-    "vfk_session_set_obstacles", "vfk_session_set_aux", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_jp_limits", "vfk_session_set_ns_input",
+    "vfk_session_set_obstacles", "vfk_session_set_shared_obstacles", "vfk_session_set_aux", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_jp_limits", "vfk_session_set_ns_input",
     "vfk_session_cycle", "vfk_session_solve", "vfk_session_enable", "vfk_session_read", "vfk_session_buffers", "vfk_session_destroy",
 ]
 
@@ -82,7 +83,7 @@ class BuffersC(C.Structure):
         ("ns_in", C.c_void_p),
         ("ns_lastvec", C.c_void_p), ("q_cmded", C.c_void_p), ("ext_cmd", C.c_void_p * 3), ("qdot_vf", C.c_void_p),
         ("qdot_ns", C.c_void_p), ("qdot_jp", C.c_void_p), ("qdot", C.c_void_p), ("cmd", C.c_void_p),
-        ("pose", C.c_void_p), ("twist", C.c_void_p), ("flags", C.c_void_p), ("n_aux", C.c_int32), ("reserved", C.c_int32),
+        ("pose", C.c_void_p), ("twist", C.c_void_p), ("flags", C.c_void_p), ("n_aux", C.c_int32), ("obst_shared", C.c_int32),
         ("jp_lo", C.c_void_p), ("jp_hi", C.c_void_p),
     ]
 
@@ -127,6 +128,7 @@ def load():
     for name in ("vfk_session_set_goal", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_ns_input"):
         getattr(lib, name).argtypes = [vp, vp]
     lib.vfk_session_set_obstacles.argtypes = [vp, vp, vp]
+    lib.vfk_session_set_shared_obstacles.argtypes = [vp, vp, vp, i32]
     lib.vfk_session_set_jp_limits.argtypes = [vp, vp, vp]
     lib.vfk_session_set_aux.argtypes = [vp, vp, i32]
     lib.vfk_session_cycle.argtypes = [vp, vp, i32, vp, vp, vp]

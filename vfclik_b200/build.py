@@ -10,10 +10,10 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libvfk.so")
 OBJ_DIR = os.path.join(os.path.dirname(HERE), "build", "obj")
-# one translation unit per (precision, joint-count group) of the cycle kernel, one per precision of its vfk_solve variant,
-# and the ABI: compiled in parallel
+# one translation unit per (precision, joint-count group) of the cycle kernel, one per precision of its vfk_solve variant and
+# of the shared-scene step and solve variants, and the ABI: compiled in parallel
 UNITS = ["vfk_api", "vfk_cycle_f32_small", "vfk_cycle_f32_large", "vfk_cycle_f64_small", "vfk_cycle_f64_large", "vfk_solve_f32",
-         "vfk_solve_f64"]
+         "vfk_solve_f64", "vfk_shared_f32", "vfk_shared_f64", "vfk_shared_solve_f32", "vfk_shared_solve_f64"]
 SOURCES = [os.path.join(CSRC, u + ".cu") for u in UNITS]
 HEADERS = [os.path.join(CSRC, f) for f in ("vfk_kernels.cuh", "vfk_math.cuh", "vfk_tma.cuh", "vfk_nullspace.cuh", "vfk_split.cuh", "vfk_ctx.cuh", "vfk_launch.cuh", "vfk_ring.cuh")] + [
     os.path.join(os.path.dirname(HERE), "include", "vfk.h")]

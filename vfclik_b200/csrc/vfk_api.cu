@@ -286,6 +286,9 @@ static int check_step(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, i
     for (int e = 0; e < 3; ++e)
         if ((rc = check_layout(h, b->ext_cmd[e], "ext_cmd", false))) return rc;
     if ((b->jp_lo == nullptr) != (b->jp_hi == nullptr)) return fail(h, VFK_ERR_INVALID, "jp_lo and jp_hi go together");
+    if (b->obst_shared != 0 && b->obst_shared != 1) return fail(h, VFK_ERR_INVALID, "obst_shared must be 0 or 1 (got %d)", b->obst_shared);
+    if (b->obst_shared && n_obst > VFK_MAX_SHARED_OBSTACLES)
+        return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, n_obst);
     return VFK_OK;
 }
 
@@ -296,6 +299,8 @@ static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, in
     if (n == 0) return 0;
     VFK_CUDA(h, cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (b->obst_shared && n_obst > 0)
+        return h->precision == 32 ? vfk_launch_shared_f32(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_shared_f64(h, b, n, n_obst, k_cycles, st, io);
     const bool small = h->n_kernel <= 7;
     if (h->precision == 32)
         return small ? vfk_launch_f32_small(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_f32_large(h, b, n, n_obst, k_cycles, st, io);
@@ -330,6 +335,8 @@ extern "C" int vfk_solve(vfk_handle h, const vfk_buffers* b, int64_t n, int n_ob
     sv.tol_rot = tol_rot;
     sv.cycles = cycles_out;
     sv.dist = dist_out;
+    if (b->obst_shared && n_obst > 0)
+        return h->precision == 32 ? vfk_solve_shared_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_shared_f64(h, b, n, n_obst, max_cycles, st, &sv);
     return h->precision == 32 ? vfk_solve_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_f64(h, b, n, n_obst, max_cycles, st, &sv);
 }
 
@@ -502,6 +509,9 @@ struct vfk_session_s {
     void *d_jp_ref, *d_ns_in, *d_jp_lo, *d_jp_hi;
     void *d_cycles, *d_dist;         // vfk_session_solve's results: cycles [1] int32, dist [2]
     char* aux_dev;                   // auxiliary field records (blocked + dense staging), grown on demand
+    char* shared_dev;                // shared scene: dense [VFK_MAX_SHARED_OBSTACLES][4], then [..][2] ext; allocated on first use
+    int shared_m;                    // obstacles in it
+    bool shared_on, shared_ext;      // cycles and solves use the shared scene; it has ext rows
     char* pin;                       // pinned host staging: q in (N rows), qdot / q out (2N rows), flags
     size_t pin_bytes;
     int launches;                    // kernels launched by the last call
@@ -577,6 +587,9 @@ extern "C" int vfk_session_create(vfk_handle h, int64_t n, int n_obst, int with_
     s->launches = 0;
     s->n_aux = 0;
     s->aux_dev = nullptr;
+    s->shared_dev = nullptr;
+    s->shared_m = 0;
+    s->shared_on = s->shared_ext = false;
     s->generation = 1;
     s->graph_exec = nullptr;
     s->graph_launches = 0;
@@ -623,9 +636,42 @@ extern "C" int vfk_session_set_obstacles(vfk_session s, const void* o, const voi
     if (s->n_obst == 0) return VFK_OK;
     if (!o) return fail(s->h, VFK_ERR_INVALID, "vfk_session_set_obstacles: null argument");
     if (s->has_ext && !ext) return fail(s->h, VFK_ERR_INVALID, "vfk_session_set_obstacles: session was created with obstacle ext rows");
+    if (s->shared_on) { s->shared_on = false; s->generation++; }      // back to the per-instance scene
     int rc = upload_blocked(s, const_cast<void*>(s->b.obst), o, s->n_obst, 4);
     if (rc == VFK_OK && s->has_ext) rc = upload_blocked(s, const_cast<void*>(s->b.obst_ext), ext, s->n_obst, 2);
     return rc;
+}
+
+// one scene for every instance: dense [M][4] host list (ext [M][2] or NULL) -> the session's shared-scene buffer
+extern "C" int vfk_session_set_shared_obstacles(vfk_session s, const void* o, const void* ext, int M) {
+    if (!s) return fail(nullptr, VFK_ERR_INVALID, "vfk_session_set_shared_obstacles: null session");
+    vfk_ctx* h = s->h;
+    if (M < 0) return fail(h, VFK_ERR_INVALID, "n_obstacles must be >= 0");
+    if (M > VFK_MAX_SHARED_OBSTACLES)
+        return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, M);
+    if (M > 0 && !o) return fail(h, VFK_ERR_INVALID, "vfk_session_set_shared_obstacles: null obstacle list");
+    VFK_CUDA(h, cudaSetDevice(h->device));
+    const size_t list = (size_t)VFK_MAX_SHARED_OBSTACLES * 4 * s->es;
+    if (!s->shared_dev) VFK_CUDA(h, cudaMalloc((void**)&s->shared_dev, list + (size_t)VFK_MAX_SHARED_OBSTACLES * 2 * s->es));
+    if (M > 0) {
+        VFK_CUDA(h, cudaMemcpyAsync(s->shared_dev, o, (size_t)M * 4 * s->es, cudaMemcpyHostToDevice, s->stream));
+        if (ext) VFK_CUDA(h, cudaMemcpyAsync(s->shared_dev + list, ext, (size_t)M * 2 * s->es, cudaMemcpyHostToDevice, s->stream));
+        VFK_CUDA(h, cudaStreamSynchronize(s->stream));
+    }
+    s->shared_on = true;
+    s->shared_m = M;
+    s->shared_ext = ext != nullptr;
+    s->generation++;
+    return VFK_OK;
+}
+
+// The scene the session's calls use: the shared list (un-offset by any tile range) or the per-instance arrays; returns M.
+static int session_scene(const vfk_session_s* s, vfk_buffers* b) {
+    if (!s->shared_on) return s->n_obst;
+    b->obst = s->shared_dev;
+    b->obst_ext = s->shared_ext ? s->shared_dev + (size_t)VFK_MAX_SHARED_OBSTACLES * 4 * s->es : nullptr;
+    b->obst_shared = 1;
+    return s->shared_m;
 }
 
 extern "C" int vfk_session_set_aux(vfk_session s, const void* aux, int n_aux) {
@@ -689,13 +735,14 @@ extern "C" int vfk_session_set_ns_input(vfk_session s, const void* x) {
     return upload_blocked(s, s->d_ns_in, x, s->h->params.ns_mode == VFK_NS_CONTROL ? 4 : s->N, 1);
 }
 
-// Offset every buffer of a blocked view to the tile range starting at tile0.
+// Offset every per-instance buffer of a blocked view to the tile range starting at tile0 (a shared scene stays whole).
 static vfk_buffers offset_view(const vfk_buffers& b, int64_t tile0, int N, int M, size_t es) {
     vfk_buffers o = b;
     auto off = [&](const void* p, size_t comps) -> void* {
         return p ? (void*)((char*)const_cast<void*>(p) + (size_t)tile0 * comps * 32 * es) : nullptr;
     };
-    o.q = off(b.q, N); o.goal = off(b.goal, 13); o.obst = off(b.obst, (size_t)((M + 1) & ~1) * 4); o.obst_ext = off(b.obst_ext, (size_t)M * 2);
+    o.q = off(b.q, N); o.goal = off(b.goal, 13);
+    if (!b.obst_shared) { o.obst = off(b.obst, (size_t)((M + 1) & ~1) * 4); o.obst_ext = off(b.obst_ext, (size_t)M * 2); }
     o.aux = off(b.aux, (size_t)b.n_aux * 12);
     o.jp_ref = off(b.jp_ref, N); o.jp_lo = off(b.jp_lo, N); o.jp_hi = off(b.jp_hi, N); o.ns_lastvec = off(b.ns_lastvec, (size_t)(ns_ctrl_vectors(N) > 0 ? ns_ctrl_vectors(N) : 1) * N); o.q_cmded = off(b.q_cmded, N);
     for (int e = 0; e < 3; ++e) o.ext_cmd[e] = off(b.ext_cmd[e], N);
@@ -713,6 +760,7 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
     const int N = s->N;
     const size_t es = s->es;
     vfk_buffers b = s->b;
+    const int M = session_scene(s, &b);
     b.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
     b.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
     b.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
@@ -740,7 +788,7 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
         const int64_t t1 = t0 + tiles_per_chunk < s->tiles ? t0 + tiles_per_chunk : s->tiles;
         const int64_t i0 = t0 * 32;
         const int64_t cnt = (t1 * 32 < s->n ? t1 * 32 : s->n) - i0;
-        vfk_buffers v = offset_view(b, t0, N, s->n_obst, es);
+        vfk_buffers v = offset_view(b, t0, N, M, es);
         if (s->have_ns_in) v.ns_in = (char*)s->d_ns_in + (size_t)t0 * ns_comps * 32 * es;
         if (src_q) {
             VFK_CUDA(h, cudaMemcpy2DAsync(stage_q + i0 * es, pitch, src_q + i0 * es, pitch, (size_t)cnt * es, N,
@@ -752,7 +800,7 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
             if ((rc = pack_dispatch(h, stage_q + i0 * es, v.q, N, 1, cnt, false, st_k, s->n)) < 0) return rc;
             launches += rc;
         }
-        if ((rc = vfk_step(h, &v, cnt, s->n_obst, k_cycles, st_k)) < 0) return rc;
+        if ((rc = vfk_step(h, &v, cnt, M, k_cycles, st_k)) < 0) return rc;
         launches += rc;
         if (dst_qd) {
             if ((rc = pack_dispatch(h, stage_qd + i0 * es, v.qdot, N, 1, cnt, true, st_k, s->n)) < 0) return rc;
@@ -823,6 +871,7 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
     void* dqd = (direct_ok && qdot_out) ? mapped(qdot_out) : nullptr;
     if (dq && (!qdot_out || dqd) && ((uintptr_t)dq % 16 == 0) && ((uintptr_t)dqd % 16 == 0)) {
         vfk_buffers b = s->b;
+        const int M = session_scene(s, &b);
         b.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
     b.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
     b.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
@@ -838,7 +887,7 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
         vfk_io io;
         io.q_src = dq; io.q_src_ld = s->n;
         io.qdot = dqd; io.qdot_ld = dqd ? s->n : 0;
-        int rc = step_impl(h, &b, s->n, s->n_obst, k_cycles, st, &io);
+        int rc = step_impl(h, &b, s->n, M, k_cycles, st, &io);
         if (rc < 0) return rc;
         int launches = rc;
         char* dst_qo = q_out ? (d_qo ? (char*)q_out : pin_qo) : nullptr;
@@ -932,7 +981,7 @@ extern "C" int vfk_session_solve(vfk_session s, const void* q_in, int max_cycles
     if ((rc = vfk_session_buffers(s, &b)) != VFK_OK) return rc;
     b.qdot_vf = b.qdot_ns = b.qdot_jp = b.qdot = b.cmd = b.pose = b.twist = nullptr;
     b.flags = nullptr;
-    if ((rc = vfk_solve(h, &b, s->n, s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
+    if ((rc = vfk_solve(h, &b, s->n, s->shared_on ? s->shared_m : s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
                         s->stream)) < 0)
         return rc;
     int launches = rc;
@@ -997,6 +1046,7 @@ extern "C" int vfk_session_read(vfk_session s, const char* what, void* out) {
 extern "C" int vfk_session_buffers(vfk_session s, vfk_buffers* out) {
     if (!s || !out) return fail(s ? s->h : nullptr, VFK_ERR_INVALID, "vfk_session_buffers: null argument");
     *out = s->b;
+    session_scene(s, out);
     out->jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
     out->jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
     out->jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
@@ -1012,6 +1062,7 @@ static void session_release(vfk_session_s* s) {
     if (s->pin) cudaFreeHost(s->pin);
     if (s->dev) cudaFree(s->dev);
     if (s->aux_dev) cudaFree(s->aux_dev);
+    if (s->shared_dev) cudaFree(s->shared_dev);
     if (s->graph_exec) cudaGraphExecDestroy(s->graph_exec);
     if (s->stream) cudaStreamDestroy(s->stream);
     for (int k = 0; k < 3; ++k) if (s->pipe[k]) cudaStreamDestroy(s->pipe[k]);

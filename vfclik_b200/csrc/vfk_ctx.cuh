@@ -70,3 +70,8 @@ int vfk_launch_f64_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst
 // The vfk_solve variants, one translation unit per precision.
 int vfk_solve_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
 int vfk_solve_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+// The shared-scene variants (vfk_buffers.obst_shared), step and solve, one translation unit each per precision.
+int vfk_launch_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
+int vfk_launch_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
+int vfk_solve_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+int vfk_solve_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);

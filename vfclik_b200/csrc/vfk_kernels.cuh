@@ -344,6 +344,40 @@ template <> struct ObstPairs<double> {
     }
 };
 
+// A scene shared by the whole batch (vfk_buffers.obst_shared) sits in shared memory once per CTA, in the form of ONE lane of
+// ObstPairs: pair p = {x0, x1, y0, y1, z0, z1, r0, r1} in T (FP32: two float4, FP64: four double2), then, with EXT, the dense
+// {safe, order} of every obstacle.  Every lane reads the same address: a broadcast, one wavefront per 16-byte read.
+template <typename T, bool EXT>
+__host__ __device__ constexpr uint32_t shared_scene_bytes(int n_obst_p, int n_obst) {
+    return (uint32_t)n_obst_p * (uint32_t)sizeof(Vec4<T>) + (EXT ? ((uint32_t)n_obst * (uint32_t)sizeof(Vec2<T>) + 15u) & ~15u : 0u);
+}
+
+template <typename T>
+__device__ __forceinline__ Vec4<T> shared_obst(const Vec4<T>* pair, int s) {
+    const T* f = reinterpret_cast<const T*>(pair) + s;
+    Vec4<T> o;
+    o.x = f[0]; o.y = f[2]; o.z = f[4]; o.w = f[6];
+    return o;
+}
+
+// The whole CTA converts the dense list [M][4] (and [M][2] ext) from global memory into that form; an odd M's padding slot
+// is zero, whose radius 0 contributes exactly 0 as in the per-instance layout.  Plain loads rather than a bulk copy: the list
+// is at most 48 KB read once per CTA from L2, and a bulk copy would want 16-byte multiples that an odd FP32 ext list is not.
+template <typename T, bool EXT>
+__device__ __forceinline__ void stage_shared_scene(const KArgs<T>& a, unsigned char* dst) {
+    const T* src = reinterpret_cast<const T*>(a.obst);
+    T* o = reinterpret_cast<T*>(dst);
+    for (int i = (int)threadIdx.x; i < a.n_obst_p * 4; i += kBlock) {    // scalar i of the pair form: pair i / 8, slot i % 2,
+        const int m = (i >> 3) * 2 + (i & 1);                              // component (i / 2) % 4
+        o[i] = m < a.n_obst ? __ldg(src + m * 4 + ((i >> 1) & 3)) : T(0);
+    }
+    if constexpr (EXT) {
+        const T* se = reinterpret_cast<const T*>(a.obst_ext);
+        T* oe = reinterpret_cast<T*>(dst + (size_t)a.n_obst_p * sizeof(Vec4<T>));
+        for (int i = (int)threadIdx.x; i < a.n_obst * 2; i += kBlock) oe[i] = __ldg(se + i);
+    }
+}
+
 // ------------------------------------------------------------------------------ field pieces
 // One decay repeller (vfl type 2): acc += (o - p)/d * (radius / max(d, safe))^order.
 // d^2 carries a 1e-30 (1e-300 in FP64) bias so that d = 0 gives a finite 1/d and a zero contribution
@@ -580,10 +614,16 @@ __device__ __forceinline__ void issue_qg(const KArgs<T>& a, int64_t tile, int bu
 // group follows its lane 0.  Once every lane of the unit is done the warp retires the unit's part of the obstacle ring
 // (ring_leave, vfk_ring.cuh) and moves on to its next unit.  The per-cycle outputs (qdot, flags, pose, ...) do not exist
 // in this mode; the state a cycle carries (q, jp_ref, ns_lastvec) freezes with the instance.
-template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool SOLVE = false>
+// SHARED = one obstacle list for the whole batch (vfk_buffers.obst_shared; G = 1 only): the CTA stages it into shared memory
+// once (stage_shared_scene) before its one CTA-wide barrier, and the repulsor loop reads it there.  The obstacle ring, its
+// mbarrier waits and refills and the L2 prefetch do not exist in this mode (n_stages = 0); an instance costs q and goal only.
+// The per-obstacle arithmetic is the per-instance path's (the same repel2 / one() calls, chunk split and order
+// specialisations), so the field is bit-identical to it on a replicated scene.
+template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool SOLVE = false, bool SHARED = false>
 __global__ void __launch_bounds__(kBlock, MINB)
 vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a) {
     using WS = WarpStage<T, N, EXT>;
+    static_assert(!SHARED || G == 1, "a shared scene runs the one-thread-per-instance shape");
     extern __shared__ __align__(128) unsigned char smem[];
     const int lane = threadIdx.x & 31;
     // read through a shuffle so that the compiler knows it is warp-uniform: tile numbers, ring positions and the addresses of
@@ -592,6 +632,8 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem) + warp * WS::kBars;
     unsigned char* region = smem + kSmemHeader + kTabBytes<T> + (size_t)warp * WS::warp_bytes(a.n_stages);
     [[maybe_unused]] const double2* sctab = reinterpret_cast<const double2*>(smem + kSmemHeader);
+    [[maybe_unused]] unsigned char* scene = smem + kSmemHeader + kTabBytes<T>;      // SHARED: the staged list, before the warps' regions
+    if constexpr (SHARED) region += shared_scene_bytes<T, EXT>(a.n_obst_p, a.n_obst);
     const uint32_t bars_a = smem_u32(bars), region_a = smem_u32(region);       // shared-window addresses, once per warp
     static_assert(G == 1 || G == kChunk, "a cooperative group takes one obstacle of a chunk per lane");
     constexpr int kSub = G == 1 ? 1 : G;                        // work units per tile (G == 8: 8 units of 4 instances)
@@ -599,7 +641,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     const int64_t n_units = n_tiles * kSub;
     const int64_t stride = (int64_t)gridDim.x * (kBlock / 32);
     int64_t unit = (int64_t)blockIdx.x * (kBlock / 32) + warp;
-    if constexpr (kTabBytes<T> == 0) {
+    if constexpr (kTabBytes<T> == 0 && !SHARED) {
         if (unit >= n_units) return;
     }
     const int ol = lane & (G - 1);                              // obstacle lane within the group
@@ -625,7 +667,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     __syncwarp();
     int64_t p_unit = unit;
     int p_u = 0, p_chunk = 0;
-    if (kTabBytes<T> == 0 || unit < n_units) {
+    if ((kTabBytes<T> == 0 && !SHARED) || unit < n_units) {
         issue_qg<T, N, EXT>(a, unit / kSub, 0, region_a, bars_a, lane, nc);
         for (int u = 0; u < S; ++u) {
             issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, u, region_a, bars_a, lane);
@@ -633,10 +675,15 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             if (++p_u == U) { p_u = 0; p_unit += stride; }
         }
     }
+    // SHARED: the scene is staged behind the first tile's copies too, and the same barrier publishes it (FP64 kernels have no
+    // table and get a barrier of their own, which is why no warp of a SHARED kernel leaves before it)
+    if constexpr (SHARED) stage_shared_scene<T, EXT>(a, scene);
     if constexpr (kTabBytes<T> != 0) {
         // the sin / cos table is built behind the first tile's copies; the only CTA-wide barrier, passed once by every warp
         // (those without work included) before any can leave
         sincos_table_fill(c.sincos, reinterpret_cast<double2*>(smem + kSmemHeader), (int)threadIdx.x, kBlock);
+        __syncthreads();
+    } else if constexpr (SHARED) {
         __syncthreads();
     }
     int c_stage = 0;
@@ -660,7 +707,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         // tile's kinematic chain (~1.5 us) a third of what it gains here.  Blocks over 32 KB (M = 256) are left to the ring,
         // which is at the copy peak there; a launch of fewer than four tiles per warp is dominated by its start, where every
         // warp's demand copies are queued at once, and skips the prefetch on its first tile (FP64 config 2: -3 % otherwise).
-        if constexpr (G == 1) {
+        if constexpr (G == 1 && !SHARED) {
             const int first = S * kChunk;
             const uint32_t bytes = a.n_obst_p > first ? (uint32_t)(a.n_obst_p - first) * 32u * (uint32_t)sizeof(Vec4<T>) : 0u;
             if (!resident && bytes != 0 && bytes <= 32768u && (it > 0 || n_units >= 4 * stride) && lane == 0)
@@ -741,16 +788,18 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                 if (__all_sync(0xffffffffu, done)) {
                     // the whole unit has stopped: wait what the ring still has in flight for it, refill those slots with the
                     // next unit's chunks, and move on.  A resident ring requests the next unit's chunks in the last cycle,
-                    // so a cycle that leaves early does that instead.
-                    const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
-                                              : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
-                    for (int i = 0; i < left; ++i) {
-                        const int stage = resident ? i : c_stage;
-                        mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
-                        __syncwarp();
-                        if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                        ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
-                        if (!resident) ring_consumed(c_stage, c_phase, S);
+                    // so a cycle that leaves early does that instead.  A shared scene has no ring: the warp just leaves.
+                    if constexpr (!SHARED) {
+                        const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
+                                                  : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
+                        for (int i = 0; i < left; ++i) {
+                            const int stage = resident ? i : c_stage;
+                            mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
+                            __syncwarp();
+                            if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
+                            ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
+                            if (!resident) ring_consumed(c_stage, c_phase, S);
+                        }
                     }
                     break;
                 }
@@ -758,19 +807,22 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             [[maybe_unused]] NegPos2 np2;                               // FP32 packed repulsor: duplicated tool position, paired sums
             [[maybe_unused]] float2 acc2[3] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) np2.set(pt);
+            // SHARED: a chunk is kChunk consecutive obstacles of the staged list, one lane's worth of each pair and ext row
+            constexpr int kPairStride = SHARED ? 2 : 64, kPlaneStride = SHARED ? 1 : 32;     // in 16-byte vectors
             for (int ch = 0; ch < a.n_chunks; ++ch) {
                 const int stage = resident ? ch : c_stage;
-                mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
-                const unsigned char* sb = region + (size_t)stage * WS::kStage;
+                if constexpr (!SHARED) mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
+                const unsigned char* sb = SHARED ? scene + (size_t)ch * (kChunk * sizeof(Vec4<T>)) : region + (size_t)stage * WS::kStage;
                 const Vec4<T>* sp = reinterpret_cast<const Vec4<T>*>(sb);                      // pair p starts at sp + p * 64
-                const Vec2<T>* se = reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot;
+                const Vec2<T>* se = SHARED ? reinterpret_cast<const Vec2<T>*>(scene + (size_t)a.n_obst_p * sizeof(Vec4<T>)) + ch * kChunk
+                                           : reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot;
                 const int n_here = ch < a.n_full ? kChunk : a.n_rem;                           // obstacles in this chunk
                 // one obstacle by its index in the chunk: scalar form (FP64, per-obstacle {safe, order}, cooperative shape)
                 auto one = [&](int m, auto order_c) {
                     constexpr int ORD = decltype(order_c)::value;
-                    const Vec4<T> o = ObstPairs<T>::load(sp + (m >> 1) * 64, slot, m & 1);
+                    const Vec4<T> o = SHARED ? shared_obst<T>(sp + (m >> 1) * 2, m & 1) : ObstPairs<T>::load(sp + (m >> 1) * 64, slot, m & 1);
                     T safe_inv = c.obst_safe_inv, order = c.obst_order;
-                    if (EXT) { const Vec2<T> e = se[m * 32]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
+                    if (EXT) { const Vec2<T> e = se[m * kPlaneStride]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
                     repel<T, ORD>(o, safe_inv, order, pt, acc);
                 };
                 if constexpr (G > 1) {
@@ -778,12 +830,13 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     if (ol < n_here) one(ol, std::integral_constant<int, 0>{});
                 } else if constexpr (sizeof(T) == 4 && !EXT) {
                     // FP32: two obstacles per step on the packed FP32 pipe; a zero-radius padding slot contributes exactly 0
-                    const float4* pl = reinterpret_cast<const float4*>(sb) + slot;
+                    const float4* pl = reinterpret_cast<const float4*>(sb) + (SHARED ? 0 : slot);
                     if (ch < a.n_full) {
                         auto full_chunk = [&](auto order_c) {
 #pragma unroll
                             for (int p = 0; p < kChunk / 2; ++p)
-                                repel2<decltype(order_c)::value>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
+                                repel2<decltype(order_c)::value>(pl[p * kPairStride], pl[p * kPairStride + kPlaneStride], c.obst_safe_inv,
+                                                                 c.obst_order, np2, acc2);
                         };
                         // decay order 20 (the reference's typical value, old/README.old:75) by five multiplications instead of
                         // MUFU lg2 / ex2: two more instructions per obstacle but two fewer on the quarter-rate XU pipe, which also
@@ -793,7 +846,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                         else full_chunk(std::integral_constant<int, 0>{});
                     } else {
                         for (int p = 0; p < (a.n_rem + 1) >> 1; ++p)
-                            repel2<0>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
+                            repel2<0>(pl[p * kPairStride], pl[p * kPairStride + kPlaneStride], c.obst_safe_inv, c.obst_order, np2, acc2);
                     }
                 } else if (ch < a.n_full) {
                     // FP64 with a uniform small-integer decay order: fixed multiplication chain instead of pow()
@@ -809,13 +862,15 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     for (int m = 0; m < a.n_rem; ++m) one(m, std::integral_constant<int, 0>{});
                 }
                 // this slot is free again: request the chunk that will occupy it S uses from now
-                if (!resident || last) {
-                    __syncwarp();
-                    if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                    if (++p_chunk == a.n_chunks) p_chunk = 0;
-                    if (++p_u == U) { p_u = 0; p_unit += stride; }
+                if constexpr (!SHARED) {
+                    if (!resident || last) {
+                        __syncwarp();
+                        if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
+                        if (++p_chunk == a.n_chunks) p_chunk = 0;
+                        if (++p_u == U) { p_u = 0; p_unit += stride; }
+                    }
+                    if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
                 }
-                if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
             }
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) {
 #pragma unroll

@@ -68,7 +68,8 @@ static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
 // spills).  Measured on B200, 1 M instances: 109.5 us vs 111.2 us per launch at K = 1 (more warps hide more HBM latency),
 // but 1.6 % slower at K = 100, where the kernel is issue-bound and the tighter register budget costs instructions.
 // SOLVE: the vfk_solve variant (vfk_kernels.cuh), with its stop rule and result buffers in `sv`.
-template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false, bool SOLVE = false>
+// SHARED: one obstacle list for the whole batch (vfk_buffers.obst_shared), staged into shared memory per CTA instead of a ring.
+template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false, bool SOLVE = false, bool SHARED = false>
 static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     KArgs<T> a;
@@ -111,12 +112,26 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
         a.dist = static_cast<T*>(sv->dist);
     }
     size_t smem = 0;
-    plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
+    if constexpr (SHARED) {
+        // The list takes at most half the bytes of the two-stage ring it replaces, so a shared kernel never has fewer resident
+        // CTAs per SM for shared memory than its per-instance twin (the same MINB gives it the same register budget).
+        static_assert(shared_scene_bytes<T, EXT>(VFK_MAX_SHARED_OBSTACLES, VFK_MAX_SHARED_OBSTACLES) * 2 <=
+                      (kBlock / 32) * 2 * WarpStage<T, N, EXT>::kStage, "shared-scene cap exceeds the ring's budget");
+        a.n_chunks = (n_obst + kChunk - 1) / kChunk;
+        a.n_stages = 0;
+        smem = kSmemHeader + kTabBytes<T> + shared_scene_bytes<T, EXT>(a.n_obst_p, n_obst) +
+               (size_t)(kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(0);
+    } else {
+        plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
+    }
     a.n_full = n_obst / kChunk;
     a.n_rem = n_obst % kChunk;
-    // resident CTAs per SM that the register allocation aims for
-    constexpr int MINB = HIOCC ? 4 : (sizeof(T) == 4 ? (N <= 10 ? 3 : 2) : (N <= 7 ? 2 : 1));
-    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, SOLVE>;
+    // resident CTAs per SM that the register allocation aims for.  The shared-scene FP32 lean solve kernels of N <= 7 ask for
+    // four: at three the LWR one took 130 registers where its per-instance twin takes 128, one resident CTA fewer (at four it
+    // takes 127 without spilling; the 7-joint generic one spills 24 bytes, as its HIOCC step twin does)
+    constexpr int MINB = (HIOCC || (SHARED && SOLVE && LEAN && sizeof(T) == 4 && N <= 7)) ? 4
+                         : (sizeof(T) == 4 ? (N <= 10 ? 3 : 2) : (N <= 7 ? 2 : 1));
+    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, SOLVE, SHARED>;
     // per (instantiation, device, smem size): opt in to > 48 KB of dynamic shared memory and ask the occupancy once
     static PlanCache plans;
     int per_sm = 0;
@@ -224,7 +239,10 @@ static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
 
 // SOLVE: the same choice of shape for vfk_solve, except that the lane-split shape has no solve variant (those calls run
 // the one-thread-per-instance kernel) and the lean kernel's output conditions do not apply.
-template <typename T, int N, class PAT, bool SOLVE = false>
+// SHARED (a shared scene, M > 0): the same choices among the one-thread-per-instance kernels -- EXT, lean / general, HIOCC --
+// but neither the cooperative shape (FP64, n <= 4096) nor the lane-split shape (FP64, 17 joints) has a shared variant:
+// those calls run the one-thread kernel, whose field they match bit for bit (DESIGN.md section 4.5).
+template <typename T, int N, class PAT, bool SOLVE = false, bool SHARED = false>
 static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
                          cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     const bool ext = b->obst_ext && n_obst > 0;
@@ -232,34 +250,34 @@ static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, i
     // Measured (scripts/latency.py, one robot, 1000 fused cycles): FP64 M = 32: 6.4 vs 7.1 us per cycle, M = 256: 23.6 vs
     // 36.3 us.  In FP32 the repeller is three MUFU instructions and the shape only adds ring overhead (3.7 vs 2.7 us),
     // so it is neither selected nor instantiated there.
-    if constexpr (sizeof(T) == 8) {
+    if constexpr (sizeof(T) == 8 && !SHARED) {
         const bool coop = n <= kCoopMaxInstances && n_obst >= 2 * kChunk && !getenv("VFK_NO_COOP");
         if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv)
                              : launch_cycle<T, N, PAT, false, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     // Two lanes per instance (vfk_split.cuh) for the FP64 17-joint kernel.
-    if constexpr (kSplit<T, N> && !SOLVE) {
+    if constexpr (kSplit<T, N> && !SOLVE && !SHARED) {
         if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N>(h, c, b, n, n_obst, k_cycles, st);
     }
     if ((SOLVE ? lean_inputs<T>(c, b) : is_lean<T>(c, b)) && h->chain.n_joints == N) {
         if constexpr (sizeof(T) == 4 && N <= 7 && !SOLVE) {
-            if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true>(h, c, b, n, n_obst, k_cycles, st, io);
+            if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true, false, SHARED>(h, c, b, n, n_obst, k_cycles, st, io);
         }
-        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
 }
 
-template <typename T, int N, bool SOLVE = false>
+template <typename T, int N, bool SOLVE = false, bool SHARED = false>
 static int dispatch_ext(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
     if constexpr (N == 7) {
-        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
     if constexpr (N >= 10) {
-        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    return dispatch_feat<T, N, GenericPattern, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    return dispatch_feat<T, N, GenericPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
 }
 

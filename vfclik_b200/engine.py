@@ -195,9 +195,8 @@ class Engine:
             stream = torch.cuda.current_stream(self.device).cuda_stream
         return C.c_void_p(stream)
 
-    def step(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, k_cycles: int = 1,
-             stream: Optional[int] = None, ext_cmd=(None, None, None)) -> int:
-        """K fused cycles on blocked device buffers; returns the number of kernels launched."""
+    @staticmethod
+    def _buffers(bufs, ext_cmd, obst_shared) -> BuffersC:
         b = BuffersC()
         for f in _BUF_FIELDS:
             setattr(b, f, _dev_ptr(bufs.get(f)))
@@ -205,25 +204,29 @@ class Engine:
             b.ext_cmd[e] = _dev_ptr(ext_cmd[e])
         aux = bufs.get("aux")
         b.n_aux = 0 if aux is None else int(aux.shape[1]) // 12
+        b.obst_shared = int(bufs.get("obst_shared", False) if obst_shared is None else obst_shared)
+        return b
+
+    def step(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, k_cycles: int = 1,
+             stream: Optional[int] = None, ext_cmd=(None, None, None), obst_shared: Optional[bool] = None) -> int:
+        """K fused cycles on blocked device buffers; returns the number of kernels launched.  ``obst_shared`` (default:
+        ``bufs["obst_shared"]``, else False) says that ``obst`` / ``obst_ext`` are one dense ``[M, 4]`` / ``[M, 2]`` list for
+        the whole batch (``vfk_buffers.obst_shared``, include/vfk.h)."""
+        b = self._buffers(bufs, ext_cmd, obst_shared)
         rc = self._check(self._lib.vfk_step(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(k_cycles),
                                             self._stream(stream)))
         self.launches += rc
         return rc
 
     def solve(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, max_cycles: int, tol_trans: float,
-              tol_rot: float, cycles_out, dist_out=None, stream: Optional[int] = None, ext_cmd=(None, None, None)) -> int:
+              tol_rot: float, cycles_out, dist_out=None, stream: Optional[int] = None, ext_cmd=(None, None, None),
+              obst_shared: Optional[bool] = None) -> int:
         """Run each instance's control loop until its tool frame is within ``tol_trans`` metres and ``tol_rot`` radians of
         its goal (strict), for at most ``max_cycles`` cycles (``vfk_solve``, include/vfk.h): the batched
         ``HandleArm.gotoFrame``.  ``cycles_out`` [1] int32 gets the cycle at which each instance stopped (-1: never),
         ``dist_out`` [2] the distance and angle to the goal at the returned q; q is updated in place.  ``bufs`` may hold
-        no per-cycle output.  Returns the number of kernels launched."""
-        b = BuffersC()
-        for f in _BUF_FIELDS:
-            setattr(b, f, _dev_ptr(bufs.get(f)))
-        for e in range(3):
-            b.ext_cmd[e] = _dev_ptr(ext_cmd[e])
-        aux = bufs.get("aux")
-        b.n_aux = 0 if aux is None else int(aux.shape[1]) // 12
+        no per-cycle output; ``obst_shared`` as in ``step``.  Returns the number of kernels launched."""
+        b = self._buffers(bufs, ext_cmd, obst_shared)
         rc = self._check(self._lib.vfk_solve(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(max_cycles),
                                              float(tol_trans), float(tol_rot), _dev_ptr(cycles_out), _dev_ptr(dist_out),
                                              self._stream(stream)))
@@ -342,6 +345,21 @@ class Session:
                 raise ValueError("obstacle ext must be [M, n, 2], got %r" % (x.shape,))
         self.e._check(self.e._lib.vfk_session_set_obstacles(self._s, _lib.np_ptr(a), None if x is None else _lib.np_ptr(x)))
 
+    def set_shared_obstacles(self, obst, obst_ext=None):
+        """One scene for every instance (``vfk_session_set_shared_obstacles``): ``obst`` ``[M, 4]`` {x, y, z, radius},
+        ``obst_ext`` ``[M, 2]`` {safe, order} or None (the parameters' values); M <= ``VFK_MAX_SHARED_OBSTACLES``.  Later
+        cycles and solves use it until ``set_obstacles`` is called (on a session created with obstacles)."""
+        a = np.ascontiguousarray(obst, dtype=self.e.np_dtype)
+        if a.ndim != 2 or a.shape[1] != 4:
+            raise ValueError("shared obstacles must be [M, 4], got %r" % (a.shape,))
+        x = None
+        if obst_ext is not None:
+            x = np.ascontiguousarray(obst_ext, dtype=self.e.np_dtype)
+            if x.shape != (a.shape[0], 2):
+                raise ValueError("shared obstacle ext must be [M, 2], got %r" % (x.shape,))
+        self.e._check(self.e._lib.vfk_session_set_shared_obstacles(self._s, _lib.np_ptr(a), None if x is None else _lib.np_ptr(x),
+                                                                   int(a.shape[0])))
+
     def set_aux(self, aux):
         """Auxiliary field records ``[n_aux, 12, n]`` ({type, force, 10 params}; types 4 and 5), or None to clear."""
         if aux is None:
@@ -448,17 +466,28 @@ class DeviceBatch:
     the multi-GPU driver).  ``upload`` takes dense numpy arrays (``[comps, n]``; obstacles
     ``[M, n, 4]``, ext ``[M, n, 2]``), moves them to the device and converts them with the
     library's pack kernel; ``download`` converts back.  ``bufs`` is what ``Engine.step`` takes.
+    ``shared_obstacles=True``: one scene for the whole batch, ``obst`` dense ``[M, 4]`` and ``obst_ext`` ``[M, 2]`` on the
+    device as they are uploaded (``vfk_buffers.obst_shared``).
     """
 
     _ROWS = {"goal": 13, "pose": 12, "flags": 1, "twist": 6, "track": 8, "dist": 2, "mon_f": 32, "solve_dist": 2}
 
     def __init__(self, engine: Engine, n_instances: int, n_obstacles: int, obst_ext: bool = False,
-                 outputs=("qdot",), inputs=()):
+                 outputs=("qdot",), inputs=(), shared_obstacles: bool = False):
         self.e, self.n, self.m = engine, int(n_instances), int(n_obstacles)
+        self.shared = bool(shared_obstacles)
         self.t: Dict[str, object] = {}
         self.t["q"] = engine.alloc(engine.n_joints, self.n)
         self.t["goal"] = engine.alloc(13, self.n)
-        if self.m:
+        if self.m and self.shared:
+            import torch
+            if self.m > _lib.VFK_MAX_SHARED_OBSTACLES:
+                raise ValueError("a shared obstacle list holds at most %d obstacles" % _lib.VFK_MAX_SHARED_OBSTACLES)
+            dev = "cuda:%d" % engine.device
+            self.t["obst"] = torch.zeros((self.m, 4), dtype=engine.torch_dtype, device=dev)
+            if obst_ext:
+                self.t["obst_ext"] = torch.zeros((self.m, 2), dtype=engine.torch_dtype, device=dev)
+        elif self.m:
             self.t["obst"] = engine.alloc(self.m, self.n, width=4)
             if obst_ext:
                 self.t["obst_ext"] = engine.alloc(self.m, self.n, width=2)
@@ -508,6 +537,14 @@ class DeviceBatch:
         return self.t["aux"]
 
     def upload(self, name: str, arr: np.ndarray):
+        if self.shared and name in ("obst", "obst_ext"):           # dense on both sides: a plain copy
+            import torch
+            t = self._ensure(name)
+            a = np.ascontiguousarray(arr, dtype=self.e.np_dtype)
+            if a.shape != tuple(t.shape):
+                raise ValueError("%s: expected %r, got %r" % (name, tuple(t.shape), a.shape))
+            t.copy_(torch.from_numpy(a))
+            return t
         t = self._ensure(name)
         width = {"obst": 4, "obst_ext": 2}.get(name, 1)
         a = np.asarray(arr)
@@ -522,6 +559,8 @@ class DeviceBatch:
         """Blocked device tensor -> dense numpy ``[comps, n]`` (``[M, n, width]`` for obstacles)."""
         import torch
         t = self.t[name]
+        if self.shared and name in ("obst", "obst_ext"):
+            return t.cpu().numpy()
         if t.dtype == torch.int32:                                   # int32 arrays: un-block on the host
             a = t.cpu().numpy()                                      # [tiles, comps, 32]
             return np.ascontiguousarray(a.transpose(1, 0, 2).reshape(a.shape[1], -1)[:, :self.n])
@@ -537,6 +576,8 @@ class DeviceBatch:
         the pair-interleaved blocked array on the device (for sampling batches too large to convert as a whole)."""
         import torch
         t = self.t["obst"]
+        if self.shared:
+            return np.repeat(t.cpu().numpy()[:, None], len(idx), axis=1)
         ti = torch.as_tensor(np.asarray(idx), device=t.device)
         tiles, mp, k = t.shape[0], t.shape[1], int(ti.numel())
         if self.e.precision == 32:       # pair = planes {x0, x1, y0, y1}, {z0, z1, r0, r1} of 32 lanes x float4
@@ -549,7 +590,10 @@ class DeviceBatch:
 
     @property
     def bufs(self) -> Dict[str, object]:
-        return {k: v for k, v in self.t.items() if k in _BUF_FIELDS}
+        b = {k: v for k, v in self.t.items() if k in _BUF_FIELDS}
+        if self.shared:
+            b["obst_shared"] = True
+        return b
 
     def monitor(self, stream=None) -> int:
         """Run ``vfk_monitor`` on this batch's pose / twist / goal (allocates state and outputs on first use)."""

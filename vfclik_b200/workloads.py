@@ -69,6 +69,26 @@ def random_batch(chain: ChainDesc, n_instances: int, n_obstacles: int, seed: int
     return out
 
 
+def shared_scene_batch(chain: ChainDesc, n_instances: int, n_obstacles: int, seed: int, dtype=np.float64,
+                       obst_ext: bool = False, **kw):
+    """One workcell for the whole batch (``vfk_buffers.obst_shared``): per-instance starts and goals, one obstacle list.
+    Starts and goals are :func:`random_batch`'s with ``seed``; the scene is the obstacle list :func:`random_batch` draws for
+    a single instance with ``seed + 1``, so every distribution is :func:`random_batch`'s.
+
+    Returns dict(q [N,I], goal [13,I], obst [M,4] {x,y,z,radius} [, obst_ext [M,2] {safe, order}]) of ``dtype``."""
+    w = random_batch(chain, n_instances, 0, seed, dtype=dtype, **kw)
+    scene = random_batch(chain, 1, n_obstacles, seed + 1, dtype=dtype, obst_ext=obst_ext, **kw)
+    out = dict(q=w["q"], goal=w["goal"], obst=np.ascontiguousarray(scene["obst"][:, 0]))
+    if obst_ext:
+        out["obst_ext"] = np.ascontiguousarray(scene["obst_ext"][:, 0])
+    return out
+
+
+def replicate_scene(obst: np.ndarray, n_instances: int) -> np.ndarray:
+    """A shared list ``[M, C]`` as the per-instance array ``[M, n, C]`` that gives every instance the same scene."""
+    return np.ascontiguousarray(np.broadcast_to(obst[:, None, :], (obst.shape[0], int(n_instances), obst.shape[1])))
+
+
 def random_batch_device(engine, n_instances: int, n_obstacles: int, seed: int, slowdown: float = 0.05, box: float = 0.8):
     """Same distributions as :func:`random_batch`, drawn on the GPU with torch's generator (large shapes:
     config 4's 2M x 256 obstacles per GPU would take minutes and 8 GB of host memory through numpy).
