@@ -53,14 +53,24 @@
 extern "C" {
 #endif
 
-#define VFK_VERSION 100          /* 0.1.0 */
+/* 0.1.0.  vfk_buffers grew by the mixed-scene fields at its end (VFK_OBST_MIXED) without a new version: the library
+ * reads them only when obst_shared == VFK_OBST_MIXED, which no caller built against the shorter struct can set, and
+ * vfk_session_buffers writes them only for a session switched to that mode, so an older caller's struct is never read
+ * or written past its end. */
+#define VFK_VERSION 100
 #define VFK_MAX_JOINTS 17
 #define VFK_TILE 32              /* instances per layout tile */
 #define VFK_N_PORTS 6            /* mixer inputs, order of scripts/bridge:593-596 */
 #define VFK_GOAL_COMPS 13        /* R_goal row-major (9), p_goal (3), slowdown distance (1) */
 #define VFK_POSE_COMPS 12        /* R row-major (9), p (3) */
 #define VFK_AUX_COMPS 12         /* auxiliary field record: type, force, 10 parameters */
-#define VFK_MAX_SHARED_OBSTACLES 1024  /* largest shared obstacle list (vfk_buffers.obst_shared = 1) */
+#define VFK_MAX_SHARED_OBSTACLES 1024  /* largest shared obstacle list (vfk_buffers.obst_shared = 1 or 2) */
+
+/* vfk_buffers.obst_shared: which obstacle lists a call uses */
+enum { VFK_OBST_PER_INSTANCE = 0,  /* obst / obst_ext per instance (blocked layout above) */
+       VFK_OBST_SHARED = 1,        /* obst / obst_ext: one dense list for the whole batch */
+       VFK_OBST_MIXED = 2 };       /* obst / obst_ext per instance (n_obstacles of them) plus shared_obst / shared_obst_ext,
+                                      one dense list of n_shared_obst for the whole batch */
 
 typedef enum vfk_status {
     VFK_OK = 0,
@@ -185,17 +195,30 @@ typedef struct vfk_buffers {
     void*       twist;           /* out [6]  commanded tool twist velPos, velRot (/vectorField/vector_out, scripts/vf:346-347) */
     int32_t*    flags;           /* out [1]  VFK_FLAG_*                                            */
     int32_t     n_aux;           /* slots in aux (0..64)                                           */
-    int32_t     obst_shared;     /* 0: obst / obst_ext are per instance (layout above).  1: one scene for the whole batch:
-                                    obst is dense [M][4] {x, y, z, radius} and obst_ext (or NULL) dense [M][2] {safe, order},
-                                    in the handle's precision, 128-byte aligned, M <= VFK_MAX_SHARED_OBSTACLES (larger M:
-                                    VFK_ERR_UNSUPPORTED).  Each CTA reads the list into shared memory once per launch, so
-                                    an instance costs no obstacle traffic at all; the field is bit-identical to the
-                                    per-instance path given the same list replicated to every instance.  aux stays per
-                                    instance.  This field was once reserved: C callers must zero it (ctypes structures
-                                    start zeroed).  A library that has it exports vfk_session_set_shared_obstacles. */
+    int32_t     obst_shared;     /* VFK_OBST_*.  0: obst / obst_ext are per instance (layout above).  1: one scene for the
+                                    whole batch: obst is dense [M][4] {x, y, z, radius} and obst_ext (or NULL) dense [M][2]
+                                    {safe, order}, in the handle's precision, 128-byte aligned, M <= VFK_MAX_SHARED_OBSTACLES
+                                    (larger M: VFK_ERR_UNSUPPORTED).  Each CTA reads the list into shared memory once per
+                                    launch, so an instance costs no obstacle traffic at all; the field is bit-identical to the
+                                    per-instance path given the same list replicated to every instance.  2: both -- obst /
+                                    obst_ext per instance as in mode 0 (n_obstacles = Mi of them) and the shared list in
+                                    shared_obst / shared_obst_ext below; see those fields.  aux stays per instance.  This field
+                                    was once reserved: C callers must zero it (ctypes structures start zeroed).  A library
+                                    that has it exports vfk_session_set_shared_obstacles (modes 0 / 1) and
+                                    vfk_session_use_obstacles (mode 2). */
     const void* jp_lo;           /* [N]  per-instance joint limits the joint controller clamps its reference into --      */
     const void* jp_hi;           /* [N]  config.updateJntLimits(q) (scripts/joint_p_controller:79-89; posture-dependent on the
                                     iCub) evaluated by the caller per instance -- or NULL (both) -> the chain's static limits */
+    /* Read only when obst_shared == VFK_OBST_MIXED (appended fields: a caller built against the struct without them never
+     * sets that mode).  The field of an instance sums its own Mi obstacles first, then the Ms shared ones, as if its list
+     * were [own ; shared]; it equals mode 0 on that concatenated list bit for bit when Mi is a multiple of 8 (the repulsor
+     * works in chunks of 8) and to rounding otherwise.  Ms = 0 runs exactly the per-instance call, Mi = 0 exactly mode 1. */
+    const void* shared_obst;     /* dense [Ms][4] {x, y, z, radius}, 128-byte aligned; required in this mode even when Ms = 0
+                                    (a mode-2 call without it is refused rather than read a shared-only obst as per instance) */
+    const void* shared_obst_ext; /* dense [Ms][2] {safe, order}, 128-byte aligned, or NULL.  With both lists non-empty, obst_ext
+                                    and shared_obst_ext come both or neither (VFK_ERR_INVALID otherwise) */
+    int32_t     n_shared_obst;   /* Ms in 0..VFK_MAX_SHARED_OBSTACLES (< 0: VFK_ERR_INVALID; larger: VFK_ERR_UNSUPPORTED) */
+    int32_t     reserved2;       /* must be 0 */
 } vfk_buffers;
 
 typedef struct vfk_ctx* vfk_handle;
@@ -247,6 +270,12 @@ int  vfk_solve(vfk_handle h, const vfk_buffers* bufs, int64_t n_instances, int n
 int  vfk_field_eval(vfk_handle h, const void* pose_in, const void* goal, const void* obst,
                     const void* obst_ext, const void* aux, int n_aux, void* twist_out,
                     int64_t n_instances, int n_obstacles, void* stream);
+/* The same query on the scene a vfk_step call would use: goal, obst, obst_ext, aux, n_aux, obst_shared and, in
+ * VFK_OBST_MIXED, the shared_* fields are taken from `scene` (every other field is ignored); n_obstacles means what it
+ * means to vfk_step (mode 1: the shared list's length; mode 2: the per-instance count).  Sums the own obstacles, then
+ * the shared ones, one at a time: bit-identical to vfk_field_eval on the replicated or concatenated per-instance list. */
+int  vfk_field_eval_scene(vfk_handle h, const void* pose_in, const vfk_buffers* scene, int64_t n_instances, int n_obstacles,
+                          void* twist_out, void* stream);
 
 /* Weighted sum of command ports (src/command_mixer.py:78-82) on device buffers:
  * out(c, i) = sum_p w[p] * cmds[p](c, i); cmds[p] may be NULL (skipped); nan_flags [1] optional. */
@@ -299,6 +328,11 @@ int  vfk_session_set_obstacles(vfk_session s, const void* obst_host,         /* 
  * session created with n_obstacles > 0 (on one created with 0 that call stays a no-op).  A session created with
  * n_obstacles = 0 allocates no per-instance scene. */
 int  vfk_session_set_shared_obstacles(vfk_session s, const void* obst_host, const void* obst_ext_host, int n_obstacles);
+/* Which lists vfk_session_cycle, vfk_session_solve and vfk_session_buffers use: VFK_OBST_PER_INSTANCE,
+ * VFK_OBST_SHARED (needs a shared list) or VFK_OBST_MIXED (needs a session created with n_obstacles > 0 and a shared list;
+ * when both are non-empty their ext rows come both or neither).  Otherwise VFK_ERR_INVALID.  The two setters above
+ * keep their side effects (set_obstacles selects mode 0, set_shared_obstacles mode 1): call this after both. */
+int  vfk_session_use_obstacles(vfk_session s, int mode);
 int  vfk_session_set_aux(vfk_session s, const void* aux_host, int n_aux);   /* [n_aux * 12][n] records, or NULL / 0 to clear */
 int  vfk_session_set_q(vfk_session s, const void* q_host);                  /* [N][n] */
 int  vfk_session_set_jp_ref(vfk_session s, const void* ref_host);           /* [N][n] or NULL -> params.jp_ref */

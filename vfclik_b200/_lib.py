@@ -17,7 +17,9 @@ VFK_GOAL_COMPS = 13
 VFK_POSE_COMPS = 12
 VFK_AUX_COMPS = 12
 VFK_TILE = 32
-VFK_MAX_SHARED_OBSTACLES = 1024     # largest shared obstacle list (BuffersC.obst_shared = 1)
+VFK_MAX_SHARED_OBSTACLES = 1024     # largest shared obstacle list (BuffersC.obst_shared = 1 or 2)
+# BuffersC.obst_shared: per-instance lists, one list for the whole batch, or both (the mixed fields at the struct's end)
+VFK_OBST_PER_INSTANCE, VFK_OBST_SHARED, VFK_OBST_MIXED = 0, 1, 2
 
 VFK_OK = 0
 VFK_ERR_INVALID = -1
@@ -35,8 +37,8 @@ LIB_PATH = os.environ.get("VFK_LIB") or os.path.join(os.path.dirname(os.path.abs
 EXPORTS = [
     "vfk_version", "vfk_default_params", "vfk_create", "vfk_set_params", "vfk_get_params", "vfk_chain_pattern",
     "vfk_destroy",
-    "vfk_last_error", "vfk_step", "vfk_solve", "vfk_field_eval", "vfk_mix", "vfk_set_vel", "vfk_monitor", "vfk_pack", "vfk_unpack", "vfk_session_create", "vfk_session_set_goal",
-    "vfk_session_set_obstacles", "vfk_session_set_shared_obstacles", "vfk_session_set_aux", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_jp_limits", "vfk_session_set_ns_input",
+    "vfk_last_error", "vfk_step", "vfk_solve", "vfk_field_eval", "vfk_field_eval_scene", "vfk_mix", "vfk_set_vel", "vfk_monitor", "vfk_pack", "vfk_unpack", "vfk_session_create", "vfk_session_set_goal",
+    "vfk_session_set_obstacles", "vfk_session_set_shared_obstacles", "vfk_session_use_obstacles", "vfk_session_set_aux", "vfk_session_set_q", "vfk_session_set_jp_ref", "vfk_session_set_jp_limits", "vfk_session_set_ns_input",
     "vfk_session_cycle", "vfk_session_solve", "vfk_session_enable", "vfk_session_read", "vfk_session_buffers", "vfk_session_destroy",
 ]
 
@@ -85,6 +87,8 @@ class BuffersC(C.Structure):
         ("qdot_ns", C.c_void_p), ("qdot_jp", C.c_void_p), ("qdot", C.c_void_p), ("cmd", C.c_void_p),
         ("pose", C.c_void_p), ("twist", C.c_void_p), ("flags", C.c_void_p), ("n_aux", C.c_int32), ("obst_shared", C.c_int32),
         ("jp_lo", C.c_void_p), ("jp_hi", C.c_void_p),
+        # read by the library only when obst_shared == VFK_OBST_MIXED
+        ("shared_obst", C.c_void_p), ("shared_obst_ext", C.c_void_p), ("n_shared_obst", C.c_int32), ("reserved2", C.c_int32),
     ]
 
 
@@ -119,6 +123,7 @@ def load():
     lib.vfk_step.argtypes = [vp, C.POINTER(BuffersC), i64, i32, i32, vp]
     lib.vfk_solve.argtypes = [vp, C.POINTER(BuffersC), i64, i32, i32, C.c_double, C.c_double, vp, vp, vp]
     lib.vfk_field_eval.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, i64, i32, vp]
+    lib.vfk_field_eval_scene.argtypes = [vp, vp, C.POINTER(BuffersC), i64, i32, vp, vp]
     lib.vfk_mix.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_double), i32, i32, vp, vp, i64, vp]
     lib.vfk_set_vel.argtypes = [vp, vp, vp, vp, C.c_double, i32, vp, vp, i32, i64, vp]
     lib.vfk_monitor.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, vp]
@@ -129,6 +134,7 @@ def load():
         getattr(lib, name).argtypes = [vp, vp]
     lib.vfk_session_set_obstacles.argtypes = [vp, vp, vp]
     lib.vfk_session_set_shared_obstacles.argtypes = [vp, vp, vp, i32]
+    lib.vfk_session_use_obstacles.argtypes = [vp, i32]
     lib.vfk_session_set_jp_limits.argtypes = [vp, vp, vp]
     lib.vfk_session_set_aux.argtypes = [vp, vp, i32]
     lib.vfk_session_cycle.argtypes = [vp, vp, i32, vp, vp, vp]

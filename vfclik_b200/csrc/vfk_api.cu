@@ -267,6 +267,30 @@ static int check_layout(vfk_ctx* h, const void* ptr, const char* name, bool requ
     return VFK_OK;
 }
 
+// The scene's mode and lists (vfk_step, vfk_solve, vfk_field_eval_scene).  n_obst: the per-instance count (mode 0 / 2) or
+// the shared list's (mode 1).
+static int check_scene(vfk_ctx* h, const vfk_buffers* b, int n_obst) {
+    const int mode = b->obst_shared;
+    if (mode != VFK_OBST_PER_INSTANCE && mode != VFK_OBST_SHARED && mode != VFK_OBST_MIXED)
+        return fail(h, VFK_ERR_INVALID, "obst_shared must be 0, 1 or 2 (got %d)", mode);
+    if (mode == VFK_OBST_SHARED && n_obst > VFK_MAX_SHARED_OBSTACLES)
+        return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, n_obst);
+    if (mode != VFK_OBST_MIXED) return VFK_OK;
+    const int ms = b->n_shared_obst;
+    if (ms < 0) return fail(h, VFK_ERR_INVALID, "n_shared_obst must be >= 0 (got %d)", ms);
+    if (ms > VFK_MAX_SHARED_OBSTACLES)
+        return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, ms);
+    if (b->reserved2 != 0) return fail(h, VFK_ERR_INVALID, "vfk_buffers.reserved2 must be 0");
+    int rc;
+    // shared_obst is required even when it holds no obstacle: mode 2 without it is most likely a shared-only buffer set (a
+    // dense obst) under the wrong mode, whose obst would otherwise be read as a per-instance array
+    if ((rc = check_layout(h, b->shared_obst, "shared_obst", true)) || (rc = check_layout(h, b->shared_obst_ext, "shared_obst_ext", false)))
+        return rc;
+    if (n_obst > 0 && ms > 0 && (b->obst_ext == nullptr) != (b->shared_obst_ext == nullptr))
+        return fail(h, VFK_ERR_INVALID, "obst_ext and shared_obst_ext go together in a mixed scene");
+    return VFK_OK;
+}
+
 // The argument checks vfk_step and vfk_solve share.
 static int check_step(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles) {
     if (n < 0) return fail(h, VFK_ERR_INVALID, "n_instances must be >= 0 (got %lld)", (long long)n);
@@ -286,10 +310,14 @@ static int check_step(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, i
     for (int e = 0; e < 3; ++e)
         if ((rc = check_layout(h, b->ext_cmd[e], "ext_cmd", false))) return rc;
     if ((b->jp_lo == nullptr) != (b->jp_hi == nullptr)) return fail(h, VFK_ERR_INVALID, "jp_lo and jp_hi go together");
-    if (b->obst_shared != 0 && b->obst_shared != 1) return fail(h, VFK_ERR_INVALID, "obst_shared must be 0 or 1 (got %d)", b->obst_shared);
-    if (b->obst_shared && n_obst > VFK_MAX_SHARED_OBSTACLES)
-        return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, n_obst);
-    return VFK_OK;
+    return check_scene(h, b, n_obst);
+}
+
+// The batch-wide list of a shared or mixed scene (n = 0: none).  The mixed fields are read in VFK_OBST_MIXED only.
+static vfk_shared_scene shared_scene_of(const vfk_buffers* b, int n_obst) {
+    if (b->obst_shared == VFK_OBST_SHARED) return vfk_shared_scene{b->obst, b->obst_ext, n_obst};
+    if (b->obst_shared == VFK_OBST_MIXED) return vfk_shared_scene{b->shared_obst, b->shared_obst_ext, b->n_shared_obst};
+    return vfk_shared_scene{nullptr, nullptr, 0};
 }
 
 static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream, const vfk_io* io) {
@@ -299,8 +327,14 @@ static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, in
     if (n == 0) return 0;
     VFK_CUDA(h, cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (b->obst_shared && n_obst > 0)
-        return h->precision == 32 ? vfk_launch_shared_f32(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_shared_f64(h, b, n, n_obst, k_cycles, st, io);
+    // a shared or mixed scene with a non-empty shared list runs the SHARED kernels (own list: mode 2's per-instance one);
+    // mode 2 without shared obstacles is exactly the per-instance call
+    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
+    if (sh.n > 0) {
+        const int own = b->obst_shared == VFK_OBST_MIXED ? n_obst : 0;
+        return h->precision == 32 ? vfk_launch_shared_f32(h, b, n, own, &sh, k_cycles, st, io) : vfk_launch_shared_f64(h, b, n, own, &sh, k_cycles, st, io);
+    }
+    if (b->obst_shared == VFK_OBST_SHARED) n_obst = 0;
     const bool small = h->n_kernel <= 7;
     if (h->precision == 32)
         return small ? vfk_launch_f32_small(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_f32_large(h, b, n, n_obst, k_cycles, st, io);
@@ -335,9 +369,33 @@ extern "C" int vfk_solve(vfk_handle h, const vfk_buffers* b, int64_t n, int n_ob
     sv.tol_rot = tol_rot;
     sv.cycles = cycles_out;
     sv.dist = dist_out;
-    if (b->obst_shared && n_obst > 0)
-        return h->precision == 32 ? vfk_solve_shared_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_shared_f64(h, b, n, n_obst, max_cycles, st, &sv);
+    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
+    if (sh.n > 0) {
+        const int own = b->obst_shared == VFK_OBST_MIXED ? n_obst : 0;
+        return h->precision == 32 ? vfk_solve_shared_f32(h, b, n, own, &sh, max_cycles, st, &sv) : vfk_solve_shared_f64(h, b, n, own, &sh, max_cycles, st, &sv);
+    }
+    if (b->obst_shared == VFK_OBST_SHARED) n_obst = 0;
     return h->precision == 32 ? vfk_solve_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_f64(h, b, n, n_obst, max_cycles, st, &sv);
+}
+
+// The field query's launch: n_obst per-instance obstacles (blocked) and the shared list `sh` (dense).
+static int field_launch(vfk_ctx* h, const void* pose_in, const void* goal, const void* obst, const void* obst_ext, const void* aux,
+                        int n_aux, void* twist_out, int64_t n, int n_obst, const vfk_shared_scene& sh, void* stream) {
+    VFK_CUDA(h, cudaSetDevice(h->device));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const unsigned grid = (unsigned)((n + kSmallBlock - 1) / kSmallBlock);
+    if (h->precision == 32)
+        vfk_field_kernel<float><<<grid, kSmallBlock, 0, st>>>(h->cf, (const float*)pose_in, (const float*)goal,
+                                                         (const Vec4<float>*)obst, (const Vec2<float>*)obst_ext,
+                                                         (const float*)aux, n_aux, (float*)twist_out, n, n_obst,
+                                                         (const float*)sh.obst, (const float*)sh.obst_ext, sh.n);
+    else
+        vfk_field_kernel<double><<<grid, kSmallBlock, 0, st>>>(h->cd, (const double*)pose_in, (const double*)goal,
+                                                          (const Vec4<double>*)obst, (const Vec2<double>*)obst_ext,
+                                                          (const double*)aux, n_aux, (double*)twist_out, n, n_obst,
+                                                          (const double*)sh.obst, (const double*)sh.obst_ext, sh.n);
+    VFK_CUDA(h, cudaGetLastError());
+    return 1;
 }
 
 extern "C" int vfk_field_eval(vfk_handle h, const void* pose_in, const void* goal, const void* obst, const void* obst_ext,
@@ -348,19 +406,23 @@ extern "C" int vfk_field_eval(vfk_handle h, const void* pose_in, const void* goa
     if (n_aux < 0 || n_aux > 64) return fail(h, VFK_ERR_INVALID, "n_aux must be in 0..64");
     if (n_aux == 0) aux = nullptr;
     if (n == 0) return 0;
-    VFK_CUDA(h, cudaSetDevice(h->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const unsigned grid = (unsigned)((n + kSmallBlock - 1) / kSmallBlock);
-    if (h->precision == 32)
-        vfk_field_kernel<float><<<grid, kSmallBlock, 0, st>>>(h->cf, (const float*)pose_in, (const float*)goal,
-                                                         (const Vec4<float>*)obst, (const Vec2<float>*)obst_ext,
-                                                         (const float*)aux, n_aux, (float*)twist_out, n, n_obst);
-    else
-        vfk_field_kernel<double><<<grid, kSmallBlock, 0, st>>>(h->cd, (const double*)pose_in, (const double*)goal,
-                                                          (const Vec4<double>*)obst, (const Vec2<double>*)obst_ext,
-                                                          (const double*)aux, n_aux, (double*)twist_out, n, n_obst);
-    VFK_CUDA(h, cudaGetLastError());
-    return 1;
+    return field_launch(h, pose_in, goal, obst, obst_ext, aux, n_aux, twist_out, n, n_obst, vfk_shared_scene{nullptr, nullptr, 0}, stream);
+}
+
+extern "C" int vfk_field_eval_scene(vfk_handle h, const void* pose_in, const vfk_buffers* b, int64_t n, int n_obst, void* twist_out,
+                                    void* stream) {
+    if (!h || !pose_in || !b || !b->goal || !twist_out) return fail(h, VFK_ERR_INVALID, "vfk_field_eval_scene: null argument");
+    if (n < 0) return fail(h, VFK_ERR_INVALID, "n_instances must be >= 0");
+    if (n_obst < 0) return fail(h, VFK_ERR_INVALID, "n_obstacles must be >= 0");
+    if (b->n_aux < 0 || b->n_aux > 64) return fail(h, VFK_ERR_INVALID, "n_aux must be in 0..64");
+    int rc;
+    if ((rc = check_scene(h, b, n_obst))) return rc;
+    if ((rc = check_layout(h, b->obst, "obst", n_obst > 0)) || (rc = check_layout(h, b->obst_ext, "obst_ext", false))) return rc;
+    if (n == 0) return 0;
+    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
+    const bool own = b->obst_shared != VFK_OBST_SHARED;
+    return field_launch(h, pose_in, b->goal, own ? b->obst : nullptr, own ? b->obst_ext : nullptr, b->n_aux > 0 ? b->aux : nullptr, b->n_aux,
+                        twist_out, n, own ? n_obst : 0, sh, stream);
 }
 
 extern "C" int vfk_mix(vfk_handle h, const void* const* cmds, const double* w, int n_ports, int n_channels, void* out,
@@ -511,7 +573,8 @@ struct vfk_session_s {
     char* aux_dev;                   // auxiliary field records (blocked + dense staging), grown on demand
     char* shared_dev;                // shared scene: dense [VFK_MAX_SHARED_OBSTACLES][4], then [..][2] ext; allocated on first use
     int shared_m;                    // obstacles in it
-    bool shared_on, shared_ext;      // cycles and solves use the shared scene; it has ext rows
+    bool shared_ext;                 // it has ext rows
+    int obst_mode;                   // VFK_OBST_*: the lists cycles and solves use
     char* pin;                       // pinned host staging: q in (N rows), qdot / q out (2N rows), flags
     size_t pin_bytes;
     int launches;                    // kernels launched by the last call
@@ -589,7 +652,8 @@ extern "C" int vfk_session_create(vfk_handle h, int64_t n, int n_obst, int with_
     s->aux_dev = nullptr;
     s->shared_dev = nullptr;
     s->shared_m = 0;
-    s->shared_on = s->shared_ext = false;
+    s->shared_ext = false;
+    s->obst_mode = VFK_OBST_PER_INSTANCE;
     s->generation = 1;
     s->graph_exec = nullptr;
     s->graph_launches = 0;
@@ -636,7 +700,7 @@ extern "C" int vfk_session_set_obstacles(vfk_session s, const void* o, const voi
     if (s->n_obst == 0) return VFK_OK;
     if (!o) return fail(s->h, VFK_ERR_INVALID, "vfk_session_set_obstacles: null argument");
     if (s->has_ext && !ext) return fail(s->h, VFK_ERR_INVALID, "vfk_session_set_obstacles: session was created with obstacle ext rows");
-    if (s->shared_on) { s->shared_on = false; s->generation++; }      // back to the per-instance scene
+    if (s->obst_mode != VFK_OBST_PER_INSTANCE) { s->obst_mode = VFK_OBST_PER_INSTANCE; s->generation++; }  // back to the per-instance scene
     int rc = upload_blocked(s, const_cast<void*>(s->b.obst), o, s->n_obst, 4);
     if (rc == VFK_OK && s->has_ext) rc = upload_blocked(s, const_cast<void*>(s->b.obst_ext), ext, s->n_obst, 2);
     return rc;
@@ -658,20 +722,45 @@ extern "C" int vfk_session_set_shared_obstacles(vfk_session s, const void* o, co
         if (ext) VFK_CUDA(h, cudaMemcpyAsync(s->shared_dev + list, ext, (size_t)M * 2 * s->es, cudaMemcpyHostToDevice, s->stream));
         VFK_CUDA(h, cudaStreamSynchronize(s->stream));
     }
-    s->shared_on = true;
+    s->obst_mode = VFK_OBST_SHARED;
     s->shared_m = M;
     s->shared_ext = ext != nullptr;
     s->generation++;
     return VFK_OK;
 }
 
-// The scene the session's calls use: the shared list (un-offset by any tile range) or the per-instance arrays; returns M.
+// Which lists the session's calls use (vfk_session_use_obstacles): the per-instance arrays, the shared list or both.
+extern "C" int vfk_session_use_obstacles(vfk_session s, int mode) {
+    if (!s) return fail(nullptr, VFK_ERR_INVALID, "vfk_session_use_obstacles: null session");
+    vfk_ctx* h = s->h;
+    if (mode != VFK_OBST_PER_INSTANCE && mode != VFK_OBST_SHARED && mode != VFK_OBST_MIXED)
+        return fail(h, VFK_ERR_INVALID, "vfk_session_use_obstacles: mode must be 0, 1 or 2 (got %d)", mode);
+    if (mode != VFK_OBST_PER_INSTANCE && !s->shared_dev)
+        return fail(h, VFK_ERR_INVALID, "vfk_session_use_obstacles: no shared obstacle list was set (vfk_session_set_shared_obstacles)");
+    if (mode == VFK_OBST_MIXED && s->n_obst == 0)
+        return fail(h, VFK_ERR_INVALID, "vfk_session_use_obstacles: a mixed scene needs a session created with n_obstacles > 0");
+    if (mode == VFK_OBST_MIXED && s->shared_m > 0 && (s->has_ext != 0) != s->shared_ext)
+        return fail(h, VFK_ERR_INVALID, "vfk_session_use_obstacles: the per-instance and shared lists' ext rows go together");
+    s->obst_mode = mode;
+    s->generation++;
+    return VFK_OK;
+}
+
+// The scene the session's calls use: the shared list (un-offset by any tile range), the per-instance arrays or both; returns
+// the n_obstacles argument of the call (the shared count in mode 1, the per-instance one otherwise).
 static int session_scene(const vfk_session_s* s, vfk_buffers* b) {
-    if (!s->shared_on) return s->n_obst;
-    b->obst = s->shared_dev;
-    b->obst_ext = s->shared_ext ? s->shared_dev + (size_t)VFK_MAX_SHARED_OBSTACLES * 4 * s->es : nullptr;
-    b->obst_shared = 1;
-    return s->shared_m;
+    if (s->obst_mode == VFK_OBST_PER_INSTANCE) return s->n_obst;
+    const void* ext = s->shared_ext ? s->shared_dev + (size_t)VFK_MAX_SHARED_OBSTACLES * 4 * s->es : nullptr;
+    b->obst_shared = s->obst_mode;
+    if (s->obst_mode == VFK_OBST_SHARED) {
+        b->obst = s->shared_dev;
+        b->obst_ext = ext;
+        return s->shared_m;
+    }
+    b->shared_obst = s->shared_dev;
+    b->shared_obst_ext = ext;
+    b->n_shared_obst = s->shared_m;
+    return s->n_obst;
 }
 
 extern "C" int vfk_session_set_aux(vfk_session s, const void* aux, int n_aux) {
@@ -735,14 +824,15 @@ extern "C" int vfk_session_set_ns_input(vfk_session s, const void* x) {
     return upload_blocked(s, s->d_ns_in, x, s->h->params.ns_mode == VFK_NS_CONTROL ? 4 : s->N, 1);
 }
 
-// Offset every per-instance buffer of a blocked view to the tile range starting at tile0 (a shared scene stays whole).
+// Offset every per-instance buffer of a blocked view to the tile range starting at tile0 (a shared list stays whole; a mixed
+// scene's own list is offset like any per-instance buffer).
 static vfk_buffers offset_view(const vfk_buffers& b, int64_t tile0, int N, int M, size_t es) {
     vfk_buffers o = b;
     auto off = [&](const void* p, size_t comps) -> void* {
         return p ? (void*)((char*)const_cast<void*>(p) + (size_t)tile0 * comps * 32 * es) : nullptr;
     };
     o.q = off(b.q, N); o.goal = off(b.goal, 13);
-    if (!b.obst_shared) { o.obst = off(b.obst, (size_t)((M + 1) & ~1) * 4); o.obst_ext = off(b.obst_ext, (size_t)M * 2); }
+    if (b.obst_shared != VFK_OBST_SHARED) { o.obst = off(b.obst, (size_t)((M + 1) & ~1) * 4); o.obst_ext = off(b.obst_ext, (size_t)M * 2); }
     o.aux = off(b.aux, (size_t)b.n_aux * 12);
     o.jp_ref = off(b.jp_ref, N); o.jp_lo = off(b.jp_lo, N); o.jp_hi = off(b.jp_hi, N); o.ns_lastvec = off(b.ns_lastvec, (size_t)(ns_ctrl_vectors(N) > 0 ? ns_ctrl_vectors(N) : 1) * N); o.q_cmded = off(b.q_cmded, N);
     for (int e = 0; e < 3; ++e) o.ext_cmd[e] = off(b.ext_cmd[e], N);
@@ -981,7 +1071,7 @@ extern "C" int vfk_session_solve(vfk_session s, const void* q_in, int max_cycles
     if ((rc = vfk_session_buffers(s, &b)) != VFK_OK) return rc;
     b.qdot_vf = b.qdot_ns = b.qdot_jp = b.qdot = b.cmd = b.pose = b.twist = nullptr;
     b.flags = nullptr;
-    if ((rc = vfk_solve(h, &b, s->n, s->shared_on ? s->shared_m : s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
+    if ((rc = vfk_solve(h, &b, s->n, s->obst_mode == VFK_OBST_SHARED ? s->shared_m : s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
                         s->stream)) < 0)
         return rc;
     int launches = rc;
@@ -1045,12 +1135,15 @@ extern "C" int vfk_session_read(vfk_session s, const char* what, void* out) {
 
 extern "C" int vfk_session_buffers(vfk_session s, vfk_buffers* out) {
     if (!s || !out) return fail(s ? s->h : nullptr, VFK_ERR_INVALID, "vfk_session_buffers: null argument");
-    *out = s->b;
-    session_scene(s, out);
-    out->jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
-    out->jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
-    out->jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
-    out->ns_in = s->have_ns_in ? s->d_ns_in : nullptr;
+    vfk_buffers v = s->b;
+    session_scene(s, &v);
+    v.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
+    v.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
+    v.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
+    v.ns_in = s->have_ns_in ? s->d_ns_in : nullptr;
+    // the mixed-scene fields at the struct's end are written only in that mode: a caller built against the struct without
+    // them never selects it, and its shorter struct is not written past its end
+    memcpy(out, &v, s->obst_mode == VFK_OBST_MIXED ? sizeof v : offsetof(vfk_buffers, shared_obst));
     return VFK_OK;
 }
 

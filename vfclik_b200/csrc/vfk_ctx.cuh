@@ -70,8 +70,15 @@ int vfk_launch_f64_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst
 // The vfk_solve variants, one translation unit per precision.
 int vfk_solve_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
 int vfk_solve_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
-// The shared-scene variants (vfk_buffers.obst_shared), step and solve, one translation unit each per precision.
-int vfk_launch_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
-int vfk_launch_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
-int vfk_solve_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
-int vfk_solve_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+// The list a shared (obst_shared = 1) or mixed (2) scene gives the whole batch, resolved from vfk_buffers by the ABI layer.
+struct vfk_shared_scene {
+    const void* obst;          // dense [n][4]
+    const void* obst_ext;      // dense [n][2] or null
+    int n;
+};
+// The shared-scene variants (vfk_buffers.obst_shared), step and solve, one translation unit each per precision: n_obst
+// instance-own obstacles (mode 2; 0 in mode 1) plus the shared list `sh` (n > 0).
+int vfk_launch_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int k_cycles, cudaStream_t st, const vfk_io* io);
+int vfk_launch_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int k_cycles, cudaStream_t st, const vfk_io* io);
+int vfk_solve_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+int vfk_solve_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);

@@ -134,6 +134,14 @@ struct KArgs {
     T tol_q2;                  // sin^2(tol_rot / 2) against |xyz|^2 of the error quaternion; +inf when tol_rot >= pi
     int32_t* cycles;           // [1] first cycle c whose q_c met the rule, or -1
     T* dist;                   // [2] {|p_goal - p_tool|, rotation angle} at the returned q, or null
+    // SHARED kernels: the list shared by the whole batch (vfk_buffers.obst_shared = 1 or 2), staged into shared memory per
+    // CTA.  The obst / n_obst fields above then describe the instance's own list (mode 2), which runs through the ring as in
+    // the per-instance kernels, and are empty in a shared-only call.
+    const T* sh_obst;          // dense [sh_n][4] {x, y, z, radius}
+    const T* sh_obst_ext;      // dense [sh_n][2] {safe, order} or null
+    int32_t sh_n;
+    int32_t sh_np;             // sh_n rounded up to even
+    int32_t sh_chunks, sh_full, sh_rem;     // as n_chunks / n_full / n_rem
 };
 
 // ------------------------------------------------------------------------------ chain patterns
@@ -365,16 +373,17 @@ __device__ __forceinline__ Vec4<T> shared_obst(const Vec4<T>* pair, int s) {
 // is at most 48 KB read once per CTA from L2, and a bulk copy would want 16-byte multiples that an odd FP32 ext list is not.
 template <typename T, bool EXT>
 __device__ __forceinline__ void stage_shared_scene(const KArgs<T>& a, unsigned char* dst) {
-    const T* src = reinterpret_cast<const T*>(a.obst);
+    const T* src = a.sh_obst;
     T* o = reinterpret_cast<T*>(dst);
-    for (int i = (int)threadIdx.x; i < a.n_obst_p * 4; i += kBlock) {    // scalar i of the pair form: pair i / 8, slot i % 2,
+    for (int i = (int)threadIdx.x; i < a.sh_np * 4; i += kBlock) {       // scalar i of the pair form: pair i / 8, slot i % 2,
         const int m = (i >> 3) * 2 + (i & 1);                              // component (i / 2) % 4
-        o[i] = m < a.n_obst ? __ldg(src + m * 4 + ((i >> 1) & 3)) : T(0);
+        o[i] = m < a.sh_n ? __ldg(src + m * 4 + ((i >> 1) & 3)) : T(0);
     }
     if constexpr (EXT) {
-        const T* se = reinterpret_cast<const T*>(a.obst_ext);
-        T* oe = reinterpret_cast<T*>(dst + (size_t)a.n_obst_p * sizeof(Vec4<T>));
-        for (int i = (int)threadIdx.x; i < a.n_obst * 2; i += kBlock) oe[i] = __ldg(se + i);
+        // with EXT both lists carry ext rows (the host checks it); a shared-only call without the own list passes its own
+        const T* se = a.sh_obst_ext;
+        T* oe = reinterpret_cast<T*>(dst + (size_t)a.sh_np * sizeof(Vec4<T>));
+        for (int i = (int)threadIdx.x; i < a.sh_n * 2; i += kBlock) oe[i] = __ldg(se + i);
     }
 }
 
@@ -615,10 +624,13 @@ __device__ __forceinline__ void issue_qg(const KArgs<T>& a, int64_t tile, int bu
 // (ring_leave, vfk_ring.cuh) and moves on to its next unit.  The per-cycle outputs (qdot, flags, pose, ...) do not exist
 // in this mode; the state a cycle carries (q, jp_ref, ns_lastvec) freezes with the instance.
 // SHARED = one obstacle list for the whole batch (vfk_buffers.obst_shared; G = 1 only): the CTA stages it into shared memory
-// once (stage_shared_scene) before its one CTA-wide barrier, and the repulsor loop reads it there.  The obstacle ring, its
-// mbarrier waits and refills and the L2 prefetch do not exist in this mode (n_stages = 0); an instance costs q and goal only.
-// The per-obstacle arithmetic is the per-instance path's (the same repel2 / one() calls, chunk split and order
-// specialisations), so the field is bit-identical to it on a replicated scene.
+// once (stage_shared_scene) before its one CTA-wide barrier, and the repulsor loop reads it there after the instance's own
+// obstacles.  The own list (mixed scene, obst_shared = 2) runs through the obstacle ring exactly as in the per-instance
+// kernels -- its stage plan, waits and refills, L2 prefetch and the solve's ring exit; with no own list (a shared-only call)
+// the ring is empty (n_chunks = n_stages = 0) and all of that does nothing, so an instance costs q and goal only.  The
+// per-obstacle arithmetic is the per-instance path's (the same repel2 / one() calls, chunk split and order
+// specialisations), so the field is bit-identical to it on the list [own ; shared] when the own count is a multiple of
+// kChunk (the shared chunks then start where they would in the concatenated list).
 template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool SOLVE = false, bool SHARED = false>
 __global__ void __launch_bounds__(kBlock, MINB)
 vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a) {
@@ -633,7 +645,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     unsigned char* region = smem + kSmemHeader + kTabBytes<T> + (size_t)warp * WS::warp_bytes(a.n_stages);
     [[maybe_unused]] const double2* sctab = reinterpret_cast<const double2*>(smem + kSmemHeader);
     [[maybe_unused]] unsigned char* scene = smem + kSmemHeader + kTabBytes<T>;      // SHARED: the staged list, before the warps' regions
-    if constexpr (SHARED) region += shared_scene_bytes<T, EXT>(a.n_obst_p, a.n_obst);
+    if constexpr (SHARED) region += shared_scene_bytes<T, EXT>(a.sh_np, a.sh_n);
     const uint32_t bars_a = smem_u32(bars), region_a = smem_u32(region);       // shared-window addresses, once per warp
     static_assert(G == 1 || G == kChunk, "a cooperative group takes one obstacle of a chunk per lane");
     constexpr int kSub = G == 1 ? 1 : G;                        // work units per tile (G == 8: 8 units of 4 instances)
@@ -707,7 +719,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         // tile's kinematic chain (~1.5 us) a third of what it gains here.  Blocks over 32 KB (M = 256) are left to the ring,
         // which is at the copy peak there; a launch of fewer than four tiles per warp is dominated by its start, where every
         // warp's demand copies are queued at once, and skips the prefetch on its first tile (FP64 config 2: -3 % otherwise).
-        if constexpr (G == 1 && !SHARED) {
+        if constexpr (G == 1) {
             const int first = S * kChunk;
             const uint32_t bytes = a.n_obst_p > first ? (uint32_t)(a.n_obst_p - first) * 32u * (uint32_t)sizeof(Vec4<T>) : 0u;
             if (!resident && bytes != 0 && bytes <= 32768u && (it > 0 || n_units >= 4 * stride) && lane == 0)
@@ -788,18 +800,16 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                 if (__all_sync(0xffffffffu, done)) {
                     // the whole unit has stopped: wait what the ring still has in flight for it, refill those slots with the
                     // next unit's chunks, and move on.  A resident ring requests the next unit's chunks in the last cycle,
-                    // so a cycle that leaves early does that instead.  A shared scene has no ring: the warp just leaves.
-                    if constexpr (!SHARED) {
-                        const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
-                                                  : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
-                        for (int i = 0; i < left; ++i) {
-                            const int stage = resident ? i : c_stage;
-                            mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
-                            __syncwarp();
-                            if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                            ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
-                            if (!resident) ring_consumed(c_stage, c_phase, S);
-                        }
+                    // so a cycle that leaves early does that instead.  An empty ring (a shared-only scene) has nothing left.
+                    const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
+                                              : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
+                    for (int i = 0; i < left; ++i) {
+                        const int stage = resident ? i : c_stage;
+                        mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
+                        __syncwarp();
+                        if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
+                        ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
+                        if (!resident) ring_consumed(c_stage, c_phase, S);
                     }
                     break;
                 }
@@ -807,22 +817,20 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             [[maybe_unused]] NegPos2 np2;                               // FP32 packed repulsor: duplicated tool position, paired sums
             [[maybe_unused]] float2 acc2[3] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) np2.set(pt);
-            // SHARED: a chunk is kChunk consecutive obstacles of the staged list, one lane's worth of each pair and ext row
-            constexpr int kPairStride = SHARED ? 2 : 64, kPlaneStride = SHARED ? 1 : 32;     // in 16-byte vectors
+            // the instance's own chunks, through the ring
             for (int ch = 0; ch < a.n_chunks; ++ch) {
                 const int stage = resident ? ch : c_stage;
-                if constexpr (!SHARED) mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
-                const unsigned char* sb = SHARED ? scene + (size_t)ch * (kChunk * sizeof(Vec4<T>)) : region + (size_t)stage * WS::kStage;
+                mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
+                const unsigned char* sb = region + (size_t)stage * WS::kStage;
                 const Vec4<T>* sp = reinterpret_cast<const Vec4<T>*>(sb);                      // pair p starts at sp + p * 64
-                const Vec2<T>* se = SHARED ? reinterpret_cast<const Vec2<T>*>(scene + (size_t)a.n_obst_p * sizeof(Vec4<T>)) + ch * kChunk
-                                           : reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot;
+                const Vec2<T>* se = reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot;
                 const int n_here = ch < a.n_full ? kChunk : a.n_rem;                           // obstacles in this chunk
                 // one obstacle by its index in the chunk: scalar form (FP64, per-obstacle {safe, order}, cooperative shape)
                 auto one = [&](int m, auto order_c) {
                     constexpr int ORD = decltype(order_c)::value;
-                    const Vec4<T> o = SHARED ? shared_obst<T>(sp + (m >> 1) * 2, m & 1) : ObstPairs<T>::load(sp + (m >> 1) * 64, slot, m & 1);
+                    const Vec4<T> o = ObstPairs<T>::load(sp + (m >> 1) * 64, slot, m & 1);
                     T safe_inv = c.obst_safe_inv, order = c.obst_order;
-                    if (EXT) { const Vec2<T> e = se[m * kPlaneStride]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
+                    if (EXT) { const Vec2<T> e = se[m * 32]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
                     repel<T, ORD>(o, safe_inv, order, pt, acc);
                 };
                 if constexpr (G > 1) {
@@ -830,13 +838,12 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     if (ol < n_here) one(ol, std::integral_constant<int, 0>{});
                 } else if constexpr (sizeof(T) == 4 && !EXT) {
                     // FP32: two obstacles per step on the packed FP32 pipe; a zero-radius padding slot contributes exactly 0
-                    const float4* pl = reinterpret_cast<const float4*>(sb) + (SHARED ? 0 : slot);
+                    const float4* pl = reinterpret_cast<const float4*>(sb) + slot;
                     if (ch < a.n_full) {
                         auto full_chunk = [&](auto order_c) {
 #pragma unroll
                             for (int p = 0; p < kChunk / 2; ++p)
-                                repel2<decltype(order_c)::value>(pl[p * kPairStride], pl[p * kPairStride + kPlaneStride], c.obst_safe_inv,
-                                                                 c.obst_order, np2, acc2);
+                                repel2<decltype(order_c)::value>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
                         };
                         // decay order 20 (the reference's typical value, old/README.old:75) by five multiplications instead of
                         // MUFU lg2 / ex2: two more instructions per obstacle but two fewer on the quarter-rate XU pipe, which also
@@ -846,7 +853,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                         else full_chunk(std::integral_constant<int, 0>{});
                     } else {
                         for (int p = 0; p < (a.n_rem + 1) >> 1; ++p)
-                            repel2<0>(pl[p * kPairStride], pl[p * kPairStride + kPlaneStride], c.obst_safe_inv, c.obst_order, np2, acc2);
+                            repel2<0>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
                     }
                 } else if (ch < a.n_full) {
                     // FP64 with a uniform small-integer decay order: fixed multiplication chain instead of pow()
@@ -862,14 +869,54 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     for (int m = 0; m < a.n_rem; ++m) one(m, std::integral_constant<int, 0>{});
                 }
                 // this slot is free again: request the chunk that will occupy it S uses from now
-                if constexpr (!SHARED) {
-                    if (!resident || last) {
-                        __syncwarp();
-                        if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                        if (++p_chunk == a.n_chunks) p_chunk = 0;
-                        if (++p_u == U) { p_u = 0; p_unit += stride; }
+                if (!resident || last) {
+                    __syncwarp();
+                    if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
+                    if (++p_chunk == a.n_chunks) p_chunk = 0;
+                    if (++p_u == U) { p_u = 0; p_unit += stride; }
+                }
+                if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
+            }
+            // SHARED: then the shared list's chunks from the staged scene -- kChunk consecutive obstacles, one lane's worth of each
+            // pair and ext row -- through the same per-obstacle calls as the ring loop above (own obstacles first)
+            if constexpr (SHARED) {
+                const Vec2<T>* se_all = reinterpret_cast<const Vec2<T>*>(scene + (size_t)a.sh_np * sizeof(Vec4<T>));
+                for (int ch = 0; ch < a.sh_chunks; ++ch) {
+                    const Vec4<T>* sp = reinterpret_cast<const Vec4<T>*>(scene) + (size_t)ch * kChunk;       // pair p at sp + 2 p
+                    const Vec2<T>* se = se_all + ch * kChunk;
+                    auto one = [&](int m, auto order_c) {
+                        constexpr int ORD = decltype(order_c)::value;
+                        const Vec4<T> o = shared_obst<T>(sp + (m >> 1) * 2, m & 1);
+                        T safe_inv = c.obst_safe_inv, order = c.obst_order;
+                        if (EXT) { const Vec2<T> e = se[m]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
+                        repel<T, ORD>(o, safe_inv, order, pt, acc);
+                    };
+                    if constexpr (sizeof(T) == 4 && !EXT) {
+                        const float4* pl = reinterpret_cast<const float4*>(sp);
+                        if (ch < a.sh_full) {
+                            auto full_chunk = [&](auto order_c) {
+#pragma unroll
+                                for (int p = 0; p < kChunk / 2; ++p)
+                                    repel2<decltype(order_c)::value>(pl[p * 2], pl[p * 2 + 1], c.obst_safe_inv, c.obst_order, np2, acc2);
+                            };
+                            if (c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
+                            else full_chunk(std::integral_constant<int, 0>{});
+                        } else {
+                            for (int p = 0; p < (a.sh_rem + 1) >> 1; ++p)
+                                repel2<0>(pl[p * 2], pl[p * 2 + 1], c.obst_safe_inv, c.obst_order, np2, acc2);
+                        }
+                    } else if (ch < a.sh_full) {
+                        auto full_chunk = [&](auto order_c) {
+#pragma unroll
+                            for (int m = 0; m < kChunk; ++m) one(m, order_c);
+                        };
+                        if (sizeof(T) == 8 && !EXT && c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
+                        else if (sizeof(T) == 8 && !EXT && c.order_int == 5) full_chunk(std::integral_constant<int, 5>{});
+                        else if (sizeof(T) == 8 && !EXT && c.order_int == 2) full_chunk(std::integral_constant<int, 2>{});
+                        else full_chunk(std::integral_constant<int, 0>{});
+                    } else {
+                        for (int m = 0; m < a.sh_rem; ++m) one(m, std::integral_constant<int, 0>{});
                     }
-                    if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
                 }
             }
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) {
@@ -1258,12 +1305,15 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
 }
 
 // ------------------------------------------------------------------------------ small kernels
-// Field query at given tool poses (scripts/vf:469-503); low-rate visualisation path, plain loads.
+// Field query at given tool poses (scripts/vf:469-503); low-rate visualisation path, plain loads.  The instance's own
+// obstacles (blocked, n_obst) first, then a list shared by the whole batch (dense [n_sh][4], ext [n_sh][2] or null), one
+// obstacle at a time, as if the instance's list were [own ; shared].
 template <typename T>
 __global__ void __launch_bounds__(kSmallBlock)
 vfk_field_kernel(const __grid_constant__ KConst<T> c, const T* __restrict__ pose, const T* __restrict__ goal,
                  const Vec4<T>* __restrict__ obst, const Vec2<T>* __restrict__ obst_ext, const T* __restrict__ aux, int n_aux,
-                 T* __restrict__ twist, int64_t n, int n_obst) {
+                 T* __restrict__ twist, int64_t n, int n_obst, const T* __restrict__ sh_obst, const T* __restrict__ sh_ext,
+                 int n_sh) {
     const int64_t i = (int64_t)blockIdx.x * kSmallBlock + threadIdx.x;
     if (i >= n) return;
     const int64_t tile = i >> 5;
@@ -1283,6 +1333,13 @@ vfk_field_kernel(const __grid_constant__ KConst<T> c, const T* __restrict__ pose
         const Vec4<T> o = ObstPairs<T>::load(obst + (tile * n_obst_p + (m & ~1)) * 32, lane, m & 1);
         T safe_inv = c.obst_safe_inv, order = c.obst_order;
         if (obst_ext) { const Vec2<T> e = obst_ext[(tile * n_obst + m) * 32 + lane]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
+        repel<T>(o, safe_inv, order, pt, acc);
+    }
+    for (int m = 0; m < n_sh; ++m) {
+        Vec4<T> o;
+        o.x = sh_obst[m * 4]; o.y = sh_obst[m * 4 + 1]; o.z = sh_obst[m * 4 + 2]; o.w = sh_obst[m * 4 + 3];
+        T safe_inv = c.obst_safe_inv, order = c.obst_order;
+        if (sh_ext) { safe_inv = Prec<T>::rcp(sh_ext[m * 2]); order = sh_ext[m * 2 + 1]; }
         repel<T>(o, safe_inv, order, pt, acc);
     }
     V[0] = fma(c.obst_force, acc[0], V[0]); V[1] = fma(c.obst_force, acc[1], V[1]); V[2] = fma(c.obst_force, acc[2], V[2]);

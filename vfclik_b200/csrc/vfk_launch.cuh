@@ -14,13 +14,16 @@ using namespace vfk;
 // obstacles x 32 instances) and two q/goal buffers.  Two stages measured best on B200 for both K = 1
 // (106 us vs 110 us with three at the headline shape) and K = 100 (streaming the ring from L2 every cycle at
 // full occupancy beats keeping four chunks resident at 2 CTAs/SM): gpurun_out t03, DESIGN.md section 4.1.
+// Long FP32 chains run 2 CTAs per SM on registers, so a third stage is free: config 5 0.684 -> 0.708 of the HBM roofline
+// (4: 0.697; 6 and 8 cost a resident CTA: 0.44); everywhere else a third stage costs occupancy (config 4: 1.009 -> 0.988).
+template <typename T, int N>
+constexpr int kRingStages = (sizeof(T) == 4 && N >= 10) ? 3 : 2;
+
 template <typename T, int N, bool EXT>
 static void plan_stages(int n_obst, int* n_chunks, int* n_stages, size_t* smem_bytes) {
     using WS = WarpStage<T, N, EXT>;
     *n_chunks = (n_obst + kChunk - 1) / kChunk;
-    // long FP32 chains run 2 CTAs per SM on registers, so a third stage is free: config 5 0.684 -> 0.708 of the HBM roofline
-    // (4: 0.697; 6 and 8 cost a resident CTA: 0.44); everywhere else a third stage costs occupancy (config 4: 1.009 -> 0.988)
-    int stages = (sizeof(T) == 4 && N >= 10) ? 3 : 2;
+    int stages = kRingStages<T, N>;
     if (*n_chunks > 0 && *n_chunks < stages) stages = *n_chunks;
     if (*n_chunks == 0) stages = 0;
     *n_stages = stages;
@@ -68,16 +71,18 @@ static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
 // spills).  Measured on B200, 1 M instances: 109.5 us vs 111.2 us per launch at K = 1 (more warps hide more HBM latency),
 // but 1.6 % slower at K = 100, where the kernel is issue-bound and the tighter register budget costs instructions.
 // SOLVE: the vfk_solve variant (vfk_kernels.cuh), with its stop rule and result buffers in `sv`.
-// SHARED: one obstacle list for the whole batch (vfk_buffers.obst_shared), staged into shared memory per CTA instead of a ring.
+// SHARED: one obstacle list for the whole batch (vfk_buffers.obst_shared), `sh`, staged into shared memory per CTA; the
+// n_obst obstacles of the instance's own list (a mixed scene; 0 in a shared-only call) run through the ring as usual.
 template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false, bool SOLVE = false, bool SHARED = false>
 static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
+                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
     KArgs<T> a;
     memset(&a, 0, sizeof a);
     a.q = static_cast<T*>(b->q);
     a.goal = static_cast<const T*>(b->goal);
-    a.obst = static_cast<const Vec4<T>*>(b->obst);
-    a.obst_ext = static_cast<const Vec2<T>*>(b->obst_ext);
+    // (in a shared-only call b->obst is the shared list, and there is no own list)
+    a.obst = (!SHARED || n_obst > 0) ? static_cast<const Vec4<T>*>(b->obst) : nullptr;
+    a.obst_ext = (!SHARED || n_obst > 0) ? static_cast<const Vec2<T>*>(b->obst_ext) : nullptr;
     a.aux = b->n_aux > 0 ? static_cast<const T*>(b->aux) : nullptr;
     a.n_aux = a.aux ? b->n_aux : 0;
     a.jp_ref = static_cast<T*>(b->jp_ref);
@@ -106,26 +111,31 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
         // thresholds in T: |dp|^2 against tol_trans^2, and |xyz|^2 = sin^2(angle / 2) of the error quaternion against
         // sin^2(tol_rot / 2) -- exact and monotone on [0, pi], no transcendental in the kernel
         a.tol_d2 = (T)(sv->tol_trans * sv->tol_trans);
-        const double sh = std::sin(0.5 * sv->tol_rot);
-        a.tol_q2 = sv->tol_rot >= 3.14159265358979323846 ? (T)INFINITY : (T)(sh * sh);
+        const double sh_rot = std::sin(0.5 * sv->tol_rot);
+        a.tol_q2 = sv->tol_rot >= 3.14159265358979323846 ? (T)INFINITY : (T)(sh_rot * sh_rot);
         a.cycles = sv->cycles;
         a.dist = static_cast<T*>(sv->dist);
     }
     size_t smem = 0;
-    if constexpr (SHARED) {
-        // The list takes at most half the bytes of the two-stage ring it replaces, so a shared kernel never has fewer resident
-        // CTAs per SM for shared memory than its per-instance twin (the same MINB gives it the same register budget).
-        static_assert(shared_scene_bytes<T, EXT>(VFK_MAX_SHARED_OBSTACLES, VFK_MAX_SHARED_OBSTACLES) * 2 <=
-                      (kBlock / 32) * 2 * WarpStage<T, N, EXT>::kStage, "shared-scene cap exceeds the ring's budget");
-        a.n_chunks = (n_obst + kChunk - 1) / kChunk;
-        a.n_stages = 0;
-        smem = kSmemHeader + kTabBytes<T> + shared_scene_bytes<T, EXT>(a.n_obst_p, n_obst) +
-               (size_t)(kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(0);
-    } else {
-        plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
-    }
+    plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
     a.n_full = n_obst / kChunk;
     a.n_rem = n_obst % kChunk;
+    if constexpr (SHARED) {
+        // Shared memory: the own ring (its usual plan on the own count; no stages without one), the staged shared list and
+        // the q / goal buffers.  Every instantiation fits an SM with an own list at the largest stage count and a shared
+        // list at the cap: FP64 + EXT with 17 joints takes 204.5 KiB there (one CTA per SM, as its MINB asks).
+        static_assert(kSmemHeader + kTabBytes<T> + shared_scene_bytes<T, EXT>(VFK_MAX_SHARED_OBSTACLES, VFK_MAX_SHARED_OBSTACLES) +
+                          (kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(kRingStages<T, N>) <= (227u << 10),
+                      "a mixed scene at the shared-list cap does not fit an SM");
+        a.sh_obst = static_cast<const T*>(sh->obst);
+        a.sh_obst_ext = static_cast<const T*>(sh->obst_ext);
+        a.sh_n = sh->n;
+        a.sh_np = (sh->n + 1) & ~1;
+        a.sh_chunks = (sh->n + kChunk - 1) / kChunk;
+        a.sh_full = sh->n / kChunk;
+        a.sh_rem = sh->n % kChunk;
+        smem += shared_scene_bytes<T, EXT>(a.sh_np, a.sh_n);
+    }
     // resident CTAs per SM that the register allocation aims for.  The shared-scene FP32 lean solve kernels of N <= 7 ask for
     // four: at three the LWR one took 130 registers where its per-instance twin takes 128, one resident CTA fewer (at four it
     // takes 127 without spilling; the 7-joint generic one spills 24 bytes, as its HIOCC step twin does)
@@ -242,10 +252,12 @@ static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
 // SHARED (a shared scene, M > 0): the same choices among the one-thread-per-instance kernels -- EXT, lean / general, HIOCC --
 // but neither the cooperative shape (FP64, n <= 4096) nor the lane-split shape (FP64, 17 joints) has a shared variant:
 // those calls run the one-thread kernel, whose field they match bit for bit (DESIGN.md section 4.5).
+// A mixed scene (own list and shared list) takes the same SHARED kernels; with ext rows both lists carry them.
 template <typename T, int N, class PAT, bool SOLVE = false, bool SHARED = false>
 static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
-    const bool ext = b->obst_ext && n_obst > 0;
+                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
+    bool ext = b->obst_ext && n_obst > 0;
+    if constexpr (SHARED) ext = ext || (sh->obst_ext && sh->n > 0);
     // Small FP64 batches cannot fill the GPU with one thread per instance: switch to the cooperative latency shape.
     // Measured (scripts/latency.py, one robot, 1000 fused cycles): FP64 M = 32: 6.4 vs 7.1 us per cycle, M = 256: 23.6 vs
     // 36.3 us.  In FP32 the repeller is three MUFU instructions and the shape only adds ring overhead (3.7 vs 2.7 us),
@@ -255,29 +267,29 @@ static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, i
         if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv)
                              : launch_cycle<T, N, PAT, false, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
     }
-    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
     // Two lanes per instance (vfk_split.cuh) for the FP64 17-joint kernel.
     if constexpr (kSplit<T, N> && !SOLVE && !SHARED) {
         if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N>(h, c, b, n, n_obst, k_cycles, st);
     }
     if ((SOLVE ? lean_inputs<T>(c, b) : is_lean<T>(c, b)) && h->chain.n_joints == N) {
         if constexpr (sizeof(T) == 4 && N <= 7 && !SOLVE) {
-            if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true, false, SHARED>(h, c, b, n, n_obst, k_cycles, st, io);
+            if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true, false, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, nullptr, sh);
         }
-        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
     }
-    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
 }
 
 template <typename T, int N, bool SOLVE = false, bool SHARED = false>
 static int dispatch_ext(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr) {
+                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
     if constexpr (N == 7) {
-        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
     }
     if constexpr (N >= 10) {
-        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
     }
-    return dispatch_feat<T, N, GenericPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+    return dispatch_feat<T, N, GenericPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
 }
 

@@ -19,7 +19,8 @@ from typing import Dict, Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import (BuffersC, ParamsC, VfkError, NS_CONTROL, NS_OFF, NS_PROJECTOR)  # noqa: F401
+from ._lib import (BuffersC, ParamsC, VfkError, NS_CONTROL, NS_OFF, NS_PROJECTOR,  # noqa: F401
+                   VFK_OBST_PER_INSTANCE, VFK_OBST_SHARED, VFK_OBST_MIXED)
 
 
 BRIDGE_LWR, BRIDGE_POWERCUBE, BRIDGE_ICUB = 0, 1, 2
@@ -196,7 +197,7 @@ class Engine:
         return C.c_void_p(stream)
 
     @staticmethod
-    def _buffers(bufs, ext_cmd, obst_shared) -> BuffersC:
+    def _buffers(bufs, ext_cmd, obst_shared, n_shared_obstacles=None) -> BuffersC:
         b = BuffersC()
         for f in _BUF_FIELDS:
             setattr(b, f, _dev_ptr(bufs.get(f)))
@@ -205,14 +206,25 @@ class Engine:
         aux = bufs.get("aux")
         b.n_aux = 0 if aux is None else int(aux.shape[1]) // 12
         b.obst_shared = int(bufs.get("obst_shared", False) if obst_shared is None else obst_shared)
+        if b.obst_shared == VFK_OBST_MIXED:
+            sh = bufs.get("shared_obst")
+            b.shared_obst = _dev_ptr(sh)
+            b.shared_obst_ext = _dev_ptr(bufs.get("shared_obst_ext"))
+            if n_shared_obstacles is None:
+                n_shared_obstacles = bufs.get("n_shared_obst", 0 if sh is None else int(sh.shape[0]))
+            b.n_shared_obst = int(n_shared_obstacles)
         return b
 
     def step(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, k_cycles: int = 1,
-             stream: Optional[int] = None, ext_cmd=(None, None, None), obst_shared: Optional[bool] = None) -> int:
+             stream: Optional[int] = None, ext_cmd=(None, None, None), obst_shared: Optional[int] = None,
+             n_shared_obstacles: Optional[int] = None) -> int:
         """K fused cycles on blocked device buffers; returns the number of kernels launched.  ``obst_shared`` (default:
-        ``bufs["obst_shared"]``, else False) says that ``obst`` / ``obst_ext`` are one dense ``[M, 4]`` / ``[M, 2]`` list for
-        the whole batch (``vfk_buffers.obst_shared``, include/vfk.h)."""
-        b = self._buffers(bufs, ext_cmd, obst_shared)
+        ``bufs["obst_shared"]``, else 0; ``vfk_buffers.obst_shared``, include/vfk.h): 0 (``VFK_OBST_PER_INSTANCE``) per-instance
+        lists; 1 (``VFK_OBST_SHARED``, or True) ``obst`` / ``obst_ext`` are one dense ``[M, 4]`` / ``[M, 2]`` list for the whole
+        batch; 2 (``VFK_OBST_MIXED``) ``obst`` / ``obst_ext`` are per instance (``n_obstacles`` of them) and
+        ``bufs["shared_obst"]`` / ``bufs["shared_obst_ext"]`` one dense list for the whole batch, summed after the own ones.
+        Its length is ``n_shared_obstacles``, else ``bufs["n_shared_obst"]``, else the array's."""
+        b = self._buffers(bufs, ext_cmd, obst_shared, n_shared_obstacles)
         rc = self._check(self._lib.vfk_step(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(k_cycles),
                                             self._stream(stream)))
         self.launches += rc
@@ -220,13 +232,13 @@ class Engine:
 
     def solve(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, max_cycles: int, tol_trans: float,
               tol_rot: float, cycles_out, dist_out=None, stream: Optional[int] = None, ext_cmd=(None, None, None),
-              obst_shared: Optional[bool] = None) -> int:
+              obst_shared: Optional[int] = None, n_shared_obstacles: Optional[int] = None) -> int:
         """Run each instance's control loop until its tool frame is within ``tol_trans`` metres and ``tol_rot`` radians of
         its goal (strict), for at most ``max_cycles`` cycles (``vfk_solve``, include/vfk.h): the batched
         ``HandleArm.gotoFrame``.  ``cycles_out`` [1] int32 gets the cycle at which each instance stopped (-1: never),
         ``dist_out`` [2] the distance and angle to the goal at the returned q; q is updated in place.  ``bufs`` may hold
-        no per-cycle output; ``obst_shared`` as in ``step``.  Returns the number of kernels launched."""
-        b = self._buffers(bufs, ext_cmd, obst_shared)
+        no per-cycle output; ``obst_shared`` and the shared list as in ``step``.  Returns the number of kernels launched."""
+        b = self._buffers(bufs, ext_cmd, obst_shared, n_shared_obstacles)
         rc = self._check(self._lib.vfk_solve(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(max_cycles),
                                              float(tol_trans), float(tol_rot), _dev_ptr(cycles_out), _dev_ptr(dist_out),
                                              self._stream(stream)))
@@ -238,6 +250,16 @@ class Engine:
         rc = self._check(self._lib.vfk_field_eval(self._h, _dev_ptr(pose), _dev_ptr(goal), _dev_ptr(obst),
                                                   _dev_ptr(obst_ext), _dev_ptr(aux), int(n_aux), _dev_ptr(twist_out),
                                                   int(n_instances), int(n_obstacles), self._stream(stream)))
+        self.launches += rc
+        return rc
+
+    def field_eval_scene(self, pose, bufs: Dict[str, object], twist_out, n_instances: int, n_obstacles: int,
+                         obst_shared: Optional[int] = None, n_shared_obstacles: Optional[int] = None, stream=None) -> int:
+        """The field query (``vfk_field_eval_scene``) at tool poses ``pose`` [12] on the scene of ``bufs`` as ``step`` reads
+        it: ``goal``, ``obst`` / ``obst_ext``, ``aux`` and, by ``obst_shared``, the shared list.  ``twist_out`` [6]."""
+        b = self._buffers(bufs, (None, None, None), obst_shared, n_shared_obstacles)
+        rc = self._check(self._lib.vfk_field_eval_scene(self._h, _dev_ptr(pose), C.byref(b), int(n_instances), int(n_obstacles),
+                                                        _dev_ptr(twist_out), self._stream(stream)))
         self.launches += rc
         return rc
 
@@ -360,6 +382,13 @@ class Session:
         self.e._check(self.e._lib.vfk_session_set_shared_obstacles(self._s, _lib.np_ptr(a), None if x is None else _lib.np_ptr(x),
                                                                    int(a.shape[0])))
 
+    def use_obstacles(self, mode: int):
+        """Which lists later cycles and solves use (``vfk_session_use_obstacles``): ``VFK_OBST_PER_INSTANCE`` (0),
+        ``VFK_OBST_SHARED`` (1, needs ``set_shared_obstacles``) or ``VFK_OBST_MIXED`` (2: the per-instance scene and the
+        shared list together; needs a session created with obstacles and a shared list).  ``set_obstacles`` and
+        ``set_shared_obstacles`` select 0 and 1 themselves, so call this after both."""
+        self.e._check(self.e._lib.vfk_session_use_obstacles(self._s, int(mode)))
+
     def set_aux(self, aux):
         """Auxiliary field records ``[n_aux, 12, n]`` ({type, force, 10 params}; types 4 and 5), or None to clear."""
         if aux is None:
@@ -467,15 +496,21 @@ class DeviceBatch:
     ``[M, n, 4]``, ext ``[M, n, 2]``), moves them to the device and converts them with the
     library's pack kernel; ``download`` converts back.  ``bufs`` is what ``Engine.step`` takes.
     ``shared_obstacles=True``: one scene for the whole batch, ``obst`` dense ``[M, 4]`` and ``obst_ext`` ``[M, 2]`` on the
-    device as they are uploaded (``vfk_buffers.obst_shared``).
+    device as they are uploaded (``vfk_buffers.obst_shared``).  ``n_shared_obstacles=Ms`` (with ``shared_obstacles``
+    False): a mixed scene, the per-instance ``obst`` / ``obst_ext`` of ``n_obstacles`` each plus ``shared_obst`` ``[Ms, 4]``
+    and ``shared_obst_ext`` ``[Ms, 2]`` (when ``obst_ext``) for the whole batch, uploaded as they are.
     """
 
     _ROWS = {"goal": 13, "pose": 12, "flags": 1, "twist": 6, "track": 8, "dist": 2, "mon_f": 32, "solve_dist": 2}
 
     def __init__(self, engine: Engine, n_instances: int, n_obstacles: int, obst_ext: bool = False,
-                 outputs=("qdot",), inputs=(), shared_obstacles: bool = False):
+                 outputs=("qdot",), inputs=(), shared_obstacles: bool = False, n_shared_obstacles: Optional[int] = None):
         self.e, self.n, self.m = engine, int(n_instances), int(n_obstacles)
         self.shared = bool(shared_obstacles)
+        self.mixed = n_shared_obstacles is not None
+        self.ms = int(n_shared_obstacles or 0)
+        if self.shared and self.mixed:
+            raise ValueError("shared_obstacles and n_shared_obstacles exclude each other (a mixed scene has both lists)")
         self.t: Dict[str, object] = {}
         self.t["q"] = engine.alloc(engine.n_joints, self.n)
         self.t["goal"] = engine.alloc(13, self.n)
@@ -491,6 +526,15 @@ class DeviceBatch:
             self.t["obst"] = engine.alloc(self.m, self.n, width=4)
             if obst_ext:
                 self.t["obst_ext"] = engine.alloc(self.m, self.n, width=2)
+        if self.mixed:
+            import torch
+            if not 0 <= self.ms <= _lib.VFK_MAX_SHARED_OBSTACLES:
+                raise ValueError("a shared obstacle list holds 0..%d obstacles" % _lib.VFK_MAX_SHARED_OBSTACLES)
+            dev = "cuda:%d" % engine.device
+            # at least one row, so that the pointer is a real 128-byte aligned block even for an empty list
+            self.t["shared_obst"] = torch.zeros((max(self.ms, 1), 4), dtype=engine.torch_dtype, device=dev)
+            if obst_ext:
+                self.t["shared_obst_ext"] = torch.zeros((max(self.ms, 1), 2), dtype=engine.torch_dtype, device=dev)
         for name in tuple(outputs) + tuple(inputs):
             self._ensure(name)
         self.ext_cmd = [None, None, None]
@@ -508,7 +552,7 @@ class DeviceBatch:
         import torch
         if name in ("flags", "mon_i", "tracking_state", "cycles"):
             self.t[name] = self.e.alloc({"flags": 1, "mon_i": 6, "tracking_state": 2, "cycles": 1}[name], self.n, dtype=torch.int32)
-        elif name in ("obst", "obst_ext"):
+        elif name in ("obst", "obst_ext", "shared_obst", "shared_obst_ext"):
             raise KeyError("%s was not allocated (n_obstacles = 0 or obst_ext=False)" % name)
         else:
             self.t[name] = self.e.alloc(self._comps(name), self.n)
@@ -537,10 +581,12 @@ class DeviceBatch:
         return self.t["aux"]
 
     def upload(self, name: str, arr: np.ndarray):
-        if self.shared and name in ("obst", "obst_ext"):           # dense on both sides: a plain copy
+        if (self.shared and name in ("obst", "obst_ext")) or name in ("shared_obst", "shared_obst_ext"):   # dense: a plain copy
             import torch
             t = self._ensure(name)
             a = np.ascontiguousarray(arr, dtype=self.e.np_dtype)
+            if name.startswith("shared_") and a.shape[0] == 0:
+                return t
             if a.shape != tuple(t.shape):
                 raise ValueError("%s: expected %r, got %r" % (name, tuple(t.shape), a.shape))
             t.copy_(torch.from_numpy(a))
@@ -561,6 +607,8 @@ class DeviceBatch:
         t = self.t[name]
         if self.shared and name in ("obst", "obst_ext"):
             return t.cpu().numpy()
+        if name in ("shared_obst", "shared_obst_ext"):
+            return t[:self.ms].cpu().numpy()
         if t.dtype == torch.int32:                                   # int32 arrays: un-block on the host
             a = t.cpu().numpy()                                      # [tiles, comps, 32]
             return np.ascontiguousarray(a.transpose(1, 0, 2).reshape(a.shape[1], -1)[:, :self.n])
@@ -593,6 +641,12 @@ class DeviceBatch:
         b = {k: v for k, v in self.t.items() if k in _BUF_FIELDS}
         if self.shared:
             b["obst_shared"] = True
+        if self.mixed:
+            b["obst_shared"] = VFK_OBST_MIXED
+            b["shared_obst"] = self.t["shared_obst"]
+            if "shared_obst_ext" in self.t:
+                b["shared_obst_ext"] = self.t["shared_obst_ext"]
+            b["n_shared_obst"] = self.ms
         return b
 
     def monitor(self, stream=None) -> int:

@@ -89,6 +89,33 @@ def replicate_scene(obst: np.ndarray, n_instances: int) -> np.ndarray:
     return np.ascontiguousarray(np.broadcast_to(obst[:, None, :], (obst.shape[0], int(n_instances), obst.shape[1])))
 
 
+def mixed_scene_batch(chain: ChainDesc, n_instances: int, n_own: int, n_shared: int, seed: int, dtype=np.float64,
+                      obst_ext: bool = False, **kw):
+    """A shared workcell plus obstacles of each instance's own (``vfk_buffers.obst_shared = 2``): per-instance starts, goals
+    and ``n_own`` obstacles as :func:`random_batch` draws them with ``seed``, and ``n_shared`` obstacles for the whole batch,
+    the list :func:`random_batch` draws for a single instance with ``seed + 1`` (as :func:`shared_scene_batch`).
+
+    Returns dict(q [N,I], goal [13,I], obst [Mi,I,4], shared_obst [Ms,4] [, obst_ext [Mi,I,2], shared_obst_ext [Ms,2]])
+    of ``dtype``."""
+    w = random_batch(chain, n_instances, n_own, seed, dtype=dtype, obst_ext=obst_ext, **kw)
+    scene = random_batch(chain, 1, n_shared, seed + 1, dtype=dtype, obst_ext=obst_ext, **kw)
+    out = dict(w, shared_obst=np.ascontiguousarray(scene["obst"][:, 0]))
+    if obst_ext:
+        out["shared_obst_ext"] = np.ascontiguousarray(scene["obst_ext"][:, 0])
+    return out
+
+
+def concat_scene(own: np.ndarray, shared: np.ndarray, n_instances: int) -> np.ndarray:
+    """The per-instance array ``[Mi + Ms, n, C]`` equivalent to a mixed scene: each instance's own list ``[Mi, n, C]``
+    followed by the shared list ``[Ms, C]``, in the order the field sums them."""
+    own = np.asarray(own)
+    shared = np.asarray(shared)
+    n = int(n_instances)
+    if own.shape[1:] != (n, shared.shape[1]):
+        raise ValueError("own list %r does not match %d instances of %d components" % (own.shape, n, shared.shape[1]))
+    return np.ascontiguousarray(np.concatenate([own, replicate_scene(shared.astype(own.dtype, copy=False), n)], axis=0))
+
+
 def random_batch_device(engine, n_instances: int, n_obstacles: int, seed: int, slowdown: float = 0.05, box: float = 0.8):
     """Same distributions as :func:`random_batch`, drawn on the GPU with torch's generator (large shapes:
     config 4's 2M x 256 obstacles per GPU would take minutes and 8 GB of host memory through numpy).
