@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 
 #include "vfk_ctx.cuh"
@@ -261,9 +262,21 @@ extern "C" void vfk_destroy(vfk_handle h) { delete h; }
 extern "C" const char* vfk_last_error(vfk_handle h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 
 // -------------------------------------------------------------------------------- public: step
-static int check_layout(vfk_ctx* h, const void* ptr, const char* name, bool required) {
-    if (!ptr) return required ? fail(h, VFK_ERR_INVALID, "buffer %s is required", name) : VFK_OK;
-    if (reinterpret_cast<uintptr_t>(ptr) & 127) return fail(h, VFK_ERR_INVALID, "buffer %s must be 128-byte aligned", name);
+// Device buffers: present when required, 128-byte aligned when present; the first failure in table order is reported.
+struct BufferCheck {
+    const void* ptr;
+    const char* name;
+    bool required;
+};
+
+static int check_layout(vfk_ctx* h, std::initializer_list<BufferCheck> table) {
+    for (const BufferCheck& c : table) {
+        if (!c.ptr) {
+            if (c.required) return fail(h, VFK_ERR_INVALID, "buffer %s is required", c.name);
+        } else if (reinterpret_cast<uintptr_t>(c.ptr) & 127) {
+            return fail(h, VFK_ERR_INVALID, "buffer %s must be 128-byte aligned", c.name);
+        }
+    }
     return VFK_OK;
 }
 
@@ -281,11 +294,9 @@ static int check_scene(vfk_ctx* h, const vfk_buffers* b, int n_obst) {
     if (ms > VFK_MAX_SHARED_OBSTACLES)
         return fail(h, VFK_ERR_UNSUPPORTED, "a shared obstacle list holds at most %d obstacles (got %d)", VFK_MAX_SHARED_OBSTACLES, ms);
     if (b->reserved2 != 0) return fail(h, VFK_ERR_INVALID, "vfk_buffers.reserved2 must be 0");
-    int rc;
     // shared_obst is required even when it holds no obstacle: mode 2 without it is most likely a shared-only buffer set (a
     // dense obst) under the wrong mode, whose obst would otherwise be read as a per-instance array
-    if ((rc = check_layout(h, b->shared_obst, "shared_obst", true)) || (rc = check_layout(h, b->shared_obst_ext, "shared_obst_ext", false)))
-        return rc;
+    if (int rc = check_layout(h, {{b->shared_obst, "shared_obst", true}, {b->shared_obst_ext, "shared_obst_ext", false}})) return rc;
     if (n_obst > 0 && ms > 0 && (b->obst_ext == nullptr) != (b->shared_obst_ext == nullptr))
         return fail(h, VFK_ERR_INVALID, "obst_ext and shared_obst_ext go together in a mixed scene");
     return VFK_OK;
@@ -297,27 +308,40 @@ static int check_step(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, i
     if (n_obst < 0) return fail(h, VFK_ERR_INVALID, "n_obstacles must be >= 0");
     if (k_cycles < 1) return fail(h, VFK_ERR_INVALID, "k_cycles must be >= 1");
     if (b->n_aux < 0 || b->n_aux > 64) return fail(h, VFK_ERR_INVALID, "n_aux must be in 0..64");
-    int rc;
-    if ((rc = check_layout(h, b->q, "q", true)) || (rc = check_layout(h, b->goal, "goal", true)) ||
-        (rc = check_layout(h, b->obst, "obst", n_obst > 0)) || (rc = check_layout(h, b->obst_ext, "obst_ext", false)) || (rc = check_layout(h, b->aux, "aux", false)) ||
-        (rc = check_layout(h, b->jp_ref, "jp_ref", false)) || (rc = check_layout(h, b->jp_lo, "jp_lo", false)) || (rc = check_layout(h, b->jp_hi, "jp_hi", false)) || (rc = check_layout(h, b->ns_in, "ns_in", false)) ||
-        (rc = check_layout(h, b->ns_lastvec, "ns_lastvec", h->params.ns_mode == VFK_NS_CONTROL && ns_ctrl_vectors(h->chain.n_joints) > 0)) ||
-        (rc = check_layout(h, b->q_cmded, "q_cmded", false)) || (rc = check_layout(h, b->qdot_vf, "qdot_vf", false)) ||
-        (rc = check_layout(h, b->qdot_ns, "qdot_ns", false)) || (rc = check_layout(h, b->qdot_jp, "qdot_jp", false)) ||
-        (rc = check_layout(h, b->qdot, "qdot", false)) || (rc = check_layout(h, b->cmd, "cmd", false)) ||
-        (rc = check_layout(h, b->pose, "pose", false)) || (rc = check_layout(h, b->twist, "twist", false)) || (rc = check_layout(h, b->flags, "flags", false)))
+    const bool need_lastvec = h->params.ns_mode == VFK_NS_CONTROL && ns_ctrl_vectors(h->chain.n_joints) > 0;
+    if (int rc = check_layout(h, {{b->q, "q", true}, {b->goal, "goal", true}, {b->obst, "obst", n_obst > 0}, {b->obst_ext, "obst_ext", false},
+                                  {b->aux, "aux", false}, {b->jp_ref, "jp_ref", false}, {b->jp_lo, "jp_lo", false}, {b->jp_hi, "jp_hi", false},
+                                  {b->ns_in, "ns_in", false}, {b->ns_lastvec, "ns_lastvec", need_lastvec}, {b->q_cmded, "q_cmded", false},
+                                  {b->qdot_vf, "qdot_vf", false}, {b->qdot_ns, "qdot_ns", false}, {b->qdot_jp, "qdot_jp", false},
+                                  {b->qdot, "qdot", false}, {b->cmd, "cmd", false}, {b->pose, "pose", false}, {b->twist, "twist", false},
+                                  {b->flags, "flags", false}, {b->ext_cmd[0], "ext_cmd", false}, {b->ext_cmd[1], "ext_cmd", false},
+                                  {b->ext_cmd[2], "ext_cmd", false}}))
         return rc;
-    for (int e = 0; e < 3; ++e)
-        if ((rc = check_layout(h, b->ext_cmd[e], "ext_cmd", false))) return rc;
     if ((b->jp_lo == nullptr) != (b->jp_hi == nullptr)) return fail(h, VFK_ERR_INVALID, "jp_lo and jp_hi go together");
     return check_scene(h, b, n_obst);
 }
 
-// The batch-wide list of a shared or mixed scene (n = 0: none).  The mixed fields are read in VFK_OBST_MIXED only.
-static vfk_shared_scene shared_scene_of(const vfk_buffers* b, int n_obst) {
-    if (b->obst_shared == VFK_OBST_SHARED) return vfk_shared_scene{b->obst, b->obst_ext, n_obst};
-    if (b->obst_shared == VFK_OBST_MIXED) return vfk_shared_scene{b->shared_obst, b->shared_obst_ext, b->n_shared_obst};
-    return vfk_shared_scene{nullptr, nullptr, 0};
+// The scene of a call: in mode 0 (per instance) n_obst counts the instances' own lists, in mode 1 (shared) the batch-wide
+// list in obst / obst_ext, in mode 2 (mixed) the own lists, with the batch-wide list in the appended fields.  Nothing below
+// this point reads obst_shared.
+static vfk_scene resolve_scene(const vfk_buffers* b, int n_obst) {
+    const vfk_obst_list given{b->obst, b->obst_ext, n_obst};
+    if (b->obst_shared == VFK_OBST_SHARED) return vfk_scene{{nullptr, nullptr, 0}, given};
+    if (b->obst_shared == VFK_OBST_MIXED) return vfk_scene{given, {b->shared_obst, b->shared_obst_ext, b->n_shared_obst}};
+    return vfk_scene{given, {nullptr, nullptr, 0}};
+}
+
+// The launcher (translation unit) of a call: precision, solve or step, and whether the shared list holds obstacles (the SHARED
+// kernels; an empty one runs the per-instance kernels, so a mixed scene with no shared obstacle is exactly the per-instance
+// call); the step kernels are split further by joint count.
+static int launch_cycles(vfk_ctx* h, const CycleCall& call) {
+    VFK_CUDA(h, cudaSetDevice(h->device));
+    const bool f32 = h->precision == 32, shared = call.scene.shared.m > 0;
+    if (call.sv && shared) return f32 ? vfk_solve_shared_f32(h, call) : vfk_solve_shared_f64(h, call);
+    if (call.sv) return f32 ? vfk_solve_f32(h, call) : vfk_solve_f64(h, call);
+    if (shared) return f32 ? vfk_launch_shared_f32(h, call) : vfk_launch_shared_f64(h, call);
+    if (h->n_kernel <= 7) return f32 ? vfk_launch_f32_small(h, call) : vfk_launch_f64_small(h, call);
+    return f32 ? vfk_launch_f32_large(h, call) : vfk_launch_f64_large(h, call);
 }
 
 static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream, const vfk_io* io) {
@@ -325,20 +349,7 @@ static int step_impl(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, in
     int rc = check_step(h, b, n, n_obst, k_cycles);
     if (rc) return rc;
     if (n == 0) return 0;
-    VFK_CUDA(h, cudaSetDevice(h->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    // a shared or mixed scene with a non-empty shared list runs the SHARED kernels (own list: mode 2's per-instance one);
-    // mode 2 without shared obstacles is exactly the per-instance call
-    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
-    if (sh.n > 0) {
-        const int own = b->obst_shared == VFK_OBST_MIXED ? n_obst : 0;
-        return h->precision == 32 ? vfk_launch_shared_f32(h, b, n, own, &sh, k_cycles, st, io) : vfk_launch_shared_f64(h, b, n, own, &sh, k_cycles, st, io);
-    }
-    if (b->obst_shared == VFK_OBST_SHARED) n_obst = 0;
-    const bool small = h->n_kernel <= 7;
-    if (h->precision == 32)
-        return small ? vfk_launch_f32_small(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_f32_large(h, b, n, n_obst, k_cycles, st, io);
-    return small ? vfk_launch_f64_small(h, b, n, n_obst, k_cycles, st, io) : vfk_launch_f64_large(h, b, n, n_obst, k_cycles, st, io);
+    return launch_cycles(h, CycleCall{b, n, k_cycles, static_cast<cudaStream_t>(stream), io, nullptr, resolve_scene(b, n_obst)});
 }
 
 extern "C" int vfk_step(vfk_handle h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, void* stream) {
@@ -360,40 +371,28 @@ extern "C" int vfk_solve(vfk_handle h, const vfk_buffers* b, int64_t n, int n_ob
     for (const auto& o : per_cycle)
         if (o.p) return fail(h, VFK_ERR_INVALID, "vfk_solve: output %s must be NULL (a per-cycle output has no single meaning when instances stop at different cycles)", o.name);
     int rc = check_step(h, b, n, n_obst, max_cycles);
-    if (rc || (rc = check_layout(h, cycles_out, "cycles_out", true)) || (rc = check_layout(h, dist_out, "dist_out", false))) return rc;
+    if (rc || (rc = check_layout(h, {{cycles_out, "cycles_out", true}, {dist_out, "dist_out", false}}))) return rc;
     if (n == 0) return 0;
-    VFK_CUDA(h, cudaSetDevice(h->device));
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    vfk_solve_io sv;
-    sv.tol_trans = tol_trans;
-    sv.tol_rot = tol_rot;
-    sv.cycles = cycles_out;
-    sv.dist = dist_out;
-    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
-    if (sh.n > 0) {
-        const int own = b->obst_shared == VFK_OBST_MIXED ? n_obst : 0;
-        return h->precision == 32 ? vfk_solve_shared_f32(h, b, n, own, &sh, max_cycles, st, &sv) : vfk_solve_shared_f64(h, b, n, own, &sh, max_cycles, st, &sv);
-    }
-    if (b->obst_shared == VFK_OBST_SHARED) n_obst = 0;
-    return h->precision == 32 ? vfk_solve_f32(h, b, n, n_obst, max_cycles, st, &sv) : vfk_solve_f64(h, b, n, n_obst, max_cycles, st, &sv);
+    const vfk_solve_io sv{tol_trans, tol_rot, cycles_out, dist_out};
+    return launch_cycles(h, CycleCall{b, n, max_cycles, static_cast<cudaStream_t>(stream), nullptr, &sv, resolve_scene(b, n_obst)});
 }
 
-// The field query's launch: n_obst per-instance obstacles (blocked) and the shared list `sh` (dense).
-static int field_launch(vfk_ctx* h, const void* pose_in, const void* goal, const void* obst, const void* obst_ext, const void* aux,
-                        int n_aux, void* twist_out, int64_t n, int n_obst, const vfk_shared_scene& sh, void* stream) {
+// The field query's launch on a resolved scene: the own lists (blocked), then the shared list (dense).
+static int field_launch(vfk_ctx* h, const void* pose_in, const void* goal, const vfk_scene& sc, const void* aux, int n_aux,
+                        void* twist_out, int64_t n, void* stream) {
     VFK_CUDA(h, cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const unsigned grid = (unsigned)((n + kSmallBlock - 1) / kSmallBlock);
     if (h->precision == 32)
         vfk_field_kernel<float><<<grid, kSmallBlock, 0, st>>>(h->cf, (const float*)pose_in, (const float*)goal,
-                                                         (const Vec4<float>*)obst, (const Vec2<float>*)obst_ext,
-                                                         (const float*)aux, n_aux, (float*)twist_out, n, n_obst,
-                                                         (const float*)sh.obst, (const float*)sh.obst_ext, sh.n);
+                                                         (const Vec4<float>*)sc.own.obst, (const Vec2<float>*)sc.own.obst_ext,
+                                                         (const float*)aux, n_aux, (float*)twist_out, n, sc.own.m,
+                                                         (const float*)sc.shared.obst, (const float*)sc.shared.obst_ext, sc.shared.m);
     else
         vfk_field_kernel<double><<<grid, kSmallBlock, 0, st>>>(h->cd, (const double*)pose_in, (const double*)goal,
-                                                          (const Vec4<double>*)obst, (const Vec2<double>*)obst_ext,
-                                                          (const double*)aux, n_aux, (double*)twist_out, n, n_obst,
-                                                          (const double*)sh.obst, (const double*)sh.obst_ext, sh.n);
+                                                          (const Vec4<double>*)sc.own.obst, (const Vec2<double>*)sc.own.obst_ext,
+                                                          (const double*)aux, n_aux, (double*)twist_out, n, sc.own.m,
+                                                          (const double*)sc.shared.obst, (const double*)sc.shared.obst_ext, sc.shared.m);
     VFK_CUDA(h, cudaGetLastError());
     return 1;
 }
@@ -406,7 +405,7 @@ extern "C" int vfk_field_eval(vfk_handle h, const void* pose_in, const void* goa
     if (n_aux < 0 || n_aux > 64) return fail(h, VFK_ERR_INVALID, "n_aux must be in 0..64");
     if (n_aux == 0) aux = nullptr;
     if (n == 0) return 0;
-    return field_launch(h, pose_in, goal, obst, obst_ext, aux, n_aux, twist_out, n, n_obst, vfk_shared_scene{nullptr, nullptr, 0}, stream);
+    return field_launch(h, pose_in, goal, vfk_scene{{obst, obst_ext, n_obst}, {nullptr, nullptr, 0}}, aux, n_aux, twist_out, n, stream);
 }
 
 extern "C" int vfk_field_eval_scene(vfk_handle h, const void* pose_in, const vfk_buffers* b, int64_t n, int n_obst, void* twist_out,
@@ -416,13 +415,10 @@ extern "C" int vfk_field_eval_scene(vfk_handle h, const void* pose_in, const vfk
     if (n_obst < 0) return fail(h, VFK_ERR_INVALID, "n_obstacles must be >= 0");
     if (b->n_aux < 0 || b->n_aux > 64) return fail(h, VFK_ERR_INVALID, "n_aux must be in 0..64");
     int rc;
-    if ((rc = check_scene(h, b, n_obst))) return rc;
-    if ((rc = check_layout(h, b->obst, "obst", n_obst > 0)) || (rc = check_layout(h, b->obst_ext, "obst_ext", false))) return rc;
+    if ((rc = check_scene(h, b, n_obst)) || (rc = check_layout(h, {{b->obst, "obst", n_obst > 0}, {b->obst_ext, "obst_ext", false}})))
+        return rc;
     if (n == 0) return 0;
-    const vfk_shared_scene sh = shared_scene_of(b, n_obst);
-    const bool own = b->obst_shared != VFK_OBST_SHARED;
-    return field_launch(h, pose_in, b->goal, own ? b->obst : nullptr, own ? b->obst_ext : nullptr, b->n_aux > 0 ? b->aux : nullptr, b->n_aux,
-                        twist_out, n, own ? n_obst : 0, sh, stream);
+    return field_launch(h, pose_in, b->goal, resolve_scene(b, n_obst), b->n_aux > 0 ? b->aux : nullptr, b->n_aux, twist_out, n, stream);
 }
 
 extern "C" int vfk_mix(vfk_handle h, const void* const* cmds, const double* w, int n_ports, int n_channels, void* out,
@@ -746,20 +742,40 @@ extern "C" int vfk_session_use_obstacles(vfk_session s, int mode) {
     return VFK_OK;
 }
 
-// The scene the session's calls use: the shared list (un-offset by any tile range), the per-instance arrays or both; returns
-// the n_obstacles argument of the call (the shared count in mode 1, the per-instance one otherwise).
-static int session_scene(const vfk_session_s* s, vfk_buffers* b) {
+// What a session call's view holds besides q, goal, the scene and the inputs that are set: every output
+// (vfk_session_buffers), qdot and the enabled outputs (a cycle), or none (a solve).
+enum class SessionOutputs { all, enabled, none };
+
+// The blocked device view of a session call in `v`: the scene of the session's mode (the shared list whole, never offset by a
+// tile range), the per-instance inputs that are set and the outputs `outs` selects, a cycle's flags only when `want_flags`.
+// Returns the call's n_obstacles argument: the shared count in mode 1, the per-instance one otherwise.
+static int session_view(const vfk_session_s* s, SessionOutputs outs, bool want_flags, vfk_buffers* v) {
+    *v = s->b;
+    v->jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
+    v->jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
+    v->jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
+    v->ns_in = s->have_ns_in ? s->d_ns_in : nullptr;
+    const bool all = outs == SessionOutputs::all, none = outs == SessionOutputs::none;
+    auto keep = [&](bool enabled) { return all || (enabled && !none); };
+    if (!keep(true)) v->qdot = nullptr;
+    if (!keep(s->en_vf)) v->qdot_vf = nullptr;
+    if (!keep(s->en_ns)) v->qdot_ns = nullptr;
+    if (!keep(s->en_jp)) v->qdot_jp = nullptr;
+    if (!keep(s->en_cmd)) v->cmd = nullptr;
+    if (!keep(s->en_pose)) v->pose = nullptr;
+    if (!keep(s->en_twist)) v->twist = nullptr;
+    if (!keep(want_flags)) v->flags = nullptr;
     if (s->obst_mode == VFK_OBST_PER_INSTANCE) return s->n_obst;
     const void* ext = s->shared_ext ? s->shared_dev + (size_t)VFK_MAX_SHARED_OBSTACLES * 4 * s->es : nullptr;
-    b->obst_shared = s->obst_mode;
+    v->obst_shared = s->obst_mode;
     if (s->obst_mode == VFK_OBST_SHARED) {
-        b->obst = s->shared_dev;
-        b->obst_ext = ext;
+        v->obst = s->shared_dev;
+        v->obst_ext = ext;
         return s->shared_m;
     }
-    b->shared_obst = s->shared_dev;
-    b->shared_obst_ext = ext;
-    b->n_shared_obst = s->shared_m;
+    v->shared_obst = s->shared_dev;
+    v->shared_obst_ext = ext;
+    v->n_shared_obst = s->shared_m;
     return s->n_obst;
 }
 
@@ -825,8 +841,8 @@ extern "C" int vfk_session_set_ns_input(vfk_session s, const void* x) {
 }
 
 // Offset every per-instance buffer of a blocked view to the tile range starting at tile0 (a shared list stays whole; a mixed
-// scene's own list is offset like any per-instance buffer).
-static vfk_buffers offset_view(const vfk_buffers& b, int64_t tile0, int N, int M, size_t es) {
+// scene's own list is offset like any per-instance buffer).  ns_comps: components of ns_in (4 or N).
+static vfk_buffers offset_view(const vfk_buffers& b, int64_t tile0, int N, int M, int ns_comps, size_t es) {
     vfk_buffers o = b;
     auto off = [&](const void* p, size_t comps) -> void* {
         return p ? (void*)((char*)const_cast<void*>(p) + (size_t)tile0 * comps * 32 * es) : nullptr;
@@ -834,7 +850,7 @@ static vfk_buffers offset_view(const vfk_buffers& b, int64_t tile0, int N, int M
     o.q = off(b.q, N); o.goal = off(b.goal, 13);
     if (b.obst_shared != VFK_OBST_SHARED) { o.obst = off(b.obst, (size_t)((M + 1) & ~1) * 4); o.obst_ext = off(b.obst_ext, (size_t)M * 2); }
     o.aux = off(b.aux, (size_t)b.n_aux * 12);
-    o.jp_ref = off(b.jp_ref, N); o.jp_lo = off(b.jp_lo, N); o.jp_hi = off(b.jp_hi, N); o.ns_lastvec = off(b.ns_lastvec, (size_t)(ns_ctrl_vectors(N) > 0 ? ns_ctrl_vectors(N) : 1) * N); o.q_cmded = off(b.q_cmded, N);
+    o.jp_ref = off(b.jp_ref, N); o.jp_lo = off(b.jp_lo, N); o.jp_hi = off(b.jp_hi, N); o.ns_in = off(b.ns_in, ns_comps); o.ns_lastvec = off(b.ns_lastvec, (size_t)(ns_ctrl_vectors(N) > 0 ? ns_ctrl_vectors(N) : 1) * N); o.q_cmded = off(b.q_cmded, N);
     for (int e = 0; e < 3; ++e) o.ext_cmd[e] = off(b.ext_cmd[e], N);
     o.qdot_vf = off(b.qdot_vf, N); o.qdot_ns = off(b.qdot_ns, N); o.qdot_jp = off(b.qdot_jp, N); o.qdot = off(b.qdot, N);
     o.cmd = off(b.cmd, N); o.pose = off(b.pose, 12); o.twist = off(b.twist, 6);
@@ -849,19 +865,8 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
     vfk_ctx* h = s->h;
     const int N = s->N;
     const size_t es = s->es;
-    vfk_buffers b = s->b;
-    const int M = session_scene(s, &b);
-    b.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
-    b.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
-    b.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
-    b.ns_in = nullptr;                                          // offset separately below (4 or N components)
-    if (!want_flags) b.flags = nullptr;
-    if (!s->en_vf) b.qdot_vf = nullptr;
-    if (!s->en_ns) b.qdot_ns = nullptr;
-    if (!s->en_jp) b.qdot_jp = nullptr;
-    if (!s->en_cmd) b.cmd = nullptr;
-    if (!s->en_pose) b.pose = nullptr;
-    if (!s->en_twist) b.twist = nullptr;
+    vfk_buffers b;
+    const int M = session_view(s, SessionOutputs::enabled, want_flags, &b);
     const int ns_comps = h->params.ns_mode == VFK_NS_CONTROL ? 4 : N;
     const bool piped = n_chunks > 1;
     cudaStream_t st_up = piped ? s->pipe[0] : s->pipe[1], st_k = s->pipe[1], st_dn = piped ? s->pipe[2] : s->pipe[1];
@@ -878,8 +883,7 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
         const int64_t t1 = t0 + tiles_per_chunk < s->tiles ? t0 + tiles_per_chunk : s->tiles;
         const int64_t i0 = t0 * 32;
         const int64_t cnt = (t1 * 32 < s->n ? t1 * 32 : s->n) - i0;
-        vfk_buffers v = offset_view(b, t0, N, M, es);
-        if (s->have_ns_in) v.ns_in = (char*)s->d_ns_in + (size_t)t0 * ns_comps * 32 * es;
+        vfk_buffers v = offset_view(b, t0, N, M, ns_comps, es);
         if (src_q) {
             VFK_CUDA(h, cudaMemcpy2DAsync(stage_q + i0 * es, pitch, src_q + i0 * es, pitch, (size_t)cnt * es, N,
                                           cudaMemcpyHostToDevice, st_up));
@@ -916,89 +920,50 @@ static int enqueue_cycle(vfk_session_s* s, const char* src_q, int k_cycles, char
     return launches;
 }
 
-extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, void* qdot_out, void* q_out,
-                                 int32_t* flags_out) {
-    if (!s) return fail(nullptr, VFK_ERR_INVALID, "vfk_session_cycle: null session");
+// Is p page-locked host memory (cudaHostAlloc / cudaHostRegister / torch pinned memory)?  `mapped` gets its device address,
+// or null.
+static bool host_pinned(const void* p, void** mapped = nullptr) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (mapped) *mapped = at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
+    return at.type == cudaMemoryTypeHost;
+}
+
+// Direct host I/O (zero-copy): when the caller's q_in / qdot_out are page-locked and the batch is tile-aligned, ONE
+// kernel launch reads the q tiles straight from host memory through TMA (N x 128 B bulk copies per tile, prefetched one
+// tile ahead like every other stream of the kernel) and stores qdot straight back with coalesced 128 B writes: no
+// staging copies, no layout kernels, and the PCIe reads, the arithmetic and the PCIe writes overlap at tile
+// granularity instead of chunk granularity.  Measured on B200, 1 M instances (scripts/e2e_direct.sh): 0.79 ms per call
+// against 0.91 ms for the chunked copy pipeline below; hybrids (kernel reads + DMA writes 1.04 ms, DMA reads + kernel
+// writes 0.83 ms) lose to both-direct.  SM-issued PCIe traffic runs at 51 / 52 GB/s one way whatever the request size
+// and ~37 GB/s each way when both directions are busy (scripts/pcie_probe.cu), which is where this path sits.
+// VFK_SESSION_DIRECT=0 selects the copy pipeline.
+static int session_cycle_direct(vfk_session_s* s, void* dq, void* dqd, int k_cycles, char* dst_qo, char* dst_fl, bool want_flags) {
     vfk_ctx* h = s->h;
-    if (k_cycles < 1) return fail(h, VFK_ERR_INVALID, "k_cycles must be >= 1");
-    VFK_CUDA(h, cudaSetDevice(h->device));
-    const size_t blk = (size_t)s->N * (size_t)s->n * s->es;
-    char* pin_q = s->pin;
-    char* pin_qd = s->pin + blk;
-    char* pin_qo = s->pin + 2 * blk;
-    char* pin_fl = s->pin + 3 * blk;
-    // Caller buffers that are already page-locked (cudaHostAlloc / cudaHostRegister / torch pinned
-    // memory) are used directly; pageable ones go through the session's pinned staging area.
-    auto pinned = [](const void* p) {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
-        return at.type == cudaMemoryTypeHost;
-    };
-    const char* src_q = nullptr;
-    if (q_in) {
-        src_q = (const char*)q_in;
-        if (!pinned(q_in)) { memcpy(pin_q, q_in, blk); src_q = pin_q; }
+    vfk_buffers b;
+    const int M = session_view(s, SessionOutputs::enabled, want_flags, &b);
+    cudaStream_t st = s->pipe[1];
+    vfk_io io;
+    io.q_src = dq; io.q_src_ld = s->n;
+    io.qdot = dqd; io.qdot_ld = dqd ? s->n : 0;
+    int rc = step_impl(h, &b, s->n, M, k_cycles, st, &io);
+    if (rc < 0) return rc;
+    int launches = rc;
+    if (dst_qo) {
+        char* stage_qo = (char*)s->stage_out;
+        if ((rc = pack_dispatch(h, stage_qo, b.q, s->N, 1, s->n, true, st, s->n)) < 0) return rc;
+        launches += rc;
+        VFK_CUDA(h, cudaMemcpyAsync(dst_qo, stage_qo, (size_t)s->N * (size_t)s->n * s->es, cudaMemcpyDeviceToHost, st));
     }
-    const bool d_qd = qdot_out && pinned(qdot_out), d_qo = q_out && pinned(q_out), d_fl = flags_out && pinned(flags_out);
+    if (dst_fl) VFK_CUDA(h, cudaMemcpyAsync(dst_fl, s->b.flags, (size_t)s->n * 4, cudaMemcpyDeviceToHost, st));
+    VFK_CUDA(h, cudaStreamSynchronize(st));
+    s->launches = launches;
+    return launches;
+}
 
-    // Direct host I/O (zero-copy): when the caller's q_in / qdot_out are page-locked and the batch is tile-aligned, ONE
-    // kernel launch reads the q tiles straight from host memory through TMA (N x 128 B bulk copies per tile, prefetched one
-    // tile ahead like every other stream of the kernel) and stores qdot straight back with coalesced 128 B writes: no
-    // staging copies, no layout kernels, and the PCIe reads, the arithmetic and the PCIe writes overlap at tile
-    // granularity instead of chunk granularity.  Measured on B200, 1 M instances (scripts/e2e_direct.sh): 0.79 ms per call
-    // against 0.91 ms for the chunked copy pipeline below; hybrids (kernel reads + DMA writes 1.04 ms, DMA reads + kernel
-    // writes 0.83 ms) lose to both-direct.  SM-issued PCIe traffic runs at 51 / 52 GB/s one way whatever the request size
-    // and ~37 GB/s each way when both directions are busy (scripts/pcie_probe.cu), which is where this path sits.
-    // VFK_SESSION_DIRECT=0 selects the copy pipeline.
-    auto mapped = [](const void* p) -> void* {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
-    };
-    const char* de = getenv("VFK_SESSION_DIRECT");
-    const bool direct_ok = !(de && atoi(de) == 0) && q_in && s->n % 32 == 0 && s->n >= kDirectMinInstances;
-    void* dq = direct_ok ? mapped(q_in) : nullptr;
-    void* dqd = (direct_ok && qdot_out) ? mapped(qdot_out) : nullptr;
-    if (dq && (!qdot_out || dqd) && ((uintptr_t)dq % 16 == 0) && ((uintptr_t)dqd % 16 == 0)) {
-        vfk_buffers b = s->b;
-        const int M = session_scene(s, &b);
-        b.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
-    b.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
-    b.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
-        b.ns_in = s->have_ns_in ? s->d_ns_in : nullptr;
-        if (!flags_out) b.flags = nullptr;
-        if (!s->en_vf) b.qdot_vf = nullptr;
-        if (!s->en_ns) b.qdot_ns = nullptr;
-        if (!s->en_jp) b.qdot_jp = nullptr;
-        if (!s->en_cmd) b.cmd = nullptr;
-        if (!s->en_pose) b.pose = nullptr;
-        if (!s->en_twist) b.twist = nullptr;
-        cudaStream_t st = s->pipe[1];
-        vfk_io io;
-        io.q_src = dq; io.q_src_ld = s->n;
-        io.qdot = dqd; io.qdot_ld = dqd ? s->n : 0;
-        int rc = step_impl(h, &b, s->n, M, k_cycles, st, &io);
-        if (rc < 0) return rc;
-        int launches = rc;
-        char* dst_qo = q_out ? (d_qo ? (char*)q_out : pin_qo) : nullptr;
-        char* dst_fl = flags_out ? (d_fl ? (char*)flags_out : pin_fl) : nullptr;
-        if (dst_qo) {
-            char* stage_qo = (char*)s->stage_out;
-            if ((rc = pack_dispatch(h, stage_qo, b.q, s->N, 1, s->n, true, st, s->n)) < 0) return rc;
-            launches += rc;
-            VFK_CUDA(h, cudaMemcpyAsync(dst_qo, stage_qo, blk, cudaMemcpyDeviceToHost, st));
-        }
-        if (dst_fl) VFK_CUDA(h, cudaMemcpyAsync(dst_fl, s->b.flags, (size_t)s->n * 4, cudaMemcpyDeviceToHost, st));
-        VFK_CUDA(h, cudaStreamSynchronize(st));
-        if (q_out && !d_qo) memcpy(q_out, pin_qo, blk);
-        if (flags_out && !d_fl) memcpy(flags_out, pin_fl, (size_t)s->n * 4);
-        s->launches = launches;
-        return launches;
-    }
-    char* dst_qd = qdot_out ? (d_qd ? (char*)qdot_out : pin_qd) : nullptr;
-    char* dst_qo = q_out ? (d_qo ? (char*)q_out : pin_qo) : nullptr;
-    char* dst_fl = flags_out ? (d_fl ? (char*)flags_out : pin_fl) : nullptr;
-
+static int session_cycle_pipeline(vfk_session_s* s, const char* src_q, int k_cycles, char* dst_qd, char* dst_qo, char* dst_fl,
+                                  bool want_flags) {
+    vfk_ctx* h = s->h;
     // Chunk pipeline: a three-stage software pipeline over tile-aligned chunks.  All uploads go back to back on the
     // H2D stream, the kernels of chunk c wait for its upload on the compute stream, and its downloads wait for the
     // kernels on the D2H stream, so the two DMA engines (PCIe is full duplex) and the SMs all stay busy.
@@ -1027,7 +992,7 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
         cudaError_t ce = cudaEventRecord(s->ev_fork, origin);                       // fork the two DMA streams
         if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s->pipe[0], s->ev_fork, 0);
         if (ce == cudaSuccess) ce = cudaStreamWaitEvent(s->pipe[2], s->ev_fork, 0);
-        int rc = ce == cudaSuccess ? enqueue_cycle(s, src_q, k_cycles, dst_qd, dst_qo, dst_fl, flags_out != nullptr, n_chunks) : -1;
+        int rc = ce == cudaSuccess ? enqueue_cycle(s, src_q, k_cycles, dst_qd, dst_qo, dst_fl, want_flags, n_chunks) : -1;
         if (ce == cudaSuccess) ce = cudaEventRecord(s->ev_join[0], s->pipe[0]);     // join them back
         if (ce == cudaSuccess) ce = cudaEventRecord(s->ev_join[1], s->pipe[2]);
         if (ce == cudaSuccess) ce = cudaStreamWaitEvent(origin, s->ev_join[0], 0);
@@ -1051,10 +1016,44 @@ extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, 
         if (s->graph_exec) { cudaGraphExecDestroy(s->graph_exec); s->graph_exec = nullptr; }
         key.src_q = src_q; key.dst_qd = dst_qd; key.dst_qo = dst_qo; key.dst_fl = dst_fl;
         key.k = k_cycles; key.hgen = h->generation; key.sgen = s->generation;
-        launches = enqueue_cycle(s, src_q, k_cycles, dst_qd, dst_qo, dst_fl, flags_out != nullptr, n_chunks);
+        launches = enqueue_cycle(s, src_q, k_cycles, dst_qd, dst_qo, dst_fl, want_flags, n_chunks);
         if (launches < 0) return launches;
     }
     for (int k = 0; k < 3; ++k) VFK_CUDA(h, cudaStreamSynchronize(s->pipe[k]));
+    return launches;
+}
+
+extern "C" int vfk_session_cycle(vfk_session s, const void* q_in, int k_cycles, void* qdot_out, void* q_out,
+                                 int32_t* flags_out) {
+    if (!s) return fail(nullptr, VFK_ERR_INVALID, "vfk_session_cycle: null session");
+    vfk_ctx* h = s->h;
+    if (k_cycles < 1) return fail(h, VFK_ERR_INVALID, "k_cycles must be >= 1");
+    VFK_CUDA(h, cudaSetDevice(h->device));
+    const size_t blk = (size_t)s->N * (size_t)s->n * s->es;
+    char* pin_q = s->pin;
+    char* pin_qd = s->pin + blk;
+    char* pin_qo = s->pin + 2 * blk;
+    char* pin_fl = s->pin + 3 * blk;
+    // Caller buffers that are already page-locked are used directly; pageable ones go through the session's pinned staging
+    // area.
+    const char* src_q = nullptr;
+    if (q_in) {
+        src_q = (const char*)q_in;
+        if (!host_pinned(q_in)) { memcpy(pin_q, q_in, blk); src_q = pin_q; }
+    }
+    const bool d_qd = qdot_out && host_pinned(qdot_out), d_qo = q_out && host_pinned(q_out), d_fl = flags_out && host_pinned(flags_out);
+    char* dst_qd = qdot_out ? (d_qd ? (char*)qdot_out : pin_qd) : nullptr;
+    char* dst_qo = q_out ? (d_qo ? (char*)q_out : pin_qo) : nullptr;
+    char* dst_fl = flags_out ? (d_fl ? (char*)flags_out : pin_fl) : nullptr;
+    const char* de = getenv("VFK_SESSION_DIRECT");
+    const bool direct_ok = !(de && atoi(de) == 0) && q_in && s->n % 32 == 0 && s->n >= kDirectMinInstances;
+    void *dq = nullptr, *dqd = nullptr;
+    if (direct_ok) host_pinned(q_in, &dq);
+    if (direct_ok && qdot_out) host_pinned(qdot_out, &dqd);
+    const bool direct = dq && (!qdot_out || dqd) && ((uintptr_t)dq % 16 == 0) && ((uintptr_t)dqd % 16 == 0);
+    const int launches = direct ? session_cycle_direct(s, dq, dqd, k_cycles, dst_qo, dst_fl, flags_out != nullptr)
+                                : session_cycle_pipeline(s, src_q, k_cycles, dst_qd, dst_qo, dst_fl, flags_out != nullptr);
+    if (launches < 0) return launches;
     if (qdot_out && !d_qd) memcpy(qdot_out, pin_qd, blk);
     if (q_out && !d_qo) memcpy(q_out, pin_qo, blk);
     if (flags_out && !d_fl) memcpy(flags_out, pin_fl, (size_t)s->n * 4);
@@ -1068,11 +1067,8 @@ extern "C" int vfk_session_solve(vfk_session s, const void* q_in, int max_cycles
     int rc;
     if (q_in && (rc = vfk_session_set_q(s, q_in)) != VFK_OK) return rc;
     vfk_buffers b;
-    if ((rc = vfk_session_buffers(s, &b)) != VFK_OK) return rc;
-    b.qdot_vf = b.qdot_ns = b.qdot_jp = b.qdot = b.cmd = b.pose = b.twist = nullptr;
-    b.flags = nullptr;
-    if ((rc = vfk_solve(h, &b, s->n, s->obst_mode == VFK_OBST_SHARED ? s->shared_m : s->n_obst, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr,
-                        s->stream)) < 0)
+    const int M = session_view(s, SessionOutputs::none, false, &b);
+    if ((rc = vfk_solve(h, &b, s->n, M, max_cycles, tol_trans, tol_rot, (int32_t*)s->d_cycles, dist_out ? s->d_dist : nullptr, s->stream)) < 0)
         return rc;
     int launches = rc;
     char* stage = (char*)s->stage_out;                          // dense q [N][n], then dist [2][n]
@@ -1135,12 +1131,8 @@ extern "C" int vfk_session_read(vfk_session s, const char* what, void* out) {
 
 extern "C" int vfk_session_buffers(vfk_session s, vfk_buffers* out) {
     if (!s || !out) return fail(s ? s->h : nullptr, VFK_ERR_INVALID, "vfk_session_buffers: null argument");
-    vfk_buffers v = s->b;
-    session_scene(s, &v);
-    v.jp_ref = s->have_jp_ref ? s->d_jp_ref : nullptr;
-    v.jp_lo = s->have_jp_lim ? s->d_jp_lo : nullptr;
-    v.jp_hi = s->have_jp_lim ? s->d_jp_hi : nullptr;
-    v.ns_in = s->have_ns_in ? s->d_ns_in : nullptr;
+    vfk_buffers v;
+    session_view(s, SessionOutputs::all, true, &v);
     // the mixed-scene fields at the struct's end are written only in that mode: a caller built against the struct without
     // them never selects it, and its shorter struct is not written past its end
     memcpy(out, &v, s->obst_mode == VFK_OBST_MIXED ? sizeof v : offsetof(vfk_buffers, shared_obst));

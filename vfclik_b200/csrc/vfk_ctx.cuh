@@ -62,23 +62,40 @@ inline int fail(vfk_ctx* h, int code, const char* fmt, ...) {
     } while (0)
 
 
-// Cycle-kernel launchers, one translation unit per (precision, joint-count group) so they compile in parallel.
-int vfk_launch_f32_small(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);   // N = 6, 7
-int vfk_launch_f32_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);   // N = 10, 17
-int vfk_launch_f64_small(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
-int vfk_launch_f64_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io);
-// The vfk_solve variants, one translation unit per precision.
-int vfk_solve_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
-int vfk_solve_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
-// The list a shared (obst_shared = 1) or mixed (2) scene gives the whole batch, resolved from vfk_buffers by the ABI layer.
-struct vfk_shared_scene {
-    const void* obst;          // dense [n][4]
-    const void* obst_ext;      // dense [n][2] or null
-    int n;
+// One obstacle list of a scene (m = 0: empty).
+struct vfk_obst_list {
+    const void* obst;          // own list: blocked pairs (vfk.h); shared list: dense [m][4]
+    const void* obst_ext;      // own list: blocked [m][2]; shared list: dense [m][2]; or null
+    int m;
 };
-// The shared-scene variants (vfk_buffers.obst_shared), step and solve, one translation unit each per precision: n_obst
-// instance-own obstacles (mode 2; 0 in mode 1) plus the shared list `sh` (n > 0).
-int vfk_launch_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int k_cycles, cudaStream_t st, const vfk_io* io);
-int vfk_launch_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int k_cycles, cudaStream_t st, const vfk_io* io);
-int vfk_solve_shared_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
-int vfk_solve_shared_f64(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, const vfk_shared_scene* sh, int max_cycles, cudaStream_t st, const vfk_solve_io* sv);
+
+// The scene of a call, resolved once from vfk_buffers by the ABI layer (resolve_scene in vfk_api.cu): the instances' own
+// lists, which run through the obstacle ring, and the list shared by the whole batch, which the SHARED kernels stage into
+// shared memory.  Mode 0 has only own lists, mode 1 only the shared list, mode 2 both.
+struct vfk_scene {
+    vfk_obst_list own, shared;
+};
+
+// One cycle-kernel call, from the ABI down to the launch.
+struct CycleCall {
+    const vfk_buffers* b;
+    int64_t n;
+    int k_cycles;               // vfk_solve: max_cycles
+    cudaStream_t stream;
+    const vfk_io* io;           // direct host I/O of a session, or null
+    const vfk_solve_io* sv;     // vfk_solve's stop rule and results; null for a step
+    vfk_scene scene;
+};
+
+// Cycle-kernel launchers, one translation unit each so they compile in parallel: the step kernels per (precision, joint-count
+// group), and per precision the vfk_solve kernels and the SHARED step and solve kernels (a non-empty shared list).
+int vfk_launch_f32_small(vfk_ctx* h, const CycleCall& call);   // N = 6, 7
+int vfk_launch_f32_large(vfk_ctx* h, const CycleCall& call);   // N = 10, 17
+int vfk_launch_f64_small(vfk_ctx* h, const CycleCall& call);
+int vfk_launch_f64_large(vfk_ctx* h, const CycleCall& call);
+int vfk_solve_f32(vfk_ctx* h, const CycleCall& call);
+int vfk_solve_f64(vfk_ctx* h, const CycleCall& call);
+int vfk_launch_shared_f32(vfk_ctx* h, const CycleCall& call);
+int vfk_launch_shared_f64(vfk_ctx* h, const CycleCall& call);
+int vfk_solve_shared_f32(vfk_ctx* h, const CycleCall& call);
+int vfk_solve_shared_f64(vfk_ctx* h, const CycleCall& call);

@@ -1,11 +1,4 @@
 // Instantiates the fused cycle kernel for float, N in {6, 7} (own translation unit: compiles in parallel).
 #include "vfk_launch.cuh"
 
-int vfk_launch_f32_small(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io) {
-    const KConst<float>& c = h->cf;
-    switch (h->n_kernel) {
-        case 6: return dispatch_ext<float, 6>(h, c, b, n, n_obst, k_cycles, st, io);
-        case 7: return dispatch_ext<float, 7>(h, c, b, n, n_obst, k_cycles, st, io);
-    }
-    return fail(h, VFK_ERR_UNSUPPORTED, "no kernel for n_joints = %d", h->chain.n_joints);
-}
+int vfk_launch_f32_small(vfk_ctx* h, const CycleCall& call) { return launch_family<float, false, false, 6, 7>(h, call); }

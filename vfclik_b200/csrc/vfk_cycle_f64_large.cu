@@ -1,11 +1,4 @@
 // Instantiates the fused cycle kernel for double, N in {10, 17} (own translation unit: compiles in parallel).
 #include "vfk_launch.cuh"
 
-int vfk_launch_f64_large(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st, const vfk_io* io) {
-    const KConst<double>& c = h->cd;
-    switch (h->n_kernel) {
-        case 10: return dispatch_ext<double, 10>(h, c, b, n, n_obst, k_cycles, st, io);
-        case 17: return dispatch_ext<double, 17>(h, c, b, n, n_obst, k_cycles, st, io);
-    }
-    return fail(h, VFK_ERR_UNSUPPORTED, "no kernel for n_joints = %d", h->chain.n_joints);
-}
+int vfk_launch_f64_large(vfk_ctx* h, const CycleCall& call) { return launch_family<double, false, false, 10, 17>(h, call); }

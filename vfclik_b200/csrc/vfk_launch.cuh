@@ -1,4 +1,4 @@
-// vfk_launch.cuh -- launch plan and feature dispatch of the fused cycle kernel (included by vfk_cycle_*.cu).
+// vfk_launch.cuh -- launch plan and feature dispatch of the fused cycle kernel (included by the ten launcher units).
 #pragma once
 #include <cmath>
 #include <cstdlib>
@@ -18,17 +18,6 @@ using namespace vfk;
 // (4: 0.697; 6 and 8 cost a resident CTA: 0.44); everywhere else a third stage costs occupancy (config 4: 1.009 -> 0.988).
 template <typename T, int N>
 constexpr int kRingStages = (sizeof(T) == 4 && N >= 10) ? 3 : 2;
-
-template <typename T, int N, bool EXT>
-static void plan_stages(int n_obst, int* n_chunks, int* n_stages, size_t* smem_bytes) {
-    using WS = WarpStage<T, N, EXT>;
-    *n_chunks = (n_obst + kChunk - 1) / kChunk;
-    int stages = kRingStages<T, N>;
-    if (*n_chunks > 0 && *n_chunks < stages) stages = *n_chunks;
-    if (*n_chunks == 0) stages = 0;
-    *n_stages = stages;
-    *smem_bytes = kSmemHeader + kTabBytes<T> + (size_t)(kBlock / 32) * WS::warp_bytes(stages);
-}
 
 // Launch plan of one kernel instantiation: resident CTAs per SM for a given dynamic shared-memory size, per device.  One
 // instance per instantiation (function-local static at the call site); a handful of (device, smem) entries behind a mutex, so
@@ -53,6 +42,37 @@ struct PlanCache {
 
 constexpr int64_t kCoopMaxInstances = 4096;      // <= 128 tiles: 1024 cooperative warps instead of 128 solo ones
 
+template <typename T>
+static const KConst<T>& kconst(const vfk_ctx* h) {
+    if constexpr (sizeof(T) == 4) return h->cf; else return h->cd;
+}
+
+// Chunk plan of a list of m obstacles, as KArgs holds it for the own list and for the shared list: the count, whole pairs,
+// chunks of kChunk obstacles, full chunks and the remainder.
+static void chunk_plan(int m, int32_t& n, int32_t& np, int32_t& chunks, int32_t& full, int32_t& rem) {
+    n = m;
+    np = (m + 1) & ~1;
+    chunks = (m + kChunk - 1) / kChunk;
+    full = m / kChunk;
+    rem = m % kChunk;
+}
+
+// The launch of every cycle-kernel shape: `units` warp-sized work units, each warp a persistent worker, so at most as many
+// CTAs as fit the SMs at once.  One plan cache per kernel instantiation: opt in to > 48 KB of dynamic shared memory and ask
+// the occupancy once per (device, smem size).
+template <auto kern, typename... Args>
+static int launch_persistent(vfk_ctx* h, int64_t units, size_t smem, cudaStream_t st, const Args&... args) {
+    static PlanCache plans;
+    int per_sm = 0;
+    VFK_CUDA(h, plans.get(kern, h->device, smem, &per_sm));
+    if (per_sm < 1) return fail(h, VFK_ERR_CUDA, "kernel does not fit an SM with %zu bytes of shared memory", smem);
+    const int64_t want = (units + kBlock / 32 - 1) / (kBlock / 32);
+    const int64_t cap = (int64_t)h->sm_count * per_sm;
+    kern<<<(unsigned)(want < cap ? want : cap), kBlock, smem, st>>>(args...);
+    VFK_CUDA(h, cudaGetLastError());
+    return 1;
+}
+
 // The LEAN kernel's preconditions (see vfk_kernels.cuh): on the constants and inputs (all a solve has to meet, since it
 // has no per-cycle outputs), and for a step also on the outputs.
 template <typename T>
@@ -70,19 +90,20 @@ static bool is_lean(const KConst<T>& c, const vfk_buffers* b) {
 // HIOCC: the single-cycle lean FP32 launch asks for one more resident CTA per SM (4 x 128 threads at 128 registers, no
 // spills).  Measured on B200, 1 M instances: 109.5 us vs 111.2 us per launch at K = 1 (more warps hide more HBM latency),
 // but 1.6 % slower at K = 100, where the kernel is issue-bound and the tighter register budget costs instructions.
-// SOLVE: the vfk_solve variant (vfk_kernels.cuh), with its stop rule and result buffers in `sv`.
-// SHARED: one obstacle list for the whole batch (vfk_buffers.obst_shared), `sh`, staged into shared memory per CTA; the
-// n_obst obstacles of the instance's own list (a mixed scene; 0 in a shared-only call) run through the ring as usual.
+// SOLVE: the vfk_solve variant (vfk_kernels.cuh), with its stop rule and result buffers in `call.sv`.
+// SHARED: the scene's shared list, staged into shared memory per CTA; the own list (a mixed scene; empty in a shared-only
+// call) runs through the ring as usual.
 template <typename T, int N, class PAT, bool EXT, bool LEAN, int G = 1, bool HIOCC = false, bool SOLVE = false, bool SHARED = false>
-static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
+static int launch_cycle(vfk_ctx* h, const CycleCall& call) {
+    const vfk_buffers* b = call.b;
+    const vfk_scene& sc = call.scene;
+    const vfk_io* io = call.io;
     KArgs<T> a;
     memset(&a, 0, sizeof a);
     a.q = static_cast<T*>(b->q);
     a.goal = static_cast<const T*>(b->goal);
-    // (in a shared-only call b->obst is the shared list, and there is no own list)
-    a.obst = (!SHARED || n_obst > 0) ? static_cast<const Vec4<T>*>(b->obst) : nullptr;
-    a.obst_ext = (!SHARED || n_obst > 0) ? static_cast<const Vec2<T>*>(b->obst_ext) : nullptr;
+    a.obst = static_cast<const Vec4<T>*>(sc.own.obst);
+    a.obst_ext = static_cast<const Vec2<T>*>(sc.own.obst_ext);
     a.aux = b->n_aux > 0 ? static_cast<const T*>(b->aux) : nullptr;
     a.n_aux = a.aux ? b->n_aux : 0;
     a.jp_ref = static_cast<T*>(b->jp_ref);
@@ -102,24 +123,22 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     a.flags = b->flags;
     if (io && io->q_src) { a.q_src = static_cast<const T*>(io->q_src); a.q_src_ld = io->q_src_ld; }
     if (io && io->qdot) { a.qdot = static_cast<T*>(io->qdot); a.qdot_ld = io->qdot_ld; a.qdot_dev = static_cast<T*>(b->qdot); }
-    a.n = n;
+    a.n = call.n;
     a.n_comp = h->chain.n_joints;
-    a.n_obst = n_obst;
-    a.n_obst_p = (n_obst + 1) & ~1;
-    a.k_cycles = k_cycles;
+    a.k_cycles = call.k_cycles;
     if constexpr (SOLVE) {
         // thresholds in T: |dp|^2 against tol_trans^2, and |xyz|^2 = sin^2(angle / 2) of the error quaternion against
         // sin^2(tol_rot / 2) -- exact and monotone on [0, pi], no transcendental in the kernel
+        const vfk_solve_io* sv = call.sv;
         a.tol_d2 = (T)(sv->tol_trans * sv->tol_trans);
         const double sh_rot = std::sin(0.5 * sv->tol_rot);
         a.tol_q2 = sv->tol_rot >= 3.14159265358979323846 ? (T)INFINITY : (T)(sh_rot * sh_rot);
         a.cycles = sv->cycles;
         a.dist = static_cast<T*>(sv->dist);
     }
-    size_t smem = 0;
-    plan_stages<T, N, EXT>(n_obst, &a.n_chunks, &a.n_stages, &smem);
-    a.n_full = n_obst / kChunk;
-    a.n_rem = n_obst % kChunk;
+    chunk_plan(sc.own.m, a.n_obst, a.n_obst_p, a.n_chunks, a.n_full, a.n_rem);
+    a.n_stages = a.n_chunks < kRingStages<T, N> ? a.n_chunks : kRingStages<T, N>;
+    size_t smem = kSmemHeader + kTabBytes<T> + (size_t)(kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(a.n_stages);
     if constexpr (SHARED) {
         // Shared memory: the own ring (its usual plan on the own count; no stages without one), the staged shared list and
         // the q / goal buffers.  Every instantiation fits an SM with an own list at the largest stage count and a shared
@@ -127,13 +146,9 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
         static_assert(kSmemHeader + kTabBytes<T> + shared_scene_bytes<T, EXT>(VFK_MAX_SHARED_OBSTACLES, VFK_MAX_SHARED_OBSTACLES) +
                           (kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(kRingStages<T, N>) <= (227u << 10),
                       "a mixed scene at the shared-list cap does not fit an SM");
-        a.sh_obst = static_cast<const T*>(sh->obst);
-        a.sh_obst_ext = static_cast<const T*>(sh->obst_ext);
-        a.sh_n = sh->n;
-        a.sh_np = (sh->n + 1) & ~1;
-        a.sh_chunks = (sh->n + kChunk - 1) / kChunk;
-        a.sh_full = sh->n / kChunk;
-        a.sh_rem = sh->n % kChunk;
+        a.sh_obst = static_cast<const T*>(sc.shared.obst);
+        a.sh_obst_ext = static_cast<const T*>(sc.shared.obst_ext);
+        chunk_plan(sc.shared.m, a.sh_n, a.sh_np, a.sh_chunks, a.sh_full, a.sh_rem);
         smem += shared_scene_bytes<T, EXT>(a.sh_np, a.sh_n);
     }
     // resident CTAs per SM that the register allocation aims for.  The shared-scene FP32 lean solve kernels of N <= 7 ask for
@@ -141,19 +156,9 @@ static int launch_cycle(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, in
     // takes 127 without spilling; the 7-joint generic one spills 24 bytes, as its HIOCC step twin does)
     constexpr int MINB = (HIOCC || (SHARED && SOLVE && LEAN && sizeof(T) == 4 && N <= 7)) ? 4
                          : (sizeof(T) == 4 ? (N <= 10 ? 3 : 2) : (N <= 7 ? 2 : 1));
-    auto kern = vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, SOLVE, SHARED>;
-    // per (instantiation, device, smem size): opt in to > 48 KB of dynamic shared memory and ask the occupancy once
-    static PlanCache plans;
-    int per_sm = 0;
-    VFK_CUDA(h, plans.get(kern, h->device, smem, &per_sm));
-    if (per_sm < 1) return fail(h, VFK_ERR_CUDA, "kernel does not fit an SM with %zu bytes of shared memory", smem);
-    const int64_t units = (n + 31) / 32 * G;                 // G = 8: a tile is spread over 8 warps (4 instances each)
-    const int64_t want = (units + kBlock / 32 - 1) / (kBlock / 32);
-    const int64_t cap = (int64_t)h->sm_count * per_sm;
-    const unsigned grid = (unsigned)(want < cap ? want : cap);
-    kern<<<grid, kBlock, smem, st>>>(c, a);
-    VFK_CUDA(h, cudaGetLastError());
-    return 1;
+    // G = 8: a tile is spread over 8 warps (4 instances each)
+    return launch_persistent<vfk_cycle_kernel<T, N, PAT, EXT, LEAN, MINB, G, SOLVE, SHARED>>(h, (call.n + 31) / 32 * G, smem, call.stream,
+                                                                                           kconst<T>(h), a);
 }
 
 // ------------------------------------------------------------------------------ lane-split shape (vfk_split.cuh)
@@ -201,95 +206,92 @@ constexpr bool kSplit = sizeof(T) == 8 && N == 17;
 // May this call run in the lane-split shape?  Lean call on blocked device buffers, DH-form chain of exactly the instantiated
 // length.  VFK_NO_SPLIT=1 runs the one-thread-per-instance kernel instead (the reference the tests compare against).
 template <typename T>
-static bool split_ok(vfk_ctx* h, int n_kernel, const KConst<T>& c, const vfk_buffers* b, const vfk_io* io) {
-    return !getenv("VFK_NO_SPLIT") && h->dh_chain && h->chain.n_joints == n_kernel && is_lean<T>(c, b) && !(io && (io->q_src || io->qdot));
+static bool split_ok(vfk_ctx* h, int n_kernel, const CycleCall& call) {
+    const vfk_io* io = call.io;
+    return !getenv("VFK_NO_SPLIT") && h->dh_chain && h->chain.n_joints == n_kernel && is_lean<T>(kconst<T>(h), call.b) &&
+           !(io && (io->q_src || io->qdot));
 }
 
 template <typename T, int N>
-static int launch_split(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles, cudaStream_t st) {
+static int launch_split(vfk_ctx* h, const CycleCall& call) {
     using SH = SplitShape<T, N>;
+    const vfk_buffers* b = call.b;
     KArgs<T> a;
     memset(&a, 0, sizeof a);
     a.q = static_cast<T*>(b->q);
     a.qdot = static_cast<T*>(b->qdot);
-    a.n = n;
+    a.n = call.n;
     a.n_comp = h->chain.n_joints;
-    a.n_obst = n_obst;
-    a.n_obst_p = (n_obst + 1) & ~1;
-    a.k_cycles = k_cycles;
-    a.n_chunks = (n_obst + kChunk - 1) / kChunk;
-    a.n_full = n_obst / kChunk;
-    a.n_rem = n_obst % kChunk;
+    a.k_cycles = call.k_cycles;
+    chunk_plan(call.scene.own.m, a.n_obst, a.n_obst_p, a.n_chunks, a.n_full, a.n_rem);
     a.n_stages = a.n_chunks < 2 ? a.n_chunks : 2;
     const size_t smem = kSmemHeader + SH::kTab + (size_t)(kBlock / 32) * SH::warp_bytes(a.n_stages);
-    const uint64_t tiles = (uint64_t)((n + 31) / 32);
+    const uint64_t tiles = (uint64_t)((call.n + 31) / 32);
     SplitMaps maps;
     memset(&maps, 0, sizeof maps);
     int rc;
     if ((rc = encode_map3<T>(h, &maps.q, b->q, 32, (uint64_t)a.n_comp, tiles, SH::SUB, (uint32_t)a.n_comp)) != VFK_OK) return rc;
     if ((rc = encode_map3<T>(h, &maps.goal, b->goal, 32, 13, tiles, SH::SUB, 13)) != VFK_OK) return rc;
-    if (n_obst > 0) {
+    if (a.n_obst > 0) {
         const uint64_t rows = (uint64_t)a.n_obst_p / 2 * ObstPairs<T>::kPlanes;                   // plane rows of 32 lanes x 16 bytes per tile
-        if ((rc = encode_map3<T>(h, &maps.obst, b->obst, 32 * 16 / sizeof(T), rows, tiles, SH::kRowBytes / sizeof(T), SH::kRowsPerChunk)) != VFK_OK)
+        if ((rc = encode_map3<T>(h, &maps.obst, call.scene.own.obst, 32 * 16 / sizeof(T), rows, tiles, SH::kRowBytes / sizeof(T),
+                                 SH::kRowsPerChunk)) != VFK_OK)
             return rc;
     }
-    auto kern = vfk_split_kernel<T, N>;
-    static PlanCache plans;
-    int per_sm = 0;
-    VFK_CUDA(h, plans.get(kern, h->device, smem, &per_sm));
-    if (per_sm < 1) return fail(h, VFK_ERR_CUDA, "split kernel does not fit an SM with %zu bytes of shared memory", smem);
-    const int64_t units = (n + 31) / 32 * SH::L;
-    const int64_t want = (units + kBlock / 32 - 1) / (kBlock / 32);
-    const int64_t cap = (int64_t)h->sm_count * per_sm;
-    const unsigned grid = (unsigned)(want < cap ? want : cap);
-    kern<<<grid, kBlock, smem, st>>>(c, a, maps);
-    VFK_CUDA(h, cudaGetLastError());
-    return 1;
+    return launch_persistent<vfk_split_kernel<T, N>>(h, (call.n + 31) / 32 * SH::L, smem, call.stream, kconst<T>(h), a, maps);
 }
 
 // SOLVE: the same choice of shape for vfk_solve, except that the lane-split shape has no solve variant (those calls run
 // the one-thread-per-instance kernel) and the lean kernel's output conditions do not apply.
-// SHARED (a shared scene, M > 0): the same choices among the one-thread-per-instance kernels -- EXT, lean / general, HIOCC --
+// SHARED (a non-empty shared list): the same choices among the one-thread-per-instance kernels -- EXT, lean / general, HIOCC --
 // but neither the cooperative shape (FP64, n <= 4096) nor the lane-split shape (FP64, 17 joints) has a shared variant:
 // those calls run the one-thread kernel, whose field they match bit for bit (DESIGN.md section 4.5).
 // A mixed scene (own list and shared list) takes the same SHARED kernels; with ext rows both lists carry them.
-template <typename T, int N, class PAT, bool SOLVE = false, bool SHARED = false>
-static int dispatch_feat(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                         cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
-    bool ext = b->obst_ext && n_obst > 0;
-    if constexpr (SHARED) ext = ext || (sh->obst_ext && sh->n > 0);
+template <typename T, int N, class PAT, bool SOLVE, bool SHARED>
+static int dispatch_feat(vfk_ctx* h, const CycleCall& call) {
+    const KConst<T>& c = kconst<T>(h);
+    const vfk_buffers* b = call.b;
+    const vfk_scene& sc = call.scene;
+    const bool ext = (sc.own.obst_ext && sc.own.m > 0) || (sc.shared.obst_ext && sc.shared.m > 0);
     // Small FP64 batches cannot fill the GPU with one thread per instance: switch to the cooperative latency shape.
     // Measured (scripts/latency.py, one robot, 1000 fused cycles): FP64 M = 32: 6.4 vs 7.1 us per cycle, M = 256: 23.6 vs
     // 36.3 us.  In FP32 the repeller is three MUFU instructions and the shape only adds ring overhead (3.7 vs 2.7 us),
     // so it is neither selected nor instantiated there.
     if constexpr (sizeof(T) == 8 && !SHARED) {
-        const bool coop = n <= kCoopMaxInstances && n_obst >= 2 * kChunk && !getenv("VFK_NO_COOP");
-        if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv)
-                             : launch_cycle<T, N, PAT, false, false, kChunk, false, SOLVE>(h, c, b, n, n_obst, k_cycles, st, io, sv);
+        const bool coop = call.n <= kCoopMaxInstances && sc.own.m >= 2 * kChunk && !getenv("VFK_NO_COOP");
+        if (coop) return ext ? launch_cycle<T, N, PAT, true, false, kChunk, false, SOLVE>(h, call)
+                             : launch_cycle<T, N, PAT, false, false, kChunk, false, SOLVE>(h, call);
     }
-    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+    if (ext) return launch_cycle<T, N, PAT, true, false, 1, false, SOLVE, SHARED>(h, call);
     // Two lanes per instance (vfk_split.cuh) for the FP64 17-joint kernel.
     if constexpr (kSplit<T, N> && !SOLVE && !SHARED) {
-        if (n_obst > 0 && split_ok<T>(h, N, c, b, io)) return launch_split<T, N>(h, c, b, n, n_obst, k_cycles, st);
+        if (sc.own.m > 0 && split_ok<T>(h, N, call)) return launch_split<T, N>(h, call);
     }
     if ((SOLVE ? lean_inputs<T>(c, b) : is_lean<T>(c, b)) && h->chain.n_joints == N) {
         if constexpr (sizeof(T) == 4 && N <= 7 && !SOLVE) {
-            if (k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true, false, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, nullptr, sh);
+            if (call.k_cycles == 1) return launch_cycle<T, N, PAT, false, true, 1, true, false, SHARED>(h, call);
         }
-        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+        return launch_cycle<T, N, PAT, false, true, 1, false, SOLVE, SHARED>(h, call);
     }
-    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+    return launch_cycle<T, N, PAT, false, false, 1, false, SOLVE, SHARED>(h, call);
 }
 
-template <typename T, int N, bool SOLVE = false, bool SHARED = false>
-static int dispatch_ext(vfk_ctx* h, const KConst<T>& c, const vfk_buffers* b, int64_t n, int n_obst, int k_cycles,
-                        cudaStream_t st, const vfk_io* io, const vfk_solve_io* sv = nullptr, const vfk_shared_scene* sh = nullptr) {
+template <typename T, int N, bool SOLVE, bool SHARED>
+static int dispatch_ext(vfk_ctx* h, const CycleCall& call) {
     if constexpr (N == 7) {
-        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+        if (h->pattern == 1) return dispatch_feat<T, N, LwrPattern, SOLVE, SHARED>(h, call);
     }
     if constexpr (N >= 10) {
-        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+        if (h->pattern == 2) return dispatch_feat<T, N, DhPattern, SOLVE, SHARED>(h, call);
     }
-    return dispatch_feat<T, N, GenericPattern, SOLVE, SHARED>(h, c, b, n, n_obst, k_cycles, st, io, sv, sh);
+    return dispatch_feat<T, N, GenericPattern, SOLVE, SHARED>(h, call);
 }
 
+// The body of every launcher: the kernels of one precision, step or solve, per-instance or SHARED, for the joint counts Ns
+// its translation unit instantiates, picked by the chain's kernel joint count.
+template <typename T, bool SOLVE, bool SHARED, int... Ns>
+static int launch_family(vfk_ctx* h, const CycleCall& call) {
+    int rc = 0;
+    if (((h->n_kernel == Ns && (rc = dispatch_ext<T, Ns, SOLVE, SHARED>(h, call), true)) || ...)) return rc;
+    return fail(h, VFK_ERR_UNSUPPORTED, "no kernel for n_joints = %d", h->chain.n_joints);
+}

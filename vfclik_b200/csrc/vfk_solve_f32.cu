@@ -2,13 +2,4 @@
 // translation unit: compiles in parallel with the step kernels).
 #include "vfk_launch.cuh"
 
-int vfk_solve_f32(vfk_ctx* h, const vfk_buffers* b, int64_t n, int n_obst, int max_cycles, cudaStream_t st, const vfk_solve_io* sv) {
-    const KConst<float>& c = h->cf;
-    switch (h->n_kernel) {
-        case 6: return dispatch_ext<float, 6, true>(h, c, b, n, n_obst, max_cycles, st, nullptr, sv);
-        case 7: return dispatch_ext<float, 7, true>(h, c, b, n, n_obst, max_cycles, st, nullptr, sv);
-        case 10: return dispatch_ext<float, 10, true>(h, c, b, n, n_obst, max_cycles, st, nullptr, sv);
-        case 17: return dispatch_ext<float, 17, true>(h, c, b, n, n_obst, max_cycles, st, nullptr, sv);
-    }
-    return fail(h, VFK_ERR_UNSUPPORTED, "no kernel for n_joints = %d", h->chain.n_joints);
-}
+int vfk_solve_f32(vfk_ctx* h, const CycleCall& call) { return launch_family<float, true, false, 6, 7, 10, 17>(h, call); }

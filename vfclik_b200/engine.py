@@ -174,6 +174,11 @@ class Engine:
             raise VfkError(rc, self._lib.vfk_last_error(self._h).decode())
         return rc
 
+    def _launched(self, rc: int) -> int:
+        """``_check`` for a call that returns the number of kernels it launched: counts them in ``launches``."""
+        self.launches += self._check(rc)
+        return rc
+
     def set_params(self, params: Optional[Params] = None, **over):
         if params is None:
             params = self.params
@@ -225,10 +230,8 @@ class Engine:
         ``bufs["shared_obst"]`` / ``bufs["shared_obst_ext"]`` one dense list for the whole batch, summed after the own ones.
         Its length is ``n_shared_obstacles``, else ``bufs["n_shared_obst"]``, else the array's."""
         b = self._buffers(bufs, ext_cmd, obst_shared, n_shared_obstacles)
-        rc = self._check(self._lib.vfk_step(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(k_cycles),
-                                            self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_step(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(k_cycles),
+                                                  self._stream(stream)))
 
     def solve(self, bufs: Dict[str, object], n_instances: int, n_obstacles: int, max_cycles: int, tol_trans: float,
               tol_rot: float, cycles_out, dist_out=None, stream: Optional[int] = None, ext_cmd=(None, None, None),
@@ -239,69 +242,53 @@ class Engine:
         ``dist_out`` [2] the distance and angle to the goal at the returned q; q is updated in place.  ``bufs`` may hold
         no per-cycle output; ``obst_shared`` and the shared list as in ``step``.  Returns the number of kernels launched."""
         b = self._buffers(bufs, ext_cmd, obst_shared, n_shared_obstacles)
-        rc = self._check(self._lib.vfk_solve(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(max_cycles),
-                                             float(tol_trans), float(tol_rot), _dev_ptr(cycles_out), _dev_ptr(dist_out),
-                                             self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_solve(self._h, C.byref(b), int(n_instances), int(n_obstacles), int(max_cycles),
+                                                   float(tol_trans), float(tol_rot), _dev_ptr(cycles_out), _dev_ptr(dist_out),
+                                                   self._stream(stream)))
 
     def field_eval(self, pose, goal, obst, twist_out, n_instances, n_obstacles, obst_ext=None, aux=None, n_aux=0,
                    stream=None) -> int:
-        rc = self._check(self._lib.vfk_field_eval(self._h, _dev_ptr(pose), _dev_ptr(goal), _dev_ptr(obst),
-                                                  _dev_ptr(obst_ext), _dev_ptr(aux), int(n_aux), _dev_ptr(twist_out),
-                                                  int(n_instances), int(n_obstacles), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_field_eval(self._h, _dev_ptr(pose), _dev_ptr(goal), _dev_ptr(obst),
+                                                        _dev_ptr(obst_ext), _dev_ptr(aux), int(n_aux), _dev_ptr(twist_out),
+                                                        int(n_instances), int(n_obstacles), self._stream(stream)))
 
     def field_eval_scene(self, pose, bufs: Dict[str, object], twist_out, n_instances: int, n_obstacles: int,
                          obst_shared: Optional[int] = None, n_shared_obstacles: Optional[int] = None, stream=None) -> int:
         """The field query (``vfk_field_eval_scene``) at tool poses ``pose`` [12] on the scene of ``bufs`` as ``step`` reads
         it: ``goal``, ``obst`` / ``obst_ext``, ``aux`` and, by ``obst_shared``, the shared list.  ``twist_out`` [6]."""
         b = self._buffers(bufs, (None, None, None), obst_shared, n_shared_obstacles)
-        rc = self._check(self._lib.vfk_field_eval_scene(self._h, _dev_ptr(pose), C.byref(b), int(n_instances), int(n_obstacles),
-                                                        _dev_ptr(twist_out), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_field_eval_scene(self._h, _dev_ptr(pose), C.byref(b), int(n_instances), int(n_obstacles),
+                                                              _dev_ptr(twist_out), self._stream(stream)))
 
     def mix(self, cmds, weights, out, n_channels, n_instances, nan_flags=None, stream=None) -> int:
         n_ports = len(cmds)
         arr = (C.c_void_p * n_ports)(*[_dev_ptr(c) for c in cmds])
         w = (C.c_double * n_ports)(*[float(x) for x in weights])
-        rc = self._check(self._lib.vfk_mix(self._h, arr, w, n_ports, int(n_channels), _dev_ptr(out),
-                                           _dev_ptr(nan_flags), int(n_instances), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_mix(self._h, arr, w, n_ports, int(n_channels), _dev_ptr(out),
+                                                 _dev_ptr(nan_flags), int(n_instances), self._stream(stream)))
 
     def set_vel(self, qdot, q, cmd_out, max_vel: float, direct_control: bool, n_channels: int, n_instances: int,
                 q_cmded=None, qdot_lim_out=None, stream=None) -> int:
         """``LWR_Bridge.set_vel`` arithmetic (``scripts/bridge:188-203``) on blocked device buffers."""
-        rc = self._check(self._lib.vfk_set_vel(self._h, _dev_ptr(qdot), _dev_ptr(q), _dev_ptr(q_cmded), float(max_vel),
-                                               int(bool(direct_control)), _dev_ptr(cmd_out), _dev_ptr(qdot_lim_out),
-                                               int(n_channels), int(n_instances), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_set_vel(self._h, _dev_ptr(qdot), _dev_ptr(q), _dev_ptr(q_cmded), float(max_vel),
+                                                     int(bool(direct_control)), _dev_ptr(cmd_out), _dev_ptr(qdot_lim_out),
+                                                     int(n_channels), int(n_instances), self._stream(stream)))
 
     def monitor(self, pose, twist, goal, state_f, state_i, n_instances: int, track_out=None, dist_out=None,
                 tracking_state_out=None, stream=None) -> int:
         """Tracking diagnostics + distance monitor (``scripts/vf:349-428``, ``scripts/monitor_distance:148-219``)."""
-        rc = self._check(self._lib.vfk_monitor(self._h, _dev_ptr(pose), _dev_ptr(twist), _dev_ptr(goal), _dev_ptr(state_f),
-                                               _dev_ptr(state_i), _dev_ptr(track_out), _dev_ptr(dist_out),
-                                               _dev_ptr(tracking_state_out), int(n_instances), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_monitor(self._h, _dev_ptr(pose), _dev_ptr(twist), _dev_ptr(goal), _dev_ptr(state_f),
+                                                     _dev_ptr(state_i), _dev_ptr(track_out), _dev_ptr(dist_out),
+                                                     _dev_ptr(tracking_state_out), int(n_instances), self._stream(stream)))
 
     def pack(self, dense, blocked, comps: int, width: int, n_instances: int, stream=None) -> int:
         """dense SoA [comps][n] (x width scalars) -> tile-blocked, on the device."""
-        rc = self._check(self._lib.vfk_pack(self._h, _dev_ptr(dense), _dev_ptr(blocked), int(comps), int(width),
-                                            int(n_instances), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_pack(self._h, _dev_ptr(dense), _dev_ptr(blocked), int(comps), int(width),
+                                                  int(n_instances), self._stream(stream)))
 
     def unpack(self, blocked, dense, comps: int, width: int, n_instances: int, stream=None) -> int:
-        rc = self._check(self._lib.vfk_unpack(self._h, _dev_ptr(blocked), _dev_ptr(dense), int(comps), int(width),
-                                              int(n_instances), self._stream(stream)))
-        self.launches += rc
-        return rc
+        return self._launched(self._lib.vfk_unpack(self._h, _dev_ptr(blocked), _dev_ptr(dense), int(comps), int(width),
+                                                    int(n_instances), self._stream(stream)))
 
     def alloc(self, comps: int, n_instances: int, width: int = 1, dtype=None):
         """Zeroed blocked device tensor ``[tiles, comps, 32(, width)]`` for ``n_instances`` instances
@@ -320,6 +307,15 @@ class Engine:
     # -- host-buffer path
     def session(self, n_instances: int, n_obstacles: int, obst_ext: bool = False) -> "Session":
         return Session(self, n_instances, n_obstacles, obst_ext)
+
+
+def _out_ptr(a, shape, dt):
+    """Pointer to a host output array the session fills in place (None: not requested)."""
+    if a is None:
+        return None
+    if a.dtype != dt or a.shape != shape or not a.flags.c_contiguous:
+        raise ValueError("output array must be contiguous %s %r" % (dt, shape))
+    return _lib.np_ptr(a)
 
 
 class Session:
@@ -435,22 +431,13 @@ class Session:
         """
         N = self.e.n_joints
 
-        def out_ptr(a, shape, dt):
-            if a is None:
-                return None
-            if a.dtype != dt or a.shape != shape or not a.flags.c_contiguous:
-                raise ValueError("output array must be contiguous %s %r" % (dt, shape))
-            return _lib.np_ptr(a)
-
         qp = None
         if q_in is not None:
             q_in = self._arr(q_in, N)
             qp = _lib.np_ptr(q_in)
-        rc = self.e._check(self.e._lib.vfk_session_cycle(
-            self._s, qp, int(k_cycles), out_ptr(qdot_out, (N, self.n), self.e.np_dtype),
-            out_ptr(q_out, (N, self.n), self.e.np_dtype), out_ptr(flags_out, (self.n,), np.int32)))
-        self.e.launches += rc
-        return rc
+        return self.e._launched(self.e._lib.vfk_session_cycle(
+            self._s, qp, int(k_cycles), _out_ptr(qdot_out, (N, self.n), self.e.np_dtype),
+            _out_ptr(q_out, (N, self.n), self.e.np_dtype), _out_ptr(flags_out, (self.n,), np.int32)))
 
     def solve(self, q_in=None, max_cycles: int = 1000, tol_trans: float = 1e-3, tol_rot: float = 1e-2, q_out=None,
               cycles_out=None, dist_out=None) -> int:
@@ -459,22 +446,13 @@ class Session:
         int32 ``[n]``."""
         N = self.e.n_joints
 
-        def out_ptr(a, shape, dt):
-            if a is None:
-                return None
-            if a.dtype != dt or a.shape != shape or not a.flags.c_contiguous:
-                raise ValueError("output array must be contiguous %s %r" % (dt, shape))
-            return _lib.np_ptr(a)
-
         qp = None
         if q_in is not None:
             q_in = self._arr(q_in, N)
             qp = _lib.np_ptr(q_in)
-        rc = self.e._check(self.e._lib.vfk_session_solve(
-            self._s, qp, int(max_cycles), float(tol_trans), float(tol_rot), out_ptr(q_out, (N, self.n), self.e.np_dtype),
-            out_ptr(cycles_out, (self.n,), np.int32), out_ptr(dist_out, (2, self.n), self.e.np_dtype)))
-        self.e.launches += rc
-        return rc
+        return self.e._launched(self.e._lib.vfk_session_solve(
+            self._s, qp, int(max_cycles), float(tol_trans), float(tol_rot), _out_ptr(q_out, (N, self.n), self.e.np_dtype),
+            _out_ptr(cycles_out, (self.n,), np.int32), _out_ptr(dist_out, (2, self.n), self.e.np_dtype)))
 
     def enable(self, *what: str, on: bool = True):
         """Ask the kernel to also write per-controller outputs ("qdot_vf", "qdot_ns", "qdot_jp", "cmd", "pose")."""
