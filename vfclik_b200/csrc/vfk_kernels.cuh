@@ -90,6 +90,15 @@ struct KConst {
     int32_t ns_qr;             // nullspace through the Householder basis of null(J): control mode, or the projector with ns_lambda = 0
 };
 
+// Chunk plan of one obstacle list (the instance's own list or the shared one), computed on the host (vfk_launch.cuh: chunk_plan).
+struct ChunkPlan {
+    int32_t n;                 // obstacles
+    int32_t np;                // n rounded up to even (whole pairs)
+    int32_t chunks;            // ceil(n / kChunk)
+    int32_t full;              // n / kChunk (chunks with all kChunk obstacles)
+    int32_t rem;               // n % kChunk
+};
+
 template <typename T>
 struct KArgs {
     T* q;
@@ -120,12 +129,8 @@ struct KArgs {
     int64_t qdot_ld;
     T* qdot_dev;               // direct host I/O: the blocked device mirror of qdot (kept current for vfk_session_read), or null
     int64_t n;
-    int32_t n_obst;
-    int32_t n_obst_p;          // n_obst rounded up to even: rows of 32 Vec4<T> per tile in `obst`
-    int32_t n_chunks;          // ceil(n_obst / kChunk)
-    int32_t n_full;            // n_obst / kChunk (chunks with all kChunk obstacles)
-    int32_t n_rem;             // n_obst % kChunk
-    int32_t n_stages;          // shared-memory stages (<= kMaxStages); >= n_chunks means resident
+    ChunkPlan own;             // the instance's own list in `obst`: own.np rows of 32 Vec4<T> per tile
+    int32_t n_stages;          // shared-memory stages (<= kMaxStages); >= own.chunks means resident
     int32_t k_cycles;
     int32_t n_aux;
     int32_t n_comp;            // joint components per instance in memory (<= N: generic chains of fewer joints run padded, see nc below)
@@ -135,13 +140,11 @@ struct KArgs {
     int32_t* cycles;           // [1] first cycle c whose q_c met the rule, or -1
     T* dist;                   // [2] {|p_goal - p_tool|, rotation angle} at the returned q, or null
     // SHARED kernels: the list shared by the whole batch (vfk_buffers.obst_shared = 1 or 2), staged into shared memory per
-    // CTA.  The obst / n_obst fields above then describe the instance's own list (mode 2), which runs through the ring as in
-    // the per-instance kernels, and are empty in a shared-only call.
-    const T* sh_obst;          // dense [sh_n][4] {x, y, z, radius}
-    const T* sh_obst_ext;      // dense [sh_n][2] {safe, order} or null
-    int32_t sh_n;
-    int32_t sh_np;             // sh_n rounded up to even
-    int32_t sh_chunks, sh_full, sh_rem;     // as n_chunks / n_full / n_rem
+    // CTA.  `obst` and `own` above then describe the instance's own list (mode 2), which runs through the ring as in the
+    // per-instance kernels, and are empty in a shared-only call.
+    const T* sh_obst;          // dense [sh.n][4] {x, y, z, radius}
+    const T* sh_obst_ext;      // dense [sh.n][2] {safe, order} or null
+    ChunkPlan sh;
 };
 
 // ------------------------------------------------------------------------------ chain patterns
@@ -323,14 +326,16 @@ struct Pos {
 // was a 2-way bank conflict), and in FP32 the two obstacles of a pair sit in adjacent registers exactly as sm_100's packed
 // FP32 instructions (fma / mul / add .f32x2 -> SASS FFMA2 / FMUL2 / FADD2) want their operands: the repulsor of TWO
 // obstacles issues as ~25 instructions instead of 2 x 22.
+// `load` takes the number of lanes a plane holds: 32 in the per-instance arrays and stages, 1 in a shared scene's staged list.
 template <typename T> struct ObstPairs;
 template <> struct ObstPairs<float> {
     static constexpr int kPlanes = 2;
     // obstacle `s` (0 / 1) of the pair whose first plane starts at `pair` (lane 0), for `lane`
+    template <int LANES = 32>
     static __device__ __forceinline__ Vec4<float> load(const Vec4<float>* pair, int lane, int s) {
         const float* f = reinterpret_cast<const float*>(pair) + lane * 4 + s;
         Vec4<float> o;
-        o.x = f[0]; o.y = f[2]; o.z = f[128]; o.w = f[130];
+        o.x = f[0]; o.y = f[2]; o.z = f[4 * LANES]; o.w = f[4 * LANES + 2];
         return o;
     }
     static __device__ __forceinline__ void store(Vec4<float>* pair, int lane, int s, const Vec4<float>& o) {
@@ -340,10 +345,11 @@ template <> struct ObstPairs<float> {
 };
 template <> struct ObstPairs<double> {
     static constexpr int kPlanes = 4;
+    template <int LANES = 32>
     static __device__ __forceinline__ Vec4<double> load(const Vec4<double>* pair, int lane, int s) {
         const double* f = reinterpret_cast<const double*>(pair) + lane * 2 + s;
         Vec4<double> o;
-        o.x = f[0]; o.y = f[64]; o.z = f[128]; o.w = f[192];
+        o.x = f[0]; o.y = f[2 * LANES]; o.z = f[4 * LANES]; o.w = f[6 * LANES];
         return o;
     }
     static __device__ __forceinline__ void store(Vec4<double>* pair, int lane, int s, const Vec4<double>& o) {
@@ -354,18 +360,11 @@ template <> struct ObstPairs<double> {
 
 // A scene shared by the whole batch (vfk_buffers.obst_shared) sits in shared memory once per CTA, in the form of ONE lane of
 // ObstPairs: pair p = {x0, x1, y0, y1, z0, z1, r0, r1} in T (FP32: two float4, FP64: four double2), then, with EXT, the dense
-// {safe, order} of every obstacle.  Every lane reads the same address: a broadcast, one wavefront per 16-byte read.
+// {safe, order} of every obstacle -- the per-instance layout with LANES = 1 (ObstPairs::load<1>, repel_chunk).  Every lane
+// reads the same address: a broadcast, one wavefront per 16-byte read.
 template <typename T, bool EXT>
 __host__ __device__ constexpr uint32_t shared_scene_bytes(int n_obst_p, int n_obst) {
     return (uint32_t)n_obst_p * (uint32_t)sizeof(Vec4<T>) + (EXT ? ((uint32_t)n_obst * (uint32_t)sizeof(Vec2<T>) + 15u) & ~15u : 0u);
-}
-
-template <typename T>
-__device__ __forceinline__ Vec4<T> shared_obst(const Vec4<T>* pair, int s) {
-    const T* f = reinterpret_cast<const T*>(pair) + s;
-    Vec4<T> o;
-    o.x = f[0]; o.y = f[2]; o.z = f[4]; o.w = f[6];
-    return o;
 }
 
 // The whole CTA converts the dense list [M][4] (and [M][2] ext) from global memory into that form; an odd M's padding slot
@@ -375,15 +374,15 @@ template <typename T, bool EXT>
 __device__ __forceinline__ void stage_shared_scene(const KArgs<T>& a, unsigned char* dst) {
     const T* src = a.sh_obst;
     T* o = reinterpret_cast<T*>(dst);
-    for (int i = (int)threadIdx.x; i < a.sh_np * 4; i += kBlock) {       // scalar i of the pair form: pair i / 8, slot i % 2,
+    for (int i = (int)threadIdx.x; i < a.sh.np * 4; i += kBlock) {       // scalar i of the pair form: pair i / 8, slot i % 2,
         const int m = (i >> 3) * 2 + (i & 1);                              // component (i / 2) % 4
-        o[i] = m < a.sh_n ? __ldg(src + m * 4 + ((i >> 1) & 3)) : T(0);
+        o[i] = m < a.sh.n ? __ldg(src + m * 4 + ((i >> 1) & 3)) : T(0);
     }
     if constexpr (EXT) {
         // with EXT both lists carry ext rows (the host checks it); a shared-only call without the own list passes its own
         const T* se = a.sh_obst_ext;
-        T* oe = reinterpret_cast<T*>(dst + (size_t)a.sh_np * sizeof(Vec4<T>));
-        for (int i = (int)threadIdx.x; i < a.sh_n * 2; i += kBlock) oe[i] = __ldg(se + i);
+        T* oe = reinterpret_cast<T*>(dst + (size_t)a.sh.np * sizeof(Vec4<T>));
+        for (int i = (int)threadIdx.x; i < a.sh.n * 2; i += kBlock) oe[i] = __ldg(se + i);
     }
 }
 
@@ -437,6 +436,73 @@ __device__ __forceinline__ void repel2(const float4& A, const float4& B, float s
     float2 wgt = __fmul2_rn(pw, inv);
     wgt = make_float2(fminf(wgt.x, 1e30f), fminf(wgt.y, 1e30f));          // see repel(): saturate instead of overflowing
     acc[0] = __ffma2_rn(wgt, dx, acc[0]); acc[1] = __ffma2_rn(wgt, dy, acc[1]); acc[2] = __ffma2_rn(wgt, dz, acc[2]);
+}
+
+// f(std::integral_constant<int, ORDER>{}) with the decay order the repulsor specialises for a uniform small-integer order
+// (KConst::order_int), else ORDER = 0 (pow at run time): order 20 in both precisions, 5 and 2 in FP64 too, and nothing for
+// per-obstacle orders (EXT).  A specialised order is a fixed multiplication chain instead of pow().  In FP32, order 20 by
+// five multiplications instead of MUFU lg2 / ex2 is two more instructions per obstacle but two fewer on the quarter-rate XU
+// pipe, which also carries rsqrt and the FP64 <-> FP32 conversions.  Measured on B200 (1 M instances): 109.1 us vs 110.3 us
+// per launch at K = 1, -0.6 % at K = 100; also the more accurate of the two.  20 is the reference's typical value
+// (old/README.old:75).
+template <typename T, bool EXT, class F>
+__device__ __forceinline__ void with_order(int order_int, F&& f) {
+    if constexpr (EXT) {
+        f(std::integral_constant<int, 0>{});
+    } else {
+        if (order_int == 20) f(std::integral_constant<int, 20>{});
+        else if constexpr (sizeof(T) == 8) {
+            if (order_int == 5) f(std::integral_constant<int, 5>{});
+            else if (order_int == 2) f(std::integral_constant<int, 2>{});
+            else f(std::integral_constant<int, 0>{});
+        } else {
+            f(std::integral_constant<int, 0>{});
+        }
+    }
+}
+
+// The repulsor over chunk `ch` of a list planned as `plan` and staged in shared memory, added to acc -- or, in FP32 without
+// EXT and one thread per instance, to acc2 on the packed pipe.  The chunk is in the ObstPairs layout with LANES lanes per
+// plane: pair p at pairs + 2 LANES p, its second plane LANES vectors further on, and the ext row of obstacle m at
+// ext[m * LANES] (`ext` already points at this slot).  A ring stage has 32 lanes and the instance's `slot`; a shared scene's
+// staged list has one lane, slot 0.  Both lists therefore go through the same repel / repel2 calls on the same operands in
+// the same order, with the same chunk split and order specialisations.  G > 1: lane ol of the cooperative group takes
+// obstacle ol of the chunk.  The plan is read here rather than passed in as a full-chunk flag and a count: passing those
+// reorders the instructions of most instantiations and costs registers in some.
+template <typename T, bool EXT, int G, int LANES>
+__device__ __forceinline__ void repel_chunk(const KConst<T>& c, const Vec4<T>* pairs, const Vec2<T>* ext, int slot, int ch,
+                                            const ChunkPlan& plan, int ol, const Pos<T>& pt, const NegPos2& np2, T (&acc)[3],
+                                            float2 (&acc2)[3]) {
+    // one obstacle by its index in the chunk: scalar form (FP64, per-obstacle {safe, order}, cooperative shape)
+    auto one = [&](int m, auto order_c) {
+        const Vec4<T> o = ObstPairs<T>::template load<LANES>(pairs + (m >> 1) * (2 * LANES), slot, m & 1);
+        T safe_inv = c.obst_safe_inv, order = c.obst_order;
+        if (EXT) { const Vec2<T> e = ext[m * LANES]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
+        repel<T, decltype(order_c)::value>(o, safe_inv, order, pt, acc);
+    };
+    if constexpr (G > 1) {
+        if (ol < (ch < plan.full ? kChunk : plan.rem)) one(ol, std::integral_constant<int, 0>{});
+    } else if constexpr (sizeof(T) == 4 && !EXT) {
+        // FP32: two obstacles per step on the packed FP32 pipe; a zero-radius padding slot contributes exactly 0
+        const float4* pl = reinterpret_cast<const float4*>(pairs) + slot;
+        if (ch < plan.full) {
+            with_order<T, EXT>(c.order_int, [&](auto order_c) {
+#pragma unroll
+                for (int p = 0; p < kChunk / 2; ++p)
+                    repel2<decltype(order_c)::value>(pl[p * 2 * LANES], pl[p * 2 * LANES + LANES], c.obst_safe_inv, c.obst_order, np2, acc2);
+            });
+        } else {
+            for (int p = 0; p < (plan.rem + 1) >> 1; ++p)
+                repel2<0>(pl[p * 2 * LANES], pl[p * 2 * LANES + LANES], c.obst_safe_inv, c.obst_order, np2, acc2);
+        }
+    } else if (ch < plan.full) {
+        with_order<T, EXT>(c.order_int, [&](auto order_c) {
+#pragma unroll
+            for (int m = 0; m < kChunk; ++m) one(m, order_c);
+        });
+    } else {
+        for (int m = 0; m < plan.rem; ++m) one(m, std::integral_constant<int, 0>{});
+    }
 }
 
 // What the attractor knows about the distance to the goal: d2 = |p_goal - p_tool|^2 (+ the tiny bias), dist = its root,
@@ -577,12 +643,12 @@ __device__ __forceinline__ void issue_obst(const KArgs<T>& a, int64_t tile, int 
     using WS = WarpStage<T, N, EXT>;
     if (lane == 0) {
         const int m0 = chunk * kChunk;
-        const uint32_t cnt = (uint32_t)min(kChunk, a.n_obst - m0);
+        const uint32_t cnt = (uint32_t)min(kChunk, a.own.n - m0);
         const uint32_t cntp = (cnt + 1u) & ~1u;                           // whole pairs (the odd one out carries a zero-radius slot)
         const uint32_t dst = region + (uint32_t)stage * WS::kStage, bar = bars + 8u * (uint32_t)stage;
         mbar_arrive_expect_tx_a(bar, cntp * WS::kRow + cnt * WS::kRowExt);
-        bulk_g2s_a(dst, a.obst + (tile * a.n_obst_p + m0) * 32, cntp * WS::kRow, bar);
-        if (EXT) bulk_g2s_a(dst + kChunk * WS::kRow, a.obst_ext + (tile * a.n_obst + m0) * 32, cnt * WS::kRowExt, bar);
+        bulk_g2s_a(dst, a.obst + (tile * a.own.np + m0) * 32, cntp * WS::kRow, bar);
+        if (EXT) bulk_g2s_a(dst + kChunk * WS::kRow, a.obst_ext + (tile * a.own.n + m0) * 32, cnt * WS::kRowExt, bar);
     }
 }
 
@@ -627,10 +693,10 @@ __device__ __forceinline__ void issue_qg(const KArgs<T>& a, int64_t tile, int bu
 // once (stage_shared_scene) before its one CTA-wide barrier, and the repulsor loop reads it there after the instance's own
 // obstacles.  The own list (mixed scene, obst_shared = 2) runs through the obstacle ring exactly as in the per-instance
 // kernels -- its stage plan, waits and refills, L2 prefetch and the solve's ring exit; with no own list (a shared-only call)
-// the ring is empty (n_chunks = n_stages = 0) and all of that does nothing, so an instance costs q and goal only.  The
-// per-obstacle arithmetic is the per-instance path's (the same repel2 / one() calls, chunk split and order
-// specialisations), so the field is bit-identical to it on the list [own ; shared] when the own count is a multiple of
-// kChunk (the shared chunks then start where they would in the concatenated list).
+// the ring is empty (own.chunks = n_stages = 0) and all of that does nothing, so an instance costs q and goal only.  Both
+// lists' chunks go through repel_chunk, the shared list's as a one-lane layout, so the field is bit-identical to the
+// per-instance path on the list [own ; shared] when the own count is a multiple of kChunk (the shared chunks then start
+// where they would in the concatenated list).
 template <typename T, int N, class PAT, bool EXT, bool LEAN, int MINB, int G = 1, bool SOLVE = false, bool SHARED = false>
 __global__ void __launch_bounds__(kBlock, MINB)
 vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KArgs<T> a) {
@@ -645,7 +711,7 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     unsigned char* region = smem + kSmemHeader + kTabBytes<T> + (size_t)warp * WS::warp_bytes(a.n_stages);
     [[maybe_unused]] const double2* sctab = reinterpret_cast<const double2*>(smem + kSmemHeader);
     [[maybe_unused]] unsigned char* scene = smem + kSmemHeader + kTabBytes<T>;      // SHARED: the staged list, before the warps' regions
-    if constexpr (SHARED) region += shared_scene_bytes<T, EXT>(a.sh_np, a.sh_n);
+    if constexpr (SHARED) region += shared_scene_bytes<T, EXT>(a.sh.np, a.sh.n);
     const uint32_t bars_a = smem_u32(bars), region_a = smem_u32(region);       // shared-window addresses, once per warp
     static_assert(G == 1 || G == kChunk, "a cooperative group takes one obstacle of a chunk per lane");
     constexpr int kSub = G == 1 ? 1 : G;                        // work units per tile (G == 8: 8 units of 4 instances)
@@ -653,7 +719,10 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     const int64_t n_units = n_tiles * kSub;
     const int64_t stride = (int64_t)gridDim.x * (kBlock / 32);
     int64_t unit = (int64_t)blockIdx.x * (kBlock / 32) + warp;
-    if constexpr (kTabBytes<T> == 0 && !SHARED) {
+    // The CTA fills shared memory that all its warps read (the FP32 sin / cos table, a SHARED kernel's scene) behind one
+    // CTA-wide barrier, which every warp has to pass, those without work included.  Without one a warp leaves at once.
+    constexpr bool kCtaBarrier = kTabBytes<T> != 0 || SHARED;
+    if constexpr (!kCtaBarrier) {
         if (unit >= n_units) return;
     }
     const int ol = lane & (G - 1);                              // obstacle lane within the group
@@ -662,15 +731,15 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     const int nc = (PAT::generic && !LEAN) ? a.n_comp : N;        // the lean instantiations only take chains of exactly N joints
 
     // Ring bookkeeping.  A "use" is one consumption of one chunk; a tile has U uses and the ring S slots.
-    // resident: S = n_chunks, every chunk is loaded once per tile and reused by all K cycles (U = n_chunks);
-    // streaming: S < n_chunks, chunks are re-requested every cycle (U = K * n_chunks).
+    // resident: S = own.chunks, every chunk is loaded once per tile and reused by all K cycles (U = own.chunks);
+    // streaming: S < own.chunks, chunks are re-requested every cycle (U = K * own.chunks).
     // The producer cursor (p_*) is always exactly S uses ahead of the consumer, so a refill targets the slot
     // the consumer has just finished with.  Everything advances by increments (no integer division).  The advance below is
     // what ring_produced / ring_consumed (vfk_ring.cuh) restate for the host; it stays written out here because routing it
     // through them changes the register allocation of every instantiation.
-    const bool resident = a.n_chunks <= a.n_stages;
-    const int S = resident ? a.n_chunks : a.n_stages;
-    const int U = resident ? a.n_chunks : a.n_chunks * a.k_cycles;
+    const bool resident = a.own.chunks <= a.n_stages;
+    const int S = resident ? a.own.chunks : a.n_stages;
+    const int U = resident ? a.own.chunks : a.own.chunks * a.k_cycles;
 
     if (lane == 0) {
         for (int s = 0; s < kMaxStages + 2; ++s) mbar_init(&bars[s], 1);
@@ -679,25 +748,18 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     __syncwarp();
     int64_t p_unit = unit;
     int p_u = 0, p_chunk = 0;
-    if ((kTabBytes<T> == 0 && !SHARED) || unit < n_units) {
+    if (!kCtaBarrier || unit < n_units) {
         issue_qg<T, N, EXT>(a, unit / kSub, 0, region_a, bars_a, lane, nc);
         for (int u = 0; u < S; ++u) {
             issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, u, region_a, bars_a, lane);
-            if (++p_chunk == a.n_chunks) p_chunk = 0;
+            if (++p_chunk == a.own.chunks) p_chunk = 0;
             if (++p_u == U) { p_u = 0; p_unit += stride; }
         }
     }
-    // SHARED: the scene is staged behind the first tile's copies too, and the same barrier publishes it (FP64 kernels have no
-    // table and get a barrier of their own, which is why no warp of a SHARED kernel leaves before it)
+    // the table and the scene are filled behind the first tile's copies; the barrier publishes them
     if constexpr (SHARED) stage_shared_scene<T, EXT>(a, scene);
-    if constexpr (kTabBytes<T> != 0) {
-        // the sin / cos table is built behind the first tile's copies; the only CTA-wide barrier, passed once by every warp
-        // (those without work included) before any can leave
-        sincos_table_fill(c.sincos, reinterpret_cast<double2*>(smem + kSmemHeader), (int)threadIdx.x, kBlock);
-        __syncthreads();
-    } else if constexpr (SHARED) {
-        __syncthreads();
-    }
+    if constexpr (kTabBytes<T> != 0) sincos_table_fill(c.sincos, reinterpret_cast<double2*>(smem + kSmemHeader), (int)threadIdx.x, kBlock);
+    if constexpr (kCtaBarrier) __syncthreads();
     int c_stage = 0;
     uint32_t c_phase = 0;
 
@@ -721,9 +783,9 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
         // warp's demand copies are queued at once, and skips the prefetch on its first tile (FP64 config 2: -3 % otherwise).
         if constexpr (G == 1) {
             const int first = S * kChunk;
-            const uint32_t bytes = a.n_obst_p > first ? (uint32_t)(a.n_obst_p - first) * 32u * (uint32_t)sizeof(Vec4<T>) : 0u;
+            const uint32_t bytes = a.own.np > first ? (uint32_t)(a.own.np - first) * 32u * (uint32_t)sizeof(Vec4<T>) : 0u;
             if (!resident && bytes != 0 && bytes <= 32768u && (it > 0 || n_units >= 4 * stride) && lane == 0)
-                bulk_prefetch_l2(a.obst + (tile * a.n_obst_p + first) * 32, bytes);
+                bulk_prefetch_l2(a.obst + (tile * a.own.np + first) * 32, bytes);
         }
         mbar_wait_a(bars_a + 8u * (uint32_t)(kMaxStages + (it & 1)), (uint32_t)(it >> 1) & 1u);
         const T* qg = reinterpret_cast<const T*>(region + (size_t)a.n_stages * WS::kStage + (size_t)(it & 1) * WS::kQg) + slot;
@@ -801,14 +863,14 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                     // the whole unit has stopped: wait what the ring still has in flight for it, refill those slots with the
                     // next unit's chunks, and move on.  A resident ring requests the next unit's chunks in the last cycle,
                     // so a cycle that leaves early does that instead.  An empty ring (a shared-only scene) has nothing left.
-                    const int left = resident ? (cyc < a.k_cycles ? a.n_chunks : 0)
-                                              : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.n_chunks, S, stride);
+                    const int left = resident ? (cyc < a.k_cycles ? a.own.chunks : 0)
+                                              : ring_leave(p_unit, p_u, p_chunk, (a.k_cycles - cyc) * a.own.chunks, S, stride);
                     for (int i = 0; i < left; ++i) {
                         const int stage = resident ? i : c_stage;
                         mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
                         __syncwarp();
                         if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                        ring_produced(p_unit, p_u, p_chunk, a.n_chunks, U, stride);
+                        ring_produced(p_unit, p_u, p_chunk, a.own.chunks, U, stride);
                         if (!resident) ring_consumed(c_stage, c_phase, S);
                     }
                     break;
@@ -818,106 +880,27 @@ vfk_cycle_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             [[maybe_unused]] float2 acc2[3] = {make_float2(0.f, 0.f), make_float2(0.f, 0.f), make_float2(0.f, 0.f)};
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) np2.set(pt);
             // the instance's own chunks, through the ring
-            for (int ch = 0; ch < a.n_chunks; ++ch) {
+            for (int ch = 0; ch < a.own.chunks; ++ch) {
                 const int stage = resident ? ch : c_stage;
                 mbar_wait_a(bars_a + 8u * (uint32_t)stage, resident ? (uint32_t)(it & 1) : c_phase);
                 const unsigned char* sb = region + (size_t)stage * WS::kStage;
-                const Vec4<T>* sp = reinterpret_cast<const Vec4<T>*>(sb);                      // pair p starts at sp + p * 64
-                const Vec2<T>* se = reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot;
-                const int n_here = ch < a.n_full ? kChunk : a.n_rem;                           // obstacles in this chunk
-                // one obstacle by its index in the chunk: scalar form (FP64, per-obstacle {safe, order}, cooperative shape)
-                auto one = [&](int m, auto order_c) {
-                    constexpr int ORD = decltype(order_c)::value;
-                    const Vec4<T> o = ObstPairs<T>::load(sp + (m >> 1) * 64, slot, m & 1);
-                    T safe_inv = c.obst_safe_inv, order = c.obst_order;
-                    if (EXT) { const Vec2<T> e = se[m * 32]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
-                    repel<T, ORD>(o, safe_inv, order, pt, acc);
-                };
-                if constexpr (G > 1) {
-                    // cooperative shape: lane ol of the group takes obstacle ol of this chunk
-                    if (ol < n_here) one(ol, std::integral_constant<int, 0>{});
-                } else if constexpr (sizeof(T) == 4 && !EXT) {
-                    // FP32: two obstacles per step on the packed FP32 pipe; a zero-radius padding slot contributes exactly 0
-                    const float4* pl = reinterpret_cast<const float4*>(sb) + slot;
-                    if (ch < a.n_full) {
-                        auto full_chunk = [&](auto order_c) {
-#pragma unroll
-                            for (int p = 0; p < kChunk / 2; ++p)
-                                repel2<decltype(order_c)::value>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
-                        };
-                        // decay order 20 (the reference's typical value, old/README.old:75) by five multiplications instead of
-                        // MUFU lg2 / ex2: two more instructions per obstacle but two fewer on the quarter-rate XU pipe, which also
-                        // carries rsqrt and the FP64 <-> FP32 conversions.  Measured on B200 (1 M instances): 109.1 us vs 110.3 us
-                        // per launch at K = 1, -0.6 % at K = 100; also the more accurate of the two.
-                        if (c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
-                        else full_chunk(std::integral_constant<int, 0>{});
-                    } else {
-                        for (int p = 0; p < (a.n_rem + 1) >> 1; ++p)
-                            repel2<0>(pl[p * 64], pl[p * 64 + 32], c.obst_safe_inv, c.obst_order, np2, acc2);
-                    }
-                } else if (ch < a.n_full) {
-                    // FP64 with a uniform small-integer decay order: fixed multiplication chain instead of pow()
-                    auto full_chunk = [&](auto order_c) {
-#pragma unroll
-                        for (int m = 0; m < kChunk; ++m) one(m, order_c);
-                    };
-                    if (sizeof(T) == 8 && !EXT && c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
-                    else if (sizeof(T) == 8 && !EXT && c.order_int == 5) full_chunk(std::integral_constant<int, 5>{});
-                    else if (sizeof(T) == 8 && !EXT && c.order_int == 2) full_chunk(std::integral_constant<int, 2>{});
-                    else full_chunk(std::integral_constant<int, 0>{});
-                } else {
-                    for (int m = 0; m < a.n_rem; ++m) one(m, std::integral_constant<int, 0>{});
-                }
+                repel_chunk<T, EXT, G, 32>(c, reinterpret_cast<const Vec4<T>*>(sb), reinterpret_cast<const Vec2<T>*>(sb + kChunk * WS::kRow) + slot,
+                                           slot, ch, a.own, ol, pt, np2, acc, acc2);
                 // this slot is free again: request the chunk that will occupy it S uses from now
                 if (!resident || last) {
                     __syncwarp();
                     if (p_unit < n_units) issue_obst<T, N, EXT>(a, p_unit / kSub, p_chunk, stage, region_a, bars_a, lane);
-                    if (++p_chunk == a.n_chunks) p_chunk = 0;
+                    if (++p_chunk == a.own.chunks) p_chunk = 0;
                     if (++p_u == U) { p_u = 0; p_unit += stride; }
                 }
                 if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
             }
-            // SHARED: then the shared list's chunks from the staged scene -- kChunk consecutive obstacles, one lane's worth of each
-            // pair and ext row -- through the same per-obstacle calls as the ring loop above (own obstacles first)
+            // SHARED: then the shared list's chunks from the staged scene, one lane of kChunk consecutive obstacles each
             if constexpr (SHARED) {
-                const Vec2<T>* se_all = reinterpret_cast<const Vec2<T>*>(scene + (size_t)a.sh_np * sizeof(Vec4<T>));
-                for (int ch = 0; ch < a.sh_chunks; ++ch) {
-                    const Vec4<T>* sp = reinterpret_cast<const Vec4<T>*>(scene) + (size_t)ch * kChunk;       // pair p at sp + 2 p
-                    const Vec2<T>* se = se_all + ch * kChunk;
-                    auto one = [&](int m, auto order_c) {
-                        constexpr int ORD = decltype(order_c)::value;
-                        const Vec4<T> o = shared_obst<T>(sp + (m >> 1) * 2, m & 1);
-                        T safe_inv = c.obst_safe_inv, order = c.obst_order;
-                        if (EXT) { const Vec2<T> e = se[m]; safe_inv = Prec<T>::rcp(e.x); order = e.y; }
-                        repel<T, ORD>(o, safe_inv, order, pt, acc);
-                    };
-                    if constexpr (sizeof(T) == 4 && !EXT) {
-                        const float4* pl = reinterpret_cast<const float4*>(sp);
-                        if (ch < a.sh_full) {
-                            auto full_chunk = [&](auto order_c) {
-#pragma unroll
-                                for (int p = 0; p < kChunk / 2; ++p)
-                                    repel2<decltype(order_c)::value>(pl[p * 2], pl[p * 2 + 1], c.obst_safe_inv, c.obst_order, np2, acc2);
-                            };
-                            if (c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
-                            else full_chunk(std::integral_constant<int, 0>{});
-                        } else {
-                            for (int p = 0; p < (a.sh_rem + 1) >> 1; ++p)
-                                repel2<0>(pl[p * 2], pl[p * 2 + 1], c.obst_safe_inv, c.obst_order, np2, acc2);
-                        }
-                    } else if (ch < a.sh_full) {
-                        auto full_chunk = [&](auto order_c) {
-#pragma unroll
-                            for (int m = 0; m < kChunk; ++m) one(m, order_c);
-                        };
-                        if (sizeof(T) == 8 && !EXT && c.order_int == 20) full_chunk(std::integral_constant<int, 20>{});
-                        else if (sizeof(T) == 8 && !EXT && c.order_int == 5) full_chunk(std::integral_constant<int, 5>{});
-                        else if (sizeof(T) == 8 && !EXT && c.order_int == 2) full_chunk(std::integral_constant<int, 2>{});
-                        else full_chunk(std::integral_constant<int, 0>{});
-                    } else {
-                        for (int m = 0; m < a.sh_rem; ++m) one(m, std::integral_constant<int, 0>{});
-                    }
-                }
+                const Vec2<T>* se = reinterpret_cast<const Vec2<T>*>(scene + (size_t)a.sh.np * sizeof(Vec4<T>));
+                for (int ch = 0; ch < a.sh.chunks; ++ch)
+                    repel_chunk<T, EXT, 1, 1>(c, reinterpret_cast<const Vec4<T>*>(scene) + (size_t)ch * kChunk, se + ch * kChunk, 0, ch, a.sh, 0,
+                                              pt, np2, acc, acc2);
             }
             if constexpr (sizeof(T) == 4 && !EXT && G == 1) {
 #pragma unroll

@@ -47,14 +47,9 @@ static const KConst<T>& kconst(const vfk_ctx* h) {
     if constexpr (sizeof(T) == 4) return h->cf; else return h->cd;
 }
 
-// Chunk plan of a list of m obstacles, as KArgs holds it for the own list and for the shared list: the count, whole pairs,
-// chunks of kChunk obstacles, full chunks and the remainder.
-static void chunk_plan(int m, int32_t& n, int32_t& np, int32_t& chunks, int32_t& full, int32_t& rem) {
-    n = m;
-    np = (m + 1) & ~1;
-    chunks = (m + kChunk - 1) / kChunk;
-    full = m / kChunk;
-    rem = m % kChunk;
+// Chunk plan of a list of m obstacles, as KArgs holds it for the own list and for the shared list.
+static ChunkPlan chunk_plan(int m) {
+    return ChunkPlan{m, (m + 1) & ~1, (m + kChunk - 1) / kChunk, m / kChunk, m % kChunk};
 }
 
 // The launch of every cycle-kernel shape: `units` warp-sized work units, each warp a persistent worker, so at most as many
@@ -136,8 +131,8 @@ static int launch_cycle(vfk_ctx* h, const CycleCall& call) {
         a.cycles = sv->cycles;
         a.dist = static_cast<T*>(sv->dist);
     }
-    chunk_plan(sc.own.m, a.n_obst, a.n_obst_p, a.n_chunks, a.n_full, a.n_rem);
-    a.n_stages = a.n_chunks < kRingStages<T, N> ? a.n_chunks : kRingStages<T, N>;
+    a.own = chunk_plan(sc.own.m);
+    a.n_stages = a.own.chunks < kRingStages<T, N> ? a.own.chunks : kRingStages<T, N>;
     size_t smem = kSmemHeader + kTabBytes<T> + (size_t)(kBlock / 32) * WarpStage<T, N, EXT>::warp_bytes(a.n_stages);
     if constexpr (SHARED) {
         // Shared memory: the own ring (its usual plan on the own count; no stages without one), the staged shared list and
@@ -148,8 +143,8 @@ static int launch_cycle(vfk_ctx* h, const CycleCall& call) {
                       "a mixed scene at the shared-list cap does not fit an SM");
         a.sh_obst = static_cast<const T*>(sc.shared.obst);
         a.sh_obst_ext = static_cast<const T*>(sc.shared.obst_ext);
-        chunk_plan(sc.shared.m, a.sh_n, a.sh_np, a.sh_chunks, a.sh_full, a.sh_rem);
-        smem += shared_scene_bytes<T, EXT>(a.sh_np, a.sh_n);
+        a.sh = chunk_plan(sc.shared.m);
+        smem += shared_scene_bytes<T, EXT>(a.sh.np, a.sh.n);
     }
     // resident CTAs per SM that the register allocation aims for.  The shared-scene FP32 lean solve kernels of N <= 7 ask for
     // four: at three the LWR one took 130 registers where its per-instance twin takes 128, one resident CTA fewer (at four it
@@ -223,8 +218,8 @@ static int launch_split(vfk_ctx* h, const CycleCall& call) {
     a.n = call.n;
     a.n_comp = h->chain.n_joints;
     a.k_cycles = call.k_cycles;
-    chunk_plan(call.scene.own.m, a.n_obst, a.n_obst_p, a.n_chunks, a.n_full, a.n_rem);
-    a.n_stages = a.n_chunks < 2 ? a.n_chunks : 2;
+    a.own = chunk_plan(call.scene.own.m);
+    a.n_stages = a.own.chunks < 2 ? a.own.chunks : 2;
     const size_t smem = kSmemHeader + SH::kTab + (size_t)(kBlock / 32) * SH::warp_bytes(a.n_stages);
     const uint64_t tiles = (uint64_t)((call.n + 31) / 32);
     SplitMaps maps;
@@ -232,8 +227,8 @@ static int launch_split(vfk_ctx* h, const CycleCall& call) {
     int rc;
     if ((rc = encode_map3<T>(h, &maps.q, b->q, 32, (uint64_t)a.n_comp, tiles, SH::SUB, (uint32_t)a.n_comp)) != VFK_OK) return rc;
     if ((rc = encode_map3<T>(h, &maps.goal, b->goal, 32, 13, tiles, SH::SUB, 13)) != VFK_OK) return rc;
-    if (a.n_obst > 0) {
-        const uint64_t rows = (uint64_t)a.n_obst_p / 2 * ObstPairs<T>::kPlanes;                   // plane rows of 32 lanes x 16 bytes per tile
+    if (a.own.n > 0) {
+        const uint64_t rows = (uint64_t)a.own.np / 2 * ObstPairs<T>::kPlanes;                   // plane rows of 32 lanes x 16 bytes per tile
         if ((rc = encode_map3<T>(h, &maps.obst, call.scene.own.obst, 32 * 16 / sizeof(T), rows, tiles, SH::kRowBytes / sizeof(T),
                                  SH::kRowsPerChunk)) != VFK_OK)
             return rc;

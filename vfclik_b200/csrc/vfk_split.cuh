@@ -132,9 +132,9 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     int64_t unit = (int64_t)blockIdx.x * (kBlock / 32) + warp;
     if (unit >= n_units) return;
 
-    const bool resident = a.n_chunks <= a.n_stages;
-    const int S = resident ? a.n_chunks : a.n_stages;
-    const int U = resident ? a.n_chunks : a.n_chunks * a.k_cycles;
+    const bool resident = a.own.chunks <= a.n_stages;
+    const int S = resident ? a.own.chunks : a.n_stages;
+    const int U = resident ? a.own.chunks : a.own.chunks * a.k_cycles;
     const uint32_t qg_bytes = (uint32_t)(nc + 13) * SUB * sizeof(T);
 
     auto issue_qg = [&](int64_t u, int buf) {
@@ -164,7 +164,7 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
     int p_u = 0, p_chunk = 0;
     for (int u = 0; u < S; ++u) {
         issue_obst(p_unit, p_chunk, u);
-        if (++p_chunk == a.n_chunks) p_chunk = 0;
+        if (++p_chunk == a.own.chunks) p_chunk = 0;
         if (++p_u == U) { p_u = 0; p_unit += stride; }
     }
     int c_stage = 0;
@@ -268,17 +268,17 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
             {
                 T V[3], S0, w[3], acc[3] = {T(0), T(0), T(0)};
                 attract<T>(c, g, Rt, pt, V, S0, w);
-                for (int ch = 0; ch < a.n_chunks; ++ch) {
+                for (int ch = 0; ch < a.own.chunks; ++ch) {
                     const int stage = resident ? ch : c_stage;
                     mbar_wait(&bars[stage], resident ? (uint32_t)(it & 1) : c_phase);
                     const unsigned char* sb = region + (size_t)stage * SH::kStage;
-                    const int n_here = ch < a.n_full ? kChunk : a.n_rem;
+                    const int n_here = ch < a.own.full ? kChunk : a.own.rem;
                     const int n_pairs = (n_here + 1) >> 1;
                     // stage = [pair][4 planes][SUB lanes] of double2 {slot 0, slot 1}
                     const double2* pl = reinterpret_cast<const double2*>(sb) + sl;
                     auto deal = [&](auto order_c) {
                         constexpr int ORD = decltype(order_c)::value;
-                        const bool full = ch < a.n_full;
+                        const bool full = ch < a.own.full;
 #pragma unroll
                         for (int i = 0; i < (kChunk / 2 + L - 1) / L; ++i) {
                             const int pr = i * L + h;
@@ -292,14 +292,11 @@ vfk_split_kernel(const __grid_constant__ KConst<T> c, const __grid_constant__ KA
                             }
                         }
                     };
-                    if (c.order_int == 20) deal(std::integral_constant<int, 20>{});
-                    else if (c.order_int == 5) deal(std::integral_constant<int, 5>{});
-                    else if (c.order_int == 2) deal(std::integral_constant<int, 2>{});
-                    else deal(std::integral_constant<int, 0>{});
+                    with_order<T, false>(c.order_int, deal);
                     if (!resident || last) {
                         __syncwarp();
                         if (p_unit < n_units) issue_obst(p_unit, p_chunk, stage);
-                        if (++p_chunk == a.n_chunks) p_chunk = 0;
+                        if (++p_chunk == a.own.chunks) p_chunk = 0;
                         if (++p_u == U) { p_u = 0; p_unit += stride; }
                     }
                     if (!resident && ++c_stage == S) { c_stage = 0; c_phase ^= 1u; }
